@@ -10,8 +10,15 @@ routine of examples/pmg/main.cpp:412-435 is run on ndofs * n_gpus).  One "step" 
 the per-apply throughput of the fine-level operator and its HBM roofline fraction are reported
 in "apply" / "roofline".
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--ndofs D] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--ndofs D] [--impl reference] [--dump-outputs DIR]
   torchrun --nproc-per-node N bench.py --gpus N ...     (one rank per GPU, NCCL halo exchange)
+
+--dump-outputs DIR: after the timed V-cycles, write the solution u they left behind (what a caller of
+MultigridPreconditioner::apply receives) as DIR/u.npy, a fixed seeded sample of its owned entries in
+float64, with their positions in DIR/u_index.npy (float64, exact), so that two builds run with the
+same arguments can be compared output for output.  With N ranks each rank writes a sample of at most
+2^20 / N entries as u_rank<r>.npy / u_rank<r>_index.npy, so a dump holds at most 2^20 values and
+2^20 positions (16 MiB) for any number of ranks.
 
 --impl reference: the reference's CPU path cannot be installed here (DOLFINx/PETSc absent), so
 the arm times the oracle's C/OpenMP restatement of the same V-cycle on the host cores, on a
@@ -36,6 +43,18 @@ NSMOOTH = 2
 COARSE_ITS, COARSE_RTOL = 60, 1e-5
 PGRID = {1: (1, 1, 1), 2: (2, 1, 1), 4: (2, 2, 1), 8: (2, 2, 2)}
 METRIC = "fine-level Gdof/s per p-MG V-cycle (P4->P2->P1, Chebyshev(2), CSR coarse solve)"
+DUMP_SAMPLE, DUMP_SEED = 1 << 20, 20240611   # 2^20 float64 values + positions over all ranks: 16 MiB
+
+
+def dump_output(torch, v, out_dir, name, sample):
+    """Write a fixed seeded sample of at most `sample` entries of the device vector v (all of it when it
+    is small) and the sampled positions as out_dir/<name>.npy and out_dir/<name>_index.npy, both float64."""
+    n = v.numel()
+    idx = np.arange(n) if n <= sample else np.unique(np.random.default_rng(DUMP_SEED).integers(0, n, sample))
+    vals = v[torch.from_numpy(idx).to(v.device)].cpu().numpy()
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, f"{name}.npy"), vals.astype(np.float64))
+    np.save(os.path.join(out_dir, f"{name}_index.npy"), idx.astype(np.float64))
 
 
 def b_apply(P, ncells, ndofs):
@@ -175,14 +194,19 @@ def cpu_baseline(steps=2, warmup=1, n=64):
             "ms_per_step": dt * 1e3, "apply_gdofs": nd / dta / 1e9}
 
 
+def cpu_baseline_args(args):
+    """Timed and warm-up V-cycles and sample size of the CPU leg: the run's --steps / --warmup (at least one
+    warm-up cycle), on a bounded sample: 64^3 cells (16.97 M P4 dofs, ~6 s per V-cycle on 8 cores) while
+    the whole run stays within a few minutes, else 48^3."""
+    return dict(steps=args.steps, warmup=max(args.warmup, 1),
+                n=args.cpu_cells or (64 if args.steps + args.warmup <= 24 else 48))
+
+
 def run_reference(args):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
-    # bounded sample: 64^3 cells (16.97 M P4 dofs, ~6 s per V-cycle on 8 cores) while the whole run stays
-    # within a few minutes, else 48^3
-    n = args.cpu_cells or (64 if args.steps + args.warmup <= 24 else 48)
-    cb = cpu_baseline(steps=max(args.steps, 1), warmup=max(args.warmup, 1), n=n)
+    cb = cpu_baseline(**cpu_baseline_args(args))
     line = {"impl": "reference", "metric": METRIC, "value": cb["value"], "unit": "Gdof/s", "n_gpus": args.gpus,
             "steps": args.steps, "warmup": args.warmup, "ms_per_step": cb["ms_per_step"],
             "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "f64", "data": "synthetic",
@@ -355,6 +379,9 @@ def run_gpu(args):
     e1.record(ctx.stream)
     barrier()
     ms = e0.elapsed_time(e1)
+    if args.dump_outputs:
+        dump_output(torch, u.data[:n_owned], args.dump_outputs, "u" if world == 1 else f"u_rank{rank}",
+                    DUMP_SAMPLE // world)
     import ctypes
     kms, kl = ctypes.c_double(), ctypes.c_longlong()
     api.check(api.lib.pmgx_ctx_profile_read(ctx.h, Ptop, ctypes.addressof(kms), ctypes.addressof(kl)))
@@ -424,7 +451,7 @@ def run_gpu(args):
     bb = [b, api.Vector(ctx, sp.n_owned, sp.n_ghost, halo_top)]
     us = [torch.empty(n_owned, dtype=torch.float64, device=ctx.device) for _ in range(2)]
     s_up, s_down = torch.cuda.Stream(device=ctx.device), torch.cuda.Stream(device=ctx.device)
-    e2e_steps = max(2, args.steps)
+    e2e_steps = args.steps
 
     def e2e_loop(nsteps, e_begin=None, e_end=None):
         trace = bool(os.environ.get("PMGX_E2E_TRACE")) and e_begin is not None
@@ -544,7 +571,7 @@ def run_gpu(args):
         cb = None
         if world == 1 and not args.no_cpu:
             try:
-                cb = cpu_baseline(n=args.cpu_cells or 64)
+                cb = cpu_baseline(**cpu_baseline_args(args))
             except Exception as e:  # the CPU leg must never take the GPU line down with it
                 sys.stderr.write(f"cpu_baseline failed: {e}\n")
         line = {
@@ -595,7 +622,12 @@ def main():
     ap.add_argument("--cpu-cells", type=int, default=0, help="cells per direction of the CPU sample (0: 64, or 48 for long runs)")
     ap.add_argument("--no-parity", action="store_true", help="skip the in-process parity check before the timed region")
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write a sample of the last timed V-cycle's solution to DIR")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the GPU path's solution; it needs --impl b200")
     args.ndofs = int(args.ndofs)
     if args.impl == "reference":
         run_reference(args)

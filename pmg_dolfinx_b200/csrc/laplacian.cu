@@ -9,13 +9,14 @@
 // Design (not a port): cells are re-laid-out at create time in launch order (lcells then
 // bcells); the dofmap is snapshotted with the Dirichlet marker folded into the sign bit, so
 // the apply never gathers bc_marker; G is stored component-major per batch of cells so that one
-// (ix) plane of a batch is one contiguous cp.async.bulk transaction.  Apply kernels:
-//   k_apply_affine / k_apply_affine_shfl   every cell affine: one geometry 6-vector per cell
-//   k_apply_tma                            streamed G through a TMA ring (P1..P6)
-//   k_apply_slab                           same thread mapping, register-streamed G (A/B runs)
-//   k_apply                                column kernel (P7, P8)
-// In the slab kernels a thread owns one z-index of a cell and keeps the (ix,iy) slab of the
-// element in registers: the x and y contractions are register FMAs against constant-memory
+// (ix) plane of a batch is one contiguous cp.async.bulk transaction.  One apply kernel per degree
+// and geometry, chosen in ApplyKernels<P> below:
+//   k_apply_affine / _affine_shfl / _affine2   P1..P5, every cell affine: one geometry 6-vector per cell
+//   k_apply_tma                                P1..P5, G streamed per quadrature point through a TMA ring
+//   k_apply_affine_mma                         P6, P7: FP64 tensor cores, one warp per cell (laplacian_mma.cuh)
+//   k_apply                                    P8: column kernel
+// In the slab kernels (P1..P5) a thread owns one z-index of a cell and keeps the (ix,iy) slab of
+// the element in registers: the x and y contractions are register FMAs against constant-memory
 // derivative entries, only the z contraction crosses threads.
 #include "common.hpp"
 #include "operator.hpp"
@@ -30,13 +31,13 @@
 #include <cmath>
 #include <cstdlib>
 #include <cstring>
+#include <type_traits>
 
 namespace pmgx
 {
 namespace
 {
 constexpr int MAXN = PMGX_MAX_DEGREE + 1;
-constexpr int SLAB_MAX_DEGREE = 6; // slab kernels (2 (P+1)^2 doubles of registers) up to here; above: column kernel (measured: P7 53 % vs 47 %, P8 24 % vs 27 %)
 
 // 1-D tables for every degree; index [P][...]
 __constant__ double c_D[PMGX_MAX_DEGREE + 1][MAXN * MAXN]; // D[q*n+i] = l_i'(x_q)
@@ -55,10 +56,11 @@ __device__ __forceinline__ int ldg_stream_i32(const int* p) { return __ldcs(p); 
 // How the operator-private arrays (BC-encoded dofmap, geometry factors) are laid out.  The
 // reference keeps G private (src/laplacian.hpp:512), so the layout is free: it follows the
 // thread mapping of the apply kernel so that every warp load is one aligned, contiguous run.
-//   COLUMN: enc[p][n3], G[p][6][n3]                         (thread = (iy,iz) column, P >= 5)
-//   SLAB  : enc[batch][n2][S], G[batch][n2][6][S]           (thread = iz slab,        P <= 4)
-//           batch = CPB consecutive cells of the launch list, slot = cell_in_batch*n + iz,
-//           S = 128 slots (padded); lcells and bcells batches are padded separately.
+//   COLUMN: enc[p][n3], G[p][6][n3]                         (P6..P8: a warp or an (iy,iz) column per cell)
+//   SLAB  : enc[batch][n2][SE], G[batch][n2][6][S]          (P1..P5: thread = iz slab)
+//           batch = cpb consecutive cells of the launch list (cpb of the kernel that runs),
+//           slot = cell_in_batch*n + iz, S / SE padded to 16-byte rows; lcells and bcells
+//           batches are padded separately.
 struct Lay
 {
   int mode; // 0 COLUMN, 1 SLAB
@@ -426,7 +428,75 @@ __global__ void k_offdiag(const int32_t* __restrict__ row_ptr, const int32_t* __
     off_diag[i] = row_ptr[i] + owned_count[i];
 }
 
-// ----------------------------------------------------------------- the apply kernel --
+// ---------------------------------------------------------------- apply launches --
+// One launch of an apply kernel: the cells [cell0, cell0 + count) of the launch list, whose first
+// batch in the SLAB layout is batch0 (the COLUMN-layout kernels ignore it); geom is Gc for the
+// kernels that take one geometry 6-vector per cell, G otherwise.
+struct ApplyArgs
+{
+  const double* x;
+  double* y;
+  const double* geom;
+  const int32_t* enc;
+  const int32_t* perm;
+  const double* kappa;
+  long long batch0;
+  int cell0, count;
+};
+
+// Launches a persistent apply kernel of degree P: CTAs of tpb threads stay resident and walk over the
+// n_blocks blocks of work (blockIdx.x, + gridDim.x, ...), so exactly as many are launched as fit on the
+// device at once.  The shared-memory opt-in and the occupancy query run once per device and kernel.
+template <auto kernel, typename... Tail>
+void launch_persistent(pmgx_ctx* c, cudaStream_t st, const ApplyArgs& a, const char* name, int P, int tpb,
+                       size_t smem, int n_blocks, Tail... tail)
+{
+  if (a.count <= 0)
+    return;
+  static int ctas_per_sm[64] = {0};
+  if (ctas_per_sm[c->device] == 0)
+  {
+    PMGX_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    int nb = 0;
+    PMGX_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, kernel, tpb, smem));
+    PMGX_REQUIRE(nb >= 1, "%s (P%d) does not fit on an SM", name, P);
+    ctas_per_sm[c->device] = nb;
+  }
+  const int grid = std::min(n_blocks, ctas_per_sm[c->device] * c->num_sms);
+  const bool timed = c->profiling && a.cell0 == 0; // per-kernel timing covers the interior-cell launch only
+  cudaEvent_t e0 = nullptr, e1 = nullptr;
+  if (timed)
+  {
+    PMGX_CUDA(cudaEventCreate(&e0));
+    PMGX_CUDA(cudaEventCreate(&e1));
+    PMGX_CUDA(cudaEventRecord(e0, st));
+  }
+  kernel<<<grid, tpb, smem, st>>>(a.x, a.y, a.geom, a.enc, a.perm, a.kappa, tail...);
+  check_launch(name);
+  count_launch(c);
+  if (timed)
+  {
+    PMGX_CUDA(cudaEventRecord(e1, st));
+    c->prof[P].emplace_back(e0, e1);
+  }
+}
+
+// The SLAB-layout kernels (k_apply_tma, k_apply_affine*): one block of work is one batch of Cfg::cpb cells
+template <auto kernel, typename Cfg>
+void launch_batched(pmgx_ctx* c, cudaStream_t st, const ApplyArgs& a, const char* name)
+{
+  const int nbatch = (a.count + Cfg::cpb - 1) / Cfg::cpb;
+  launch_persistent<kernel>(c, st, a, name, Cfg::n - 1, Cfg::tpb, Cfg::smem, nbatch, a.batch0, a.cell0, a.count,
+                            nbatch);
+}
+
+// Every launcher below (one per kernel family) exports
+//   cell_geometry  the kernel reads Gc (one geometry 6-vector per affine cell) instead of G
+//   cpb            cells per batch of the SLAB layout; 0: the kernel reads the COLUMN layout
+//   name()         the kernel and its template arguments, as pmgx_laplacian_kernel_name reports them
+//   launch()
+
+// ------------------------------------------------------------ the column apply kernel --
 // smem row stride: pad when a (j -> j+1) step of n doubles would alias banks (n % 8 == 0)
 template <int P>
 struct ApplyCfg
@@ -436,8 +506,8 @@ struct ApplyCfg
   static constexpr int n3 = n2 * n;
   static constexpr int row = (n % 8 == 0) ? n + 1 : n;
   static constexpr int plane = n * row;
-  // threads per block: the smallest of {128,160,192,256} wasting the fewest lanes
-  static constexpr int tpb = (P == 5 || P == 6) ? 160 : (P == 8 ? 256 : 128);
+  // threads per block: the smallest of {128,192,256} wasting the fewest lanes
+  static constexpr int tpb = P == 8 ? 256 : 128;
   static constexpr int cpb = tpb / n2; // cells per block
   static constexpr int smem_doubles = cpb * (n * plane + 4 * plane);
 };
@@ -583,255 +653,55 @@ k_apply(const double* __restrict__ x, double* __restrict__ y, const double* __re
   }
 }
 
+// Not persistent: one CTA per ApplyCfg<P>::cpb cells of the COLUMN layout
 template <int P>
-void launch_apply(pmgx_ctx* c, cudaStream_t st, const double* x, double* y, const double* G, const int32_t* enc,
-                  const int32_t* perm, const double* kappa, int first, int count)
+struct ColumnApply
 {
-  const bool timed = c->profiling && first == 0; // per-kernel timing covers the interior-cell launch only
-  if (count <= 0)
-    return;
   using C = ApplyCfg<P>;
-  const size_t smem = (size_t)C::smem_doubles * sizeof(double);
-  static bool configured[64] = {false};
-  if (!configured[c->device])
+  static constexpr bool cell_geometry = false;
+  static constexpr int cpb = 0;
+  static void name(char* s, int cap) { snprintf(s, cap, "k_apply<%d>", P); }
+  static void launch(pmgx_ctx* c, cudaStream_t st, const ApplyArgs& a)
   {
-    PMGX_CUDA(cudaFuncSetAttribute(k_apply<P>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    configured[c->device] = true;
+    if (a.count <= 0)
+      return;
+    const size_t smem = (size_t)C::smem_doubles * sizeof(double);
+    static bool configured[64] = {false};
+    if (!configured[c->device])
+    {
+      PMGX_CUDA(cudaFuncSetAttribute(k_apply<P>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+      configured[c->device] = true;
+    }
+    const int grid = (a.count + C::cpb - 1) / C::cpb;
+    const bool timed = c->profiling && a.cell0 == 0; // per-kernel timing covers the interior-cell launch only
+    cudaEvent_t e0 = nullptr, e1 = nullptr;
+    if (timed)
+    {
+      PMGX_CUDA(cudaEventCreate(&e0));
+      PMGX_CUDA(cudaEventCreate(&e1));
+      PMGX_CUDA(cudaEventRecord(e0, st));
+    }
+    k_apply<P><<<grid, C::tpb, smem, st>>>(a.x, a.y, a.geom, a.enc, a.perm, a.kappa, a.cell0, a.count);
+    check_launch("k_apply");
+    count_launch(c);
+    if (timed)
+    {
+      PMGX_CUDA(cudaEventRecord(e1, st));
+      c->prof[P].emplace_back(e0, e1);
+    }
   }
-  const int grid = (count + C::cpb - 1) / C::cpb;
-  cudaEvent_t e0 = nullptr, e1 = nullptr;
-  if (timed)
-  {
-    PMGX_CUDA(cudaEventCreate(&e0));
-    PMGX_CUDA(cudaEventCreate(&e1));
-    PMGX_CUDA(cudaEventRecord(e0, st));
-  }
-  k_apply<P><<<grid, C::tpb, smem, st>>>(x, y, G, enc, perm, kappa, first, count);
-  check_launch("k_apply");
-  count_launch(c);
-  if (timed)
-  {
-    PMGX_CUDA(cudaEventRecord(e1, st));
-    c->prof[P].emplace_back(e0, e1);
-  }
-}
+};
 
-// ------------------------------------------------------------- the slab apply kernel --
+// --------------------------------------------- the TMA-pipelined slab apply kernel --
 // Thread = one z-index k of one cell; it keeps the whole (ix,iy) slab of the element in
 // registers, so the x and y contractions are pure register FMAs with compile-time D entries
 // and only the z contraction exchanges data through shared memory (rows of n values that all
 // n threads of a cell read as a broadcast).  This moves ~1/3 of the bytes of the column
 // kernel through the LSU/shared-memory pipe, which ncu showed to be the limiter there
 // (l1tex data-pipe 80 % busy at 61 % DRAM, profiles/r1_apply_p4_column.txt).
-template <int P>
-struct SlabCfg
-{
-  static constexpr int n = P + 1;
-  static constexpr int n2 = n * n;
-  static constexpr int tpb = 128;
-  static constexpr int cpb = tpb / n;      // cells per block
-  static constexpr int S = (cpb * n + 1) & ~1; // slots per (batch, ix, iy) row of G
-  static constexpr int SE = (cpb * n + 3) & ~3; // ... and of the dofmap
-  static constexpr int kp = n + (n & 1);   // padded z-row (16-byte rows for double2 loads)
-  static constexpr int su_doubles = cpb * n2 * kp;
-  static constexpr int sf_doubles = 2 * cpb * n * kp;
-  static constexpr size_t smem = (size_t)(su_doubles + sf_doubles) * sizeof(double);
-};
-
-template <int P, int MINB>
-__global__ void __launch_bounds__(SlabCfg<P>::tpb, MINB)
-k_apply_slab(const double* __restrict__ x, double* __restrict__ y, const double* __restrict__ G,
-             const int32_t* __restrict__ enc, const int32_t* __restrict__ perm,
-             const double* __restrict__ kappa, long long batch0, int cell0, int count)
-{
-  using C = SlabCfg<P>;
-  constexpr int n = C::n, n2 = C::n2, CPB = C::cpb, S = C::S, SE = C::SE, KP = C::kp;
-  extern __shared__ __align__(16) double smem[];
-  double* su = smem;                  // [CPB][n2][KP]
-  double* sf = smem + C::su_doubles;  // [2][CPB][n][KP]
-
-  const int tid = threadIdx.x;
-  const int cl = tid / n;
-  const int k = tid - cl * n;
-  const int pl = blockIdx.x * CPB + cl;
-  const bool in_block = cl < CPB;
-  const bool active = in_block && pl < count;
-  const long long gb = batch0 + blockIdx.x;
-  const int32_t* e = enc + gb * (n2 * SE) + tid;
-  const double* g = G + gb * ((long long)n2 * 6 * S) + tid;
-  const int cls = in_block ? cl : 0;
-
-  int d[n2];
-  double u[n2];
-  double kap = 0.0;
-  if (active)
-  {
-#pragma unroll
-    for (int a = 0; a < n2; ++a)
-      d[a] = ldg_stream_i32(e + a * SE);
-    kap = kappa[perm[cell0 + pl]];
-#pragma unroll
-    for (int a = 0; a < n2; ++a)
-    {
-      const int idx = d[a] < 0 ? ~d[a] : d[a];
-      const double xv = x[idx];
-      if (d[a] < 0)
-        y[idx] = xv; // Dirichlet row: y = x (src/laplacian.hpp:273-274)
-      u[a] = d[a] < 0 ? 0.0 : xv;
-    }
-  }
-  else
-  {
-#pragma unroll
-    for (int a = 0; a < n2; ++a)
-      d[a] = -1, u[a] = 0.0;
-  }
-  if (in_block)
-  {
-#pragma unroll
-    for (int a = 0; a < n2; ++a)
-      su[(cl * n2 + a) * KP + k] = u[a];
-  }
-  double Dk[n], DTk[n];
-#pragma unroll
-  for (int l = 0; l < n; ++l)
-  {
-    Dk[l] = c_D[P][k * n + l];
-    DTk[l] = c_D[P][l * n + k];
-  }
-  double acc[n2];
-#pragma unroll
-  for (int a = 0; a < n2; ++a)
-    acc[a] = 0.0;
-  __syncthreads();
-
-#pragma unroll
-  for (int i = 0; i < n; ++i)
-  {
-    double gg[n][6];
-    if (active)
-    {
-#pragma unroll
-      for (int j = 0; j < n; ++j)
-#pragma unroll
-        for (int c = 0; c < 6; ++c)
-          gg[j][c] = ldg_stream(g + ((i * n + j) * 6 + c) * S);
-    }
-    else
-    {
-#pragma unroll
-      for (int j = 0; j < n; ++j)
-#pragma unroll
-        for (int c = 0; c < 6; ++c)
-          gg[j][c] = 0.0;
-    }
-    double fz[n];
-#pragma unroll
-    for (int j = 0; j < n; ++j)
-    {
-      double gx = 0.0, gy = 0.0, gz = 0.0;
-      const double2* row = reinterpret_cast<const double2*>(su + (cls * n2 + i * n + j) * KP);
-#pragma unroll
-      for (int l2 = 0; l2 < KP / 2; ++l2)
-      {
-        const double2 r = row[l2];
-        gz = fma(Dk[2 * l2], r.x, gz);
-        if (2 * l2 + 1 < n)
-          gz = fma(Dk[2 * l2 + 1], r.y, gz);
-      }
-#pragma unroll
-      for (int l = 0; l < n; ++l)
-      {
-        gx = fma(c_D[P][i * n + l], u[l * n + j], gx);
-        gy = fma(c_D[P][j * n + l], u[i * n + l], gy);
-      }
-      const double fx = kap * (gg[j][0] * gx + gg[j][1] * gy + gg[j][2] * gz);
-      const double fy = kap * (gg[j][1] * gx + gg[j][3] * gy + gg[j][4] * gz);
-      fz[j] = kap * (gg[j][2] * gx + gg[j][4] * gy + gg[j][5] * gz);
-#pragma unroll
-      for (int l = 0; l < n; ++l)
-      {
-        acc[l * n + j] = fma(c_D[P][i * n + l], fx, acc[l * n + j]);
-        acc[i * n + l] = fma(c_D[P][j * n + l], fy, acc[i * n + l]);
-      }
-    }
-    double* sfz = sf + (((i & 1) * CPB + cls) * n) * KP;
-    if (in_block)
-    {
-#pragma unroll
-      for (int j = 0; j < n; ++j)
-        sfz[j * KP + k] = fz[j];
-    }
-    __syncthreads();
-#pragma unroll
-    for (int j = 0; j < n; ++j)
-    {
-      const double2* row = reinterpret_cast<const double2*>(sfz + j * KP);
-      double t = 0.0;
-#pragma unroll
-      for (int q2 = 0; q2 < KP / 2; ++q2)
-      {
-        const double2 r = row[q2];
-        t = fma(DTk[2 * q2], r.x, t);
-        if (2 * q2 + 1 < n)
-          t = fma(DTk[2 * q2 + 1], r.y, t);
-      }
-      acc[i * n + j] += t;
-    }
-  }
-  if (active)
-  {
-#pragma unroll
-    for (int a = 0; a < n2; ++a)
-      if (d[a] >= 0)
-        atomicAdd(&y[d[a]], acc[a]);
-  }
-}
-
-template <int P>
-constexpr int slab_minb()
-{
-  return P <= 2 ? 4 : (P == 3 ? 3 : 2);
-}
-
-template <int P>
-void launch_apply_slab(pmgx_ctx* c, cudaStream_t st, const double* x, double* y, const double* G, const int32_t* enc,
-                       const int32_t* perm, const double* kappa, long long batch0, int cell0, int count)
-{
-  const bool timed = c->profiling && cell0 == 0; // per-kernel timing covers the interior-cell launch only
-  if (count <= 0)
-    return;
-  using C = SlabCfg<P>;
-  constexpr int MINB = slab_minb<P>();
-  static bool configured[64] = {false};
-  if (!configured[c->device])
-  {
-    PMGX_CUDA(cudaFuncSetAttribute(k_apply_slab<P, MINB>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                   (int)C::smem));
-    configured[c->device] = true;
-  }
-  const int grid = (count + C::cpb - 1) / C::cpb;
-  cudaEvent_t e0 = nullptr, e1 = nullptr;
-  if (timed)
-  {
-    PMGX_CUDA(cudaEventCreate(&e0));
-    PMGX_CUDA(cudaEventCreate(&e1));
-    PMGX_CUDA(cudaEventRecord(e0, st));
-  }
-  k_apply_slab<P, MINB><<<grid, C::tpb, C::smem, st>>>(x, y, G, enc, perm, kappa, batch0, cell0, count);
-  check_launch("k_apply_slab");
-  count_launch(c);
-  if (timed)
-  {
-    PMGX_CUDA(cudaEventRecord(e1, st));
-    c->prof[P].emplace_back(e0, e1);
-  }
-}
-
-// --------------------------------------------- the TMA-pipelined slab apply kernel --
-// Same thread mapping and arithmetic as k_apply_slab, but the one-shot streams (geometry
-// factors, encoded dofmap) no longer pass through registers with the latency exposed to a
-// handful of resident warps: a persistent CTA walks over its batches and an elected thread
+// The one-shot streams (geometry factors, encoded dofmap) do not pass through registers with
+// the latency exposed to a handful of resident warps: a persistent CTA walks over its batches
+// and an elected thread
 // keeps a ring of R geometry planes (and the next batch's dofmap) in flight with
 // cp.async.bulk (TMA) into shared memory, completion tracked by mbarriers.  Memory-level
 // parallelism is then set by the ring depth, not by occupancy or register count.
@@ -880,12 +750,13 @@ __device__ __forceinline__ void bulk_g2s(void* dst, const void* src, uint32_t by
                : "memory");
 }
 
-template <int P, int TPB, int R>
+template <int P, int TPB>
 struct TmaCfg
 {
   static constexpr int n = P + 1;
   static constexpr int n2 = n * n;
   static constexpr int tpb = TPB;
+  static constexpr int R = 2; // geometry planes in flight (measured on B200: a 2-plane ring wins for P3/P4)
   static constexpr int cpb = tpb / n;
   static constexpr int S = (cpb * n + 1) & ~1;  // G rows: 16-byte multiples, (almost) no padding streamed
   static constexpr int SE = (cpb * n + 3) & ~3; // dofmap rows: 16-byte multiples of int32
@@ -900,23 +771,21 @@ struct TmaCfg
   static constexpr uint32_t enc_bytes = n2 * SE * sizeof(int32_t);
   static constexpr int buf_doubles = 2 * cpb * cs; // double-buffered plane rows (su and sf each)
   static constexpr size_t off_enc = (size_t)R * plane_bytes;
-  // dofmap buffers: double-buffered (read again at scatter time, next batch prefetched meanwhile);
-  // a single buffer at P >= 6, where the saved 12.5 KB let a third CTA (+50 % warps) fit on the SM
-  static constexpr int EB = P >= 6 ? 1 : 2;
-  static constexpr size_t off_su = off_enc + EB * enc_bytes;
+  // dofmap buffers: double-buffered (read again at scatter time, next batch prefetched meanwhile)
+  static constexpr size_t off_su = off_enc + 2 * enc_bytes;
   static constexpr size_t off_sf = off_su + (size_t)buf_doubles * sizeof(double);
   static constexpr size_t off_bar = off_sf + (size_t)buf_doubles * sizeof(double);
   static constexpr size_t smem = off_bar + (R + 2) * sizeof(uint64_t);
 };
 
-template <int P, int TPB, int R>
-__global__ void __launch_bounds__(TPB, TmaCfg<P, TPB, R>::minb)
+template <int P, int TPB>
+__global__ void __launch_bounds__(TPB, TmaCfg<P, TPB>::minb)
 k_apply_tma(const double* __restrict__ x, double* __restrict__ y, const double* __restrict__ G,
             const int32_t* __restrict__ enc, const int32_t* __restrict__ perm,
             const double* __restrict__ kappa, long long batch0, int cell0, int count, int nbatch)
 {
-  using C = TmaCfg<P, TPB, R>;
-  constexpr int n = C::n, n2 = C::n2, CPB = C::cpb, S = C::S, SE = C::SE, KP = C::kp, CS = C::cs;
+  using C = TmaCfg<P, TPB>;
+  constexpr int n = C::n, n2 = C::n2, CPB = C::cpb, S = C::S, SE = C::SE, KP = C::kp, CS = C::cs, R = C::R;
   extern __shared__ __align__(128) unsigned char smraw[];
   double* sG = reinterpret_cast<double*>(smraw);
   const int32_t* sE = reinterpret_cast<const int32_t*>(smraw + C::off_enc);
@@ -954,11 +823,10 @@ k_apply_tma(const double* __restrict__ x, double* __restrict__ y, const double* 
     bulk_g2s(sG + (size_t)s * C::plane_doubles, G + (gb * n2 + (long long)i * n) * 6 * S, C::plane_bytes,
              &fullG[s], pol);
   };
-  constexpr int EB = C::EB;
   auto issue_enc = [&](int it)
   {
     const long long gb = batch0 + blockIdx.x + (long long)it * gridDim.x;
-    const int eb = EB == 2 ? (it & 1) : 0;
+    const int eb = it & 1;
     mbar_expect_tx(&fullE[eb], C::enc_bytes);
     bulk_g2s(const_cast<int32_t*>(sE) + eb * (n2 * SE), enc + gb * (long long)(n2 * SE), C::enc_bytes, &fullE[eb], pol);
   };
@@ -985,8 +853,8 @@ k_apply_tma(const double* __restrict__ x, double* __restrict__ y, const double* 
     const int pl = b * CPB + cl;
     const bool active = in_block && pl < count;
 
-    const int eb = EB == 2 ? (it & 1) : 0;
-    mbar_wait(&fullE[eb], EB == 2 ? (it >> 1) & 1 : it & 1);
+    const int eb = it & 1;
+    mbar_wait(&fullE[eb], (it >> 1) & 1);
     const int32_t* dE = sE + eb * (n2 * SE) + tid; // this thread's n2 encoded dofs
     double u[n2];
     double kap = 0.0;
@@ -1017,7 +885,7 @@ k_apply_tma(const double* __restrict__ x, double* __restrict__ y, const double* 
         su[cl * CS + j * KP + k] = u[j];
     }
     __syncthreads(); // z-rows of plane 0 are visible; the other dofmap buffer (batch it-1) is free
-    if (EB == 2 && tid == 0 && it + 1 < my_nb)
+    if (tid == 0 && it + 1 < my_nb)
       issue_enc(it + 1);
 
     double acc[n2];
@@ -1114,50 +982,21 @@ k_apply_tma(const double* __restrict__ x, double* __restrict__ y, const double* 
           atomicAdd(&y[da], acc[a]);
       }
     }
-    if (EB == 1 && it + 1 < my_nb)
-    {
-      __syncthreads(); // every thread has read its scatter indices: the single dofmap buffer is free
-      if (tid == 0)
-        issue_enc(it + 1);
-    }
   }
 }
 
-template <int P, int TPB, int R>
-void launch_apply_tma_t(pmgx_ctx* c, cudaStream_t st, const double* x, double* y, const double* G, const int32_t* enc,
-                        const int32_t* perm, const double* kappa, long long batch0, int cell0, int count)
+template <int P, int TPB>
+struct TmaApply
 {
-  const bool timed = c->profiling && cell0 == 0; // per-kernel timing covers the interior-cell launch only
-  using C = TmaCfg<P, TPB, R>;
-  static int ctas_per_sm[64] = {0};
-  if (ctas_per_sm[c->device] == 0)
+  using C = TmaCfg<P, TPB>;
+  static constexpr bool cell_geometry = false;
+  static constexpr int cpb = C::cpb;
+  static void name(char* s, int cap) { snprintf(s, cap, "k_apply_tma<%d,%d,%d>", P, TPB, C::R); }
+  static void launch(pmgx_ctx* c, cudaStream_t st, const ApplyArgs& a)
   {
-    PMGX_CUDA(cudaFuncSetAttribute(k_apply_tma<P, TPB, R>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                   (int)C::smem));
-    int nb = 0;
-    PMGX_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, k_apply_tma<P, TPB, R>, TPB, C::smem));
-    PMGX_REQUIRE(nb >= 1, "k_apply_tma<%d,%d,%d> does not fit on an SM", P, TPB, R);
-    ctas_per_sm[c->device] = nb;
+    launch_batched<k_apply_tma<P, TPB>, C>(c, st, a, "k_apply_tma");
   }
-  const int nbatch = (count + C::cpb - 1) / C::cpb;
-  // persistent CTAs: exactly the number that is co-resident, so every SM streams all the time
-  const int grid = std::min(nbatch, ctas_per_sm[c->device] * c->num_sms);
-  cudaEvent_t e0 = nullptr, e1 = nullptr;
-  if (timed)
-  {
-    PMGX_CUDA(cudaEventCreate(&e0));
-    PMGX_CUDA(cudaEventCreate(&e1));
-    PMGX_CUDA(cudaEventRecord(e0, st));
-  }
-  k_apply_tma<P, TPB, R><<<grid, TPB, C::smem, st>>>(x, y, G, enc, perm, kappa, batch0, cell0, count, nbatch);
-  check_launch("k_apply_tma");
-  count_launch(c);
-  if (timed)
-  {
-    PMGX_CUDA(cudaEventRecord(e1, st));
-    c->prof[P].emplace_back(e0, e1);
-  }
-}
+};
 
 // ------------------------------------------------ the affine-geometry apply kernel --
 // On a cell whose trilinear map is affine (every cell of a box / parallelepiped mesh, i.e. all
@@ -1185,10 +1024,7 @@ struct AffCfg
   static constexpr size_t off_sf = off_su + (size_t)buf_doubles * sizeof(double);
   static constexpr size_t off_bar = off_sf + (size_t)buf_doubles * sizeof(double);
   static constexpr size_t smem = off_bar + 2 * sizeof(uint64_t);
-#ifndef PMGX_AFF_MINB_P4
-#define PMGX_AFF_MINB_P4 4
-#endif
-  static constexpr int minb = P <= 2 ? 6 : (TPB <= 64 ? (P == 4 ? PMGX_AFF_MINB_P4 : 4) : 2);
+  static constexpr int minb = P <= 2 ? 6 : (TPB <= 64 ? 4 : 2);
 };
 
 template <int P, int TPB>
@@ -1373,6 +1209,19 @@ k_apply_affine(const double* __restrict__ x, double* __restrict__ y, const doubl
   }
 }
 
+template <int P, int TPB>
+struct AffineApply
+{
+  using C = AffCfg<P, TPB>;
+  static constexpr bool cell_geometry = true;
+  static constexpr int cpb = C::cpb;
+  static void name(char* s, int cap) { snprintf(s, cap, "k_apply_affine<%d,%d>", P, TPB); }
+  static void launch(pmgx_ctx* c, cudaStream_t st, const ApplyArgs& a)
+  {
+    launch_batched<k_apply_affine<P, TPB>, C>(c, st, a, "k_apply_affine");
+  }
+};
+
 // Shuffle variant of the affine kernel: a warp holds 32/n whole cells (lanes beyond that idle), so
 // the z contractions are warp shuffles from the n lanes of the thread's own cell -- no shared-memory
 // rows, no block barrier per plane.  ncu on the shared-memory variant at P4: L1/shared data pipe 78 %
@@ -1540,75 +1389,17 @@ k_apply_affine_shfl(const double* __restrict__ x, double* __restrict__ y, const 
 }
 
 template <int P, int TPB>
-void launch_apply_affine_shfl_t(pmgx_ctx* c, cudaStream_t st, const double* x, double* y, const double* Gc,
-                                const int32_t* enc, const int32_t* perm, const double* kappa, long long batch0,
-                                int cell0, int count)
+struct AffineShflApply
 {
   using C = AffShCfg<P, TPB>;
-  const bool timed = c->profiling && cell0 == 0; // per-kernel timing covers the interior-cell launch only
-  static int ctas_per_sm[64] = {0};
-  if (ctas_per_sm[c->device] == 0)
+  static constexpr bool cell_geometry = true;
+  static constexpr int cpb = C::cpb;
+  static void name(char* s, int cap) { snprintf(s, cap, "k_apply_affine_shfl<%d,%d>", P, TPB); }
+  static void launch(pmgx_ctx* c, cudaStream_t st, const ApplyArgs& a)
   {
-    PMGX_CUDA(cudaFuncSetAttribute(k_apply_affine_shfl<P, TPB>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                   (int)C::smem));
-    int nb = 0;
-    PMGX_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, k_apply_affine_shfl<P, TPB>, TPB, C::smem));
-    PMGX_REQUIRE(nb >= 1, "k_apply_affine_shfl<%d,%d> does not fit on an SM", P, TPB);
-    ctas_per_sm[c->device] = nb;
+    launch_batched<k_apply_affine_shfl<P, TPB>, C>(c, st, a, "k_apply_affine_shfl");
   }
-  const int nbatch = (count + C::cpb - 1) / C::cpb;
-  const int grid = std::min(nbatch, ctas_per_sm[c->device] * c->num_sms);
-  cudaEvent_t e0 = nullptr, e1 = nullptr;
-  if (timed)
-  {
-    PMGX_CUDA(cudaEventCreate(&e0));
-    PMGX_CUDA(cudaEventCreate(&e1));
-    PMGX_CUDA(cudaEventRecord(e0, st));
-  }
-  k_apply_affine_shfl<P, TPB><<<grid, TPB, C::smem, st>>>(x, y, Gc, enc, perm, kappa, batch0, cell0, count, nbatch);
-  check_launch("k_apply_affine_shfl");
-  count_launch(c);
-  if (timed)
-  {
-    PMGX_CUDA(cudaEventRecord(e1, st));
-    c->prof[P].emplace_back(e0, e1);
-  }
-}
-
-template <int P, int TPB>
-void launch_apply_affine_t(pmgx_ctx* c, cudaStream_t st, const double* x, double* y, const double* Gc,
-                           const int32_t* enc, const int32_t* perm, const double* kappa, long long batch0, int cell0,
-                           int count)
-{
-  using C = AffCfg<P, TPB>;
-  const bool timed = c->profiling && cell0 == 0; // per-kernel timing covers the interior-cell launch only
-  static int ctas_per_sm[64] = {0};
-  if (ctas_per_sm[c->device] == 0)
-  {
-    PMGX_CUDA(cudaFuncSetAttribute(k_apply_affine<P, TPB>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C::smem));
-    int nb = 0;
-    PMGX_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, k_apply_affine<P, TPB>, TPB, C::smem));
-    PMGX_REQUIRE(nb >= 1, "k_apply_affine<%d,%d> does not fit on an SM", P, TPB);
-    ctas_per_sm[c->device] = nb;
-  }
-  const int nbatch = (count + C::cpb - 1) / C::cpb;
-  const int grid = std::min(nbatch, ctas_per_sm[c->device] * c->num_sms);
-  cudaEvent_t e0 = nullptr, e1 = nullptr;
-  if (timed)
-  {
-    PMGX_CUDA(cudaEventCreate(&e0));
-    PMGX_CUDA(cudaEventCreate(&e1));
-    PMGX_CUDA(cudaEventRecord(e0, st));
-  }
-  k_apply_affine<P, TPB><<<grid, TPB, C::smem, st>>>(x, y, Gc, enc, perm, kappa, batch0, cell0, count, nbatch);
-  check_launch("k_apply_affine");
-  count_launch(c);
-  if (timed)
-  {
-    PMGX_CUDA(cudaEventRecord(e1, st));
-    c->prof[P].emplace_back(e0, e1);
-  }
-}
+};
 
 
 // ---------------------------------------- the re-slabbed affine-geometry apply kernel --
@@ -1623,21 +1414,21 @@ void launch_apply_affine_t(pmgx_ctx* c, cudaStream_t st, const double* x, double
 //                         x and y transposed contractions into the register accumulator
 //   3. fz(i,j,t)       -> thread j reads fz(i,j,.) and forms az(i,j,l) = sum_q D[q][l] fz(i,j,q)
 //   4. az(i,j,l)       -> thread l adds az(.,.,l) to its accumulator
-// 8 n^2 doubles per thread instead of 2 n^3 + 2 n^2 (P4: 200 vs 300; P6: 392 vs 784), four barriers
-// per batch instead of n + 1, and no broadcast reads.  Strides: slab stride SS = 1 (mod 16) and cell
+// 8 n^2 doubles per thread instead of 2 n^3 + 2 n^2 (P4: 200 vs 300; P6: 392 vs 784), no broadcast
+// reads, and one CTA barrier per batch instead of n + 1: a warp holds 32 / n WHOLE cells (the lanes
+// beyond that idle), so every exchange stays inside a warp and the phases are separated by
+// __syncwarp(): the warps of a CTA run free of each other (with 8-10 warps per SM a CTA barrier per
+// phase leaves the schedulers empty).  Strides: slab stride SS = 1 (mod 16) and cell
 // stride CS = n (mod 16) doubles make the 8-byte bank of BOTH access patterns (unit stride in t when
 // writing, stride SS in t when reading) equal to lane + const: every 64-bit access is conflict-free.
-template <int P, int TPB, bool WL>
+template <int P, int TPB>
 struct Aff2Cfg
 {
   static constexpr int n = P + 1;
   static constexpr int n2 = n * n;
   static constexpr int tpb = TPB;
-  // WL (warp-local): a warp holds 32 / n WHOLE cells (the lanes beyond that idle), so every exchange stays
-  // inside a warp and the phases are separated by __syncwarp() instead of CTA barriers: the warps of a CTA
-  // run free of each other (with 8-10 warps per SM a CTA barrier per phase leaves the schedulers empty)
-  static constexpr int cpw = 32 / n;
-  static constexpr int cpb = WL ? (TPB / 32) * cpw : TPB / n;
+  static constexpr int cpw = 32 / n;               // cells per warp
+  static constexpr int cpb = (TPB / 32) * cpw;     // cells per batch
   static constexpr int SE = (cpb * n + 3) & ~3;
   static constexpr int ss = ((n2 - 1 + 15) / 16) * 16 + 1;                 // >= n2, = 1 mod 16
   static constexpr int cs = ((n * ss - n + 15) / 16) * 16 + n;             // >= n * ss, = n mod 16
@@ -1647,16 +1438,16 @@ struct Aff2Cfg
   static constexpr size_t off_b = off_a + (size_t)buf_doubles * sizeof(double);
   static constexpr size_t off_bar = off_b + (size_t)buf_doubles * sizeof(double);
   static constexpr size_t smem = off_bar + 2 * sizeof(uint64_t);
-  static constexpr int minb = P <= 2 ? 6 : (P == 4 && TPB <= 64 ? PMGX_AFF_MINB_P4 : (P <= 4 ? 4 : 2));
+  static constexpr int minb = P <= 2 ? 6 : (P <= 4 ? 4 : 2);
 };
 
-template <int P, int TPB, bool WL>
-__global__ void __launch_bounds__(TPB, Aff2Cfg<P, TPB, WL>::minb)
+template <int P, int TPB>
+__global__ void __launch_bounds__(TPB, Aff2Cfg<P, TPB>::minb)
 k_apply_affine2(const double* __restrict__ x, double* __restrict__ y, const double* __restrict__ Gc,
                 const int32_t* __restrict__ enc, const int32_t* __restrict__ perm,
                 const double* __restrict__ kappa, long long batch0, int cell0, int count, int nbatch)
 {
-  using C = Aff2Cfg<P, TPB, WL>;
+  using C = Aff2Cfg<P, TPB>;
   constexpr int n = C::n, n2 = C::n2, CPB = C::cpb, SE = C::SE, SS = C::ss, CS = C::cs;
   extern __shared__ __align__(128) unsigned char smraw[];
   const int32_t* sE = reinterpret_cast<const int32_t*>(smraw);
@@ -1665,32 +1456,14 @@ k_apply_affine2(const double* __restrict__ x, double* __restrict__ y, const doub
   uint64_t* fullE = reinterpret_cast<uint64_t*>(smraw + C::off_bar);
 
   const int tid = threadIdx.x;
-  int cl, t;
-  bool in_block;
-  if (WL)
-  {
-    const int warp = tid >> 5, lane = tid & 31;
-    const int cw = lane / n;
-    in_block = cw < C::cpw;
-    cl = warp * C::cpw + (in_block ? cw : 0);
-    t = in_block ? lane - cw * n : 0;
-  }
-  else
-  {
-    cl = tid / n;
-    t = tid - cl * n;
-    in_block = cl < CPB;
-  }
+  const int warp = tid >> 5, lane = tid & 31;
+  const int cw = lane / n;
+  const bool in_block = cw < C::cpw;
+  const int cl = warp * C::cpw + (in_block ? cw : 0);
+  const int t = in_block ? lane - cw * n : 0;
   const int cls = in_block ? cl : 0;
-  const int slot = WL ? cls * n + t : tid;
+  const int slot = cls * n + t;
   const int my_nb = ((int)blockIdx.x < nbatch) ? (nbatch - (int)blockIdx.x + (int)gridDim.x - 1) / (int)gridDim.x : 0;
-  auto phase_sync = [&]()
-  {
-    if (WL)
-      __syncwarp();
-    else
-      __syncthreads();
-  };
 
   uint64_t pol = 0;
   if (tid == 0)
@@ -1724,13 +1497,10 @@ k_apply_affine2(const double* __restrict__ x, double* __restrict__ y, const doub
     const int pl = b * CPB + cl;
     const bool active = in_block && pl < count;
 
-    if (WL)
-    {
-      // the only CTA barrier of a batch: every warp is done with the dofmap buffer the next load will overwrite
-      __syncthreads();
-      if (tid == 0 && it + 1 < my_nb)
-        issue_enc(it + 1);
-    }
+    // the only CTA barrier of a batch: every warp is done with the dofmap buffer the next load will overwrite
+    __syncthreads();
+    if (tid == 0 && it + 1 < my_nb)
+      issue_enc(it + 1);
     mbar_wait(&fullE[it & 1], (it >> 1) & 1);
     const int32_t* dE = sE + (it & 1) * (n2 * SE) + slot;
     double u[n2];
@@ -1771,9 +1541,7 @@ k_apply_affine2(const double* __restrict__ x, double* __restrict__ y, const doub
         for (int j = 0; j < n; ++j)
           wA[j * SS + i * n] = u[i * n + j];
     }
-    phase_sync(); // (CTA-wide variant: every thread is also past the previous batch's reads of B and of the other dofmap buffer)
-    if (!WL && tid == 0 && it + 1 < my_nb)
-      issue_enc(it + 1);
+    __syncwarp();
     // phase 2: slab j = t: gz(i,t,l) = sum_m D[l][m] u(i,t,m) -> B[slab l][i][t]
 #pragma unroll
     for (int i = 0; i < n; ++i)
@@ -1793,7 +1561,7 @@ k_apply_affine2(const double* __restrict__ x, double* __restrict__ y, const doub
           wB[l * SS + i * n] = s;
       }
     }
-    phase_sync();
+    __syncwarp();
     // phase 3: all three gradients at the points (i,j,t); transform; x / y transposed contractions;
     // fz(i,j,t) -> A[slab j][i][t]
     double acc[n2];
@@ -1826,7 +1594,7 @@ k_apply_affine2(const double* __restrict__ x, double* __restrict__ y, const doub
         if (in_block)
           wA[j * SS + i * n] = fz;
       }
-    phase_sync();
+    __syncwarp();
     // phase 4: slab j = t: az(i,t,l) = sum_q D[q][l] fz(i,t,q) -> B[slab l][i][t]
 #pragma unroll
     for (int i = 0; i < n; ++i)
@@ -1846,7 +1614,7 @@ k_apply_affine2(const double* __restrict__ x, double* __restrict__ y, const doub
           wB[l * SS + i * n] = s;
       }
     }
-    phase_sync();
+    __syncwarp();
     // phase 5: acc(i,j,t) += az(i,j,t); scatter
     if (active)
     {
@@ -1858,100 +1626,81 @@ k_apply_affine2(const double* __restrict__ x, double* __restrict__ y, const doub
           atomicAdd(&y[da], acc[a] + rB[a]);
       }
     }
-    if (WL)
-      __syncwarp(); // B is rewritten in the next batch's phase 2 only after this warp's reads above
+    __syncwarp(); // B is rewritten in the next batch's phase 2 only after this warp's reads above
   }
 }
 
-template <int P, int TPB, bool WL>
-void launch_apply_affine2_t(pmgx_ctx* c, cudaStream_t st, const double* x, double* y, const double* Gc,
-                            const int32_t* enc, const int32_t* perm, const double* kappa, long long batch0, int cell0,
-                            int count)
+template <int P, int TPB>
+struct Affine2Apply
 {
-  using C = Aff2Cfg<P, TPB, WL>;
-  const bool timed = c->profiling && cell0 == 0; // per-kernel timing covers the interior-cell launch only
-  static int ctas_per_sm[64] = {0};
-  if (ctas_per_sm[c->device] == 0)
+  using C = Aff2Cfg<P, TPB>;
+  static constexpr bool cell_geometry = true;
+  static constexpr int cpb = C::cpb;
+  static void name(char* s, int cap) { snprintf(s, cap, "k_apply_affine2<%d,%d,warp-local>", P, TPB); }
+  static void launch(pmgx_ctx* c, cudaStream_t st, const ApplyArgs& a)
   {
-    PMGX_CUDA(cudaFuncSetAttribute(k_apply_affine2<P, TPB, WL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C::smem));
-    int nb = 0;
-    PMGX_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, k_apply_affine2<P, TPB, WL>, TPB, C::smem));
-    PMGX_REQUIRE(nb >= 1, "k_apply_affine2<%d,%d> does not fit on an SM", P, TPB);
-    ctas_per_sm[c->device] = nb;
+    launch_batched<k_apply_affine2<P, TPB>, C>(c, st, a, "k_apply_affine2");
   }
-  const int nbatch = (count + C::cpb - 1) / C::cpb;
-  const int grid = std::min(nbatch, ctas_per_sm[c->device] * c->num_sms);
-  cudaEvent_t e0 = nullptr, e1 = nullptr;
-  if (timed)
-  {
-    PMGX_CUDA(cudaEventCreate(&e0));
-    PMGX_CUDA(cudaEventCreate(&e1));
-    PMGX_CUDA(cudaEventRecord(e0, st));
-  }
-  k_apply_affine2<P, TPB, WL><<<grid, TPB, C::smem, st>>>(x, y, Gc, enc, perm, kappa, batch0, cell0, count, nbatch);
-  check_launch("k_apply_affine2");
-  count_launch(c);
-  if (timed)
-  {
-    PMGX_CUDA(cudaEventRecord(e1, st));
-    c->prof[P].emplace_back(e0, e1);
-  }
-}
-
-template <int P>
-void launch_apply_affine(pmgx_ctx* c, cudaStream_t st, bool shfl, int tpb, const double* x, double* y,
-                         const double* Gc, const int32_t* enc, const int32_t* perm, const double* kappa,
-                         long long batch0, int cell0, int count, int reslab = 0)
-{
-  if (count <= 0)
-    return;
-  // reslab: 1 = CTA-wide phases (batch layout of k_apply_affine), 2 = warp-local phases (batch layout of the shuffle kernel)
-  if (reslab == 2 && tpb == 64)
-    return launch_apply_affine2_t<P, 64, true>(c, st, x, y, Gc, enc, perm, kappa, batch0, cell0, count);
-  if (reslab == 2)
-    return launch_apply_affine2_t<P, 128, true>(c, st, x, y, Gc, enc, perm, kappa, batch0, cell0, count);
-  if (reslab && tpb == 64)
-    return launch_apply_affine2_t<P, 64, false>(c, st, x, y, Gc, enc, perm, kappa, batch0, cell0, count);
-  if (reslab)
-    return launch_apply_affine2_t<P, 128, false>(c, st, x, y, Gc, enc, perm, kappa, batch0, cell0, count);
-  if (shfl && tpb == 64)
-    return launch_apply_affine_shfl_t<P, 64>(c, st, x, y, Gc, enc, perm, kappa, batch0, cell0, count);
-  if (shfl)
-    return launch_apply_affine_shfl_t<P, 128>(c, st, x, y, Gc, enc, perm, kappa, batch0, cell0, count);
-  if (tpb == 64)
-    return launch_apply_affine_t<P, 64>(c, st, x, y, Gc, enc, perm, kappa, batch0, cell0, count);
-  return launch_apply_affine_t<P, 128>(c, st, x, y, Gc, enc, perm, kappa, batch0, cell0, count);
-}
-
-// default tuning (threads per CTA, geometry planes in flight); PMGX_TMA_TPB / PMGX_TMA_R override
-// (measured on B200, scripts/sweep_tma.sh: more, smaller CTAs with a 2-plane ring win for P3/P4)
-inline int tma_default_tpb(int P) { return (P == 1 || P >= 5) ? 64 : 128; }
-inline int tma_default_r(int P) { return 2; }
-// affine kernel (no geometry ring, so more small CTAs fit): measured at 100 M dofs, P1 3.45 vs 4.07 ms
-// (128 vs 64 threads), P2 1.67 vs 1.79, P3 1.61 vs 1.54, P4 1.34 vs 1.28, P5 1.20 vs 1.19, P6 2.06 vs 2.03
-inline int affine_default_tpb(int P) { return P <= 2 ? 128 : 64; } // (P3 re-slab kernel: 1.201 / 1.202 ms at 64 / 128)
-
-template <int P>
-void launch_apply_tma(pmgx_ctx* c, cudaStream_t st, int tpb, int r, const double* x, double* y, const double* G,
-                      const int32_t* enc, const int32_t* perm, const double* kappa, long long batch0, int cell0,
-                      int count)
-{
-  if (count <= 0)
-    return;
-#define PMGX_TMA_CASE(T, RR)                                                                       \
-  if (tpb == T && r == RR)                                                                         \
-    return launch_apply_tma_t<P, T, RR>(c, st, x, y, G, enc, perm, kappa, batch0, cell0, count);
-  PMGX_TMA_CASE(128, 2)
-  PMGX_TMA_CASE(128, 3)
-  PMGX_TMA_CASE(64, 2)
-  PMGX_TMA_CASE(64, 3)
-  PMGX_TMA_CASE(64, 4)
-#undef PMGX_TMA_CASE
-  set_error("unsupported TMA kernel configuration tpb=%d r=%d", tpb, r);
-  throw Error{PMGX_ERR_ARG};
-}
+};
 
 #include "laplacian_mma.cuh"
+
+// ------------------------------------------------------------- the kernel per degree --
+// Affine: every cell of the operator passed the affinity test at create (k_cell_geometry); Streamed: G per
+// quadrature point (any non-affine cell, or PMGX_LAP_STREAM_G).  The choices were measured at 100 M dofs:
+// * threads per CTA of the affine slab kernels, 128 vs 64: P1 3.45 vs 4.07 ms, P2 1.67 vs 1.79, P3 1.61 vs 1.54,
+//   P4 1.34 vs 1.28, P5 1.20 vs 1.19, P6 2.06 vs 2.03 (P3 re-slab kernel: 1.201 / 1.202 ms at 64 / 128);
+// * z contraction by warp shuffles (k_apply_affine_shfl) vs shared-memory rows: P1 3.52 vs 3.45 ms, P2 1.58 vs
+//   1.67, P3 1.63 vs 1.54, P4 1.36 vs 1.28, P5 1.57 vs 1.19, P6 2.27 vs 2.03 -- double shuffles cost two issue
+//   slots each and only pay where the element is small;
+// * re-slabbed z direction (k_apply_affine2) vs broadcast rows: P1 4.16 vs 3.44 ms, P2 1.76 vs 1.58, P3 1.20 vs
+//   1.54, P4 1.41 vs 1.28, P5 2.40 vs 1.19, P6 3.09 vs 2.03: it halves the shared-memory wavefronts (ncu: L1/shared
+//   pipe 78 -> 53 %) but both kernels sit at 2 warps per scheduler with fixed-latency (DFMA dependency) stalls on
+//   top, so it only wins where its register count drops far enough to matter (P3);
+// * streamed G: threads per CTA of k_apply_tma, the winners of a sweep over {64, 128} threads x {2, 3, 4}
+//   geometry planes in flight on a B200;
+// * P6 / P7: the FP64 tensor-core kernel against the slab kernels, see laplacian_mma.cuh;
+// * P8: the column kernel; the slab kernels keep 2 (P+1)^2 doubles in registers per thread (measured: P7 53 % vs
+//   47 %, P8 24 % vs 27 %) and n = 9 fits no 8-wide tensor-core tile.  It has no affine variant, so the affinity
+//   test is skipped and is_affine() stays 0.
+template <int P>
+struct ApplyKernels;
+template <> struct ApplyKernels<1> { using Affine = AffineApply<1, 128>;     using Streamed = TmaApply<1, 64>; };
+template <> struct ApplyKernels<2> { using Affine = AffineShflApply<2, 128>; using Streamed = TmaApply<2, 128>; };
+template <> struct ApplyKernels<3> { using Affine = Affine2Apply<3, 64>;     using Streamed = TmaApply<3, 128>; };
+template <> struct ApplyKernels<4> { using Affine = AffineApply<4, 64>;      using Streamed = TmaApply<4, 128>; };
+template <> struct ApplyKernels<5> { using Affine = AffineApply<5, 64>;      using Streamed = TmaApply<5, 64>; };
+template <> struct ApplyKernels<6> { using Affine = MmaApply<6, false>;      using Streamed = MmaApply<6, true>; };
+template <> struct ApplyKernels<7> { using Affine = MmaApply<7, false>;      using Streamed = MmaApply<7, true>; };
+template <> struct ApplyKernels<8> { using Affine = ColumnApply<8>;          using Streamed = ColumnApply<8>; };
+
+// f(K{}) with K the launcher of the apply kernel of degree P (Affine if `affine`, else Streamed)
+template <typename F>
+void with_apply_kernel(int P, bool affine, F&& f)
+{
+  const auto pick = [&](auto deg)
+  {
+    using K = ApplyKernels<decltype(deg)::value>;
+    if (affine)
+      f(typename K::Affine{});
+    else
+      f(typename K::Streamed{});
+  };
+  switch (P)
+  {
+  case 1: return pick(std::integral_constant<int, 1>{});
+  case 2: return pick(std::integral_constant<int, 2>{});
+  case 3: return pick(std::integral_constant<int, 3>{});
+  case 4: return pick(std::integral_constant<int, 4>{});
+  case 5: return pick(std::integral_constant<int, 5>{});
+  case 6: return pick(std::integral_constant<int, 6>{});
+  case 7: return pick(std::integral_constant<int, 7>{});
+  case 8: return pick(std::integral_constant<int, 8>{});
+  default:
+    set_error("Unsupported degree");
+    throw Error{PMGX_ERR_UNSUPPORTED};
+  }
+}
 
 void upload_tables(pmgx_ctx* c)
 {
@@ -1998,107 +1747,36 @@ struct Laplacian : pmgx_operator
   DevBuf<int32_t> enc;  // BC-encoded dofmap, layout `lay`
   DevBuf<double> G;     // geometry factors, layout `lay`
   Lay lay;
-  int tma_tpb = 128, tma_r = 2;
-  bool use_tma = true; // TMA-pipelined slab kernel (default); PMGX_APPLY_KERNEL=slab|column for A/B runs
   DevBuf<double> Gc;   // [n_list][6] per-cell geometry factor of affine cells
-  bool affine = false; // every cell affine: k_apply_affine replaces the streamed-G kernels
-  bool aff_shfl = false; // z contractions by warp shuffles instead of shared-memory rows (default for P <= 2)
-  int aff_reslab = 0; // re-slabbed z direction (k_apply_affine2): 1 CTA-wide phases, 2 warp-local phases
-  bool use_mma = false; // P6 / P7: FP64 tensor-core kernel (k_apply_affine_mma; G per cell if affine, else streamed), plain [p][n3] layout
+  bool affine = false; // every cell affine: ApplyKernels<P>::Affine replaces the streamed-G kernel
 
   int n_list() const { return n_l + n_b; }
 
-  template <int PP>
-  void apply_t(double* x, double* y)
+  void apply(double* x, double* y) override
   {
+    cudaSetDevice(ctx->device);
     const long long ntot = (long long)n_owned + n_ghost;
     vec::set(ctx, y, ntot, 0.0); // out.set(0) :466 (fill kernel, see vec::set)
     if (halo)
       halo_fwd_begin(halo, x);                                                    // :378
     // interior cells on the compute stream; boundary + ghost cells right behind the exchange on
     // the halo stream: they start when the ghosts are in place and fill the interior kernel's tail
-    // (both only add into y, which was zeroed before the exchange started)
-    static const bool on_compute = getenv("PMGX_BOUNDARY_ON_COMPUTE") != nullptr; // A/B switch
-    // measured at 4 GPUs (scripts/ab_apply_mgpu.py): riding the halo stream wins at P1 (0.114 vs
-    // 0.121 ms), is neutral at P2 and loses 2 % at P4, where the interior kernel is long enough to
-    // hide the join anyway
-    const bool side = halo && !on_compute && PP <= 2;
-    cudaStream_t cs = ctx->stream, bs = side ? halo_stream(halo, ctx) : ctx->stream;
-    auto join_before_boundary = [&]()
+    // (both only add into y, which was zeroed before the exchange started).  Measured at 4 GPUs:
+    // riding the halo stream wins at P1 (0.114 vs 0.121 ms), is neutral at P2 and loses 2 % at P4,
+    // where the interior kernel is long enough to hide the join anyway
+    const bool side = halo && P <= 2;
+    cudaStream_t bs = side ? halo_stream(halo, ctx) : ctx->stream;
+    with_apply_kernel(P, affine, [&](auto k)
     {
+      using K = decltype(k);
+      const double* geom = K::cell_geometry ? Gc.p : G.p;
+      K::launch(ctx, ctx->stream, {x, y, geom, enc.p, perm.p, kappa, 0, 0, n_l}); // :406-409
       if (halo && !side)
         halo_fwd_end(halo, x); // reference order: wait for the ghosts, then the boundary launch (:425)
-    };
-    bool done = false;
-    if constexpr (PP == 6 || PP == 7)
-    {
-      if (use_mma)
-      {
-        if (affine)
-          launch_apply_affine_mma<PP, false>(ctx, cs, x, y, Gc.p, enc.p, perm.p, kappa, 0, n_l);
-        else
-          launch_apply_affine_mma<PP, true>(ctx, cs, x, y, G.p, enc.p, perm.p, kappa, 0, n_l);
-        join_before_boundary();
-        if (affine)
-          launch_apply_affine_mma<PP, false>(ctx, bs, x, y, Gc.p, enc.p, perm.p, kappa, n_l, n_b);
-        else
-          launch_apply_affine_mma<PP, true>(ctx, bs, x, y, G.p, enc.p, perm.p, kappa, n_l, n_b);
-        done = true;
-      }
-    }
-    if constexpr (PP <= SLAB_MAX_DEGREE)
-    {
-      if (done)
-        ;
-      else if (lay.mode == 1 && affine)
-      {
-        launch_apply_affine<PP>(ctx, cs, aff_shfl, tma_tpb, x, y, Gc.p, enc.p, perm.p, kappa, 0, 0, n_l, aff_reslab);
-        join_before_boundary();
-        launch_apply_affine<PP>(ctx, bs, aff_shfl, tma_tpb, x, y, Gc.p, enc.p, perm.p, kappa, lay.nb_l, n_l, n_b, aff_reslab);
-        done = true;
-      }
-      else if (lay.mode == 1 && use_tma)
-      {
-        launch_apply_tma<PP>(ctx, cs, tma_tpb, tma_r, x, y, G.p, enc.p, perm.p, kappa, 0, 0, n_l); // :406-409
-        join_before_boundary();
-        launch_apply_tma<PP>(ctx, bs, tma_tpb, tma_r, x, y, G.p, enc.p, perm.p, kappa, lay.nb_l, n_l, n_b); // :449-452
-        done = true;
-      }
-      else if (lay.mode == 1)
-      {
-        launch_apply_slab<PP>(ctx, cs, x, y, G.p, enc.p, perm.p, kappa, 0, 0, n_l);
-        join_before_boundary();
-        launch_apply_slab<PP>(ctx, bs, x, y, G.p, enc.p, perm.p, kappa, lay.nb_l, n_l, n_b);
-        done = true;
-      }
-    }
-    if (!done)
-    {
-      launch_apply<PP>(ctx, cs, x, y, G.p, enc.p, perm.p, kappa, 0, n_l);
-      join_before_boundary();
-      launch_apply<PP>(ctx, bs, x, y, G.p, enc.p, perm.p, kappa, n_l, n_b);
-    }
+      K::launch(ctx, bs, {x, y, geom, enc.p, perm.p, kappa, lay.nb_l, n_l, n_b}); // :449-452
+    });
     if (side)
       halo_fwd_end(halo, x);                                                      // :425 (join)
-  }
-
-  void apply(double* x, double* y) override
-  {
-    cudaSetDevice(ctx->device);
-    switch (P)
-    {
-    case 1: apply_t<1>(x, y); break;
-    case 2: apply_t<2>(x, y); break;
-    case 3: apply_t<3>(x, y); break;
-    case 4: apply_t<4>(x, y); break;
-    case 5: apply_t<5>(x, y); break;
-    case 6: apply_t<6>(x, y); break;
-    case 7: apply_t<7>(x, y); break;
-    case 8: apply_t<8>(x, y); break;
-    default:
-      set_error("Unsupported degree");
-      throw Error{PMGX_ERR_UNSUPPORTED};
-    }
   }
 };
 } // namespace pmgx
@@ -2164,18 +1842,11 @@ int pmgx_laplacian_create(pmgx_ctx* ctx, int degree, int n_cells, const int32_t*
   pmgx::Lay& lay = L->lay;
   lay.n = n, lay.n2 = n * n, lay.n3 = L->n3;
   lay.n_l = n_lcells;
-  const char* force = getenv("PMGX_APPLY_KERNEL"); // "column" forces the column kernel (A/B runs)
-  lay.mode = (degree <= pmgx::SLAB_MAX_DEGREE && !(force && std::strcmp(force, "column") == 0)) ? 1 : 0;
-  // P6 / P7: the tensor-core kernel, with G per cell on affine meshes and G streamed per quadrature point
-  // otherwise (PMGX_APPLY_MMA=0: the slab / column kernels)
-  const bool mma_ok = (degree == 6 || degree == 7) && !force
-                      && !(getenv("PMGX_APPLY_MMA") && atoi(getenv("PMGX_APPLY_MMA")) == 0);
-  L->use_mma = mma_ok;
-  if (mma_ok)
-    lay.mode = 0; // plain enc[p][n3] / G[p][6][n3]
-  // affine cells: one geometry 6-vector per cell instead of one per quadrature point (decided
-  // first: the batch layout follows the kernel that will run)
-  if (n_list > 0 && (degree <= pmgx::SLAB_MAX_DEGREE || mma_ok) && !force && !(flags & PMGX_LAP_STREAM_G))
+  // affine cells: one geometry 6-vector per cell instead of one per quadrature point, for the degrees
+  // that have a kernel for it (decided first: the layout follows the kernel that will run)
+  bool has_affine_kernel = false;
+  pmgx::with_apply_kernel(degree, true, [&](auto k) { has_affine_kernel = decltype(k)::cell_geometry; });
+  if (n_list > 0 && has_affine_kernel && !(flags & PMGX_LAP_STREAM_G))
   {
     L->Gc.alloc((size_t)n_list * 6);
     pmgx::DevBuf<int> bad;
@@ -2191,43 +1862,16 @@ int pmgx_laplacian_create(pmgx_ctx* ctx, int degree, int n_cells, const int32_t*
     L->affine = n_bad == 0;
     if (!L->affine)
       L->Gc.release();
-    if (degree > pmgx::SLAB_MAX_DEGREE && !L->use_mma)
-    {
-      L->affine = false; // no affine kernel above the slab degrees
-      L->Gc.release();
-    }
   }
-  L->use_tma = !(force && std::strcmp(force, "slab") == 0);
-  L->tma_tpb = L->affine ? pmgx::affine_default_tpb(degree) : pmgx::tma_default_tpb(degree);
-  L->tma_r = pmgx::tma_default_r(degree);
-  if (const char* e = getenv("PMGX_TMA_TPB"))
-    L->tma_tpb = atoi(e);
-  if (const char* e = getenv("PMGX_TMA_R"))
-    L->tma_r = atoi(e);
-  if (!L->use_tma)
-    L->tma_tpb = 128;
-  PMGX_REQUIRE(L->tma_tpb == 64 || L->tma_tpb == 128, "PMGX_TMA_TPB must be 64 or 128");
-  // measured at 100 M dofs (shuffle vs shared-memory z contraction): P1 3.52 vs 3.45 ms, P2 1.58 vs 1.67,
-  // P3 1.63 vs 1.54, P4 1.36 vs 1.28, P5 1.57 vs 1.19, P6 2.27 vs 2.03 -- double shuffles cost two issue
-  // slots each and only pay where the element is small
-  L->aff_shfl = degree == 2;
-  if (const char* e = getenv("PMGX_AFFINE_SHFL"))
-    L->aff_shfl = atoi(e) != 0;
-  // re-slabbed z direction (k_apply_affine2, warp-local phases): measured at 100 M dofs against the broadcast-row
-  // kernel -- P1 4.16 vs 3.44 ms, P2 1.76 vs 1.58, P3 1.20 vs 1.54, P4 1.41 vs 1.28, P5 2.40 vs 1.19, P6 3.09 vs 2.03:
-  // it halves the shared-memory wavefronts (ncu: L1/shared pipe 78 -> 53 %) but both kernels sit at 2 warps per
-  // scheduler with fixed-latency (DFMA dependency) stalls on top, so it only wins where its register count drops
-  // far enough to matter (P3)
-  L->aff_reslab = degree == 3 ? 2 : 0;
-  if (const char* e = getenv("PMGX_AFFINE_RESLAB"))
-    L->aff_reslab = atoi(e);
-  if (L->aff_reslab)
-    L->aff_shfl = false;
-  lay.cpb = (L->affine && (L->aff_shfl || L->aff_reslab == 2)) ? (L->tma_tpb / 32) * (32 / n) : L->tma_tpb / n;
-  lay.S = (lay.cpb * n + 1) & ~1;
-  lay.SE = (lay.cpb * n + 3) & ~3;
-  lay.nb_l = (n_lcells + lay.cpb - 1) / lay.cpb;
-  lay.n_batches = lay.nb_l + (n_bcells + lay.cpb - 1) / lay.cpb;
+  pmgx::with_apply_kernel(degree, L->affine, [&](auto k) { lay.cpb = decltype(k)::cpb; });
+  lay.mode = lay.cpb > 0 ? 1 : 0;
+  if (lay.mode == 1)
+  {
+    lay.S = (lay.cpb * n + 1) & ~1;
+    lay.SE = (lay.cpb * n + 3) & ~3;
+    lay.nb_l = (n_lcells + lay.cpb - 1) / lay.cpb;
+    lay.n_batches = lay.nb_l + (n_bcells + lay.cpb - 1) / lay.cpb;
+  }
   const long long enc_size = lay.mode == 1 ? lay.enc_size() : total;
   const long long g_size = lay.mode == 1 ? lay.g_size() : total * 6;
   L->enc.alloc((size_t)enc_size);
@@ -2300,17 +1944,7 @@ int pmgx_laplacian_kernel_name(pmgx_operator* op, char* name_h, int cap)
   PMGX_API_BEGIN
   PMGX_REQUIRE(op && op->kind == pmgx_operator::LAPLACIAN && name_h && cap > 0, "laplacian_kernel_name: bad arguments");
   auto* L = static_cast<Laplacian*>(op);
-  if (L->use_mma)
-    snprintf(name_h, cap, "k_apply_affine_mma<%d,2,%s>", L->P, L->affine ? "affine" : "streamed");
-  else if (L->lay.mode == 1 && L->affine)
-    snprintf(name_h, cap, "%s<%d,%d%s>", L->aff_reslab ? "k_apply_affine2" : (L->aff_shfl ? "k_apply_affine_shfl" : "k_apply_affine"),
-             L->P, L->tma_tpb, L->aff_reslab == 2 ? ",warp-local" : "");
-  else if (L->lay.mode == 1 && L->use_tma)
-    snprintf(name_h, cap, "k_apply_tma<%d,%d,%d>", L->P, L->tma_tpb, L->tma_r);
-  else if (L->lay.mode == 1)
-    snprintf(name_h, cap, "k_apply_slab<%d>", L->P);
-  else
-    snprintf(name_h, cap, "k_apply<%d>", L->P);
+  pmgx::with_apply_kernel(L->P, L->affine, [&](auto k) { decltype(k)::name(name_h, cap); });
   PMGX_API_END
 }
 

@@ -53,13 +53,13 @@ struct MmaCfg
 
 // STREAM = false: Gc[p][6], one geometry 6-vector per (affine) cell, quadrature weights applied here;
 // STREAM = true : Gc = G[p][6][n3], the reference's data flow (G per quadrature point, weights folded in),
-//                 read in layout Y one tile ahead of the flux that uses it, the whole block of the NEXT cell
-//                 prefetched into L2 while this one is computed
+//                 read in layout Y one tile ahead of the flux that uses it; at P6 the cell's whole block is
+//                 prefetched into L2 first
 template <int P, int WPB, int MINB, bool STREAM>
 __global__ void __launch_bounds__(WPB * 32, MINB)
 k_apply_affine_mma(const double* __restrict__ x, double* __restrict__ y, const double* __restrict__ Gc,
                    const int32_t* __restrict__ enc, const int32_t* __restrict__ perm,
-                   const double* __restrict__ kappa, int first, int count, int prefetch)
+                   const double* __restrict__ kappa, int first, int count)
 {
   using C = MmaCfg<P, WPB>;
   constexpr int n = C::n, n3 = C::n3, SI = C::SI;
@@ -158,10 +158,12 @@ k_apply_affine_mma(const double* __restrict__ x, double* __restrict__ y, const d
     if constexpr (STREAM)
     {
       Gq = Gc + (size_t)p * 6 * n3 + (n == 8 ? 2 * lane : r * n + 2 * c);
-      if (prefetch == 1 || (prefetch == 2 && pl + nw < count))
-      { // this (1) or the next (2) cell's block -> L2 (6 n3 doubles, 128-byte lines)
-        const uintptr_t b0 = reinterpret_cast<uintptr_t>(Gc + ((size_t)p + (prefetch == 2 ? nw : 0)) * 6 * n3),
-                        b1 = b0 + 6 * n3 * 8;
+      // L2 prefetch of this cell's G block, measured at 100 M dofs (none / this cell / next cell): P6 2.36 / 2.22 /
+      // 2.23 ms, P7 1.76 / 1.85 / 2.19 ms (at n = 8 the 16-byte tile loads stream well on their own and the prefetch
+      // only adds DRAM traffic: 12.3 GB against 9.3 GB algorithmic, profiles/r2_apply_p7_mma.txt)
+      if constexpr (P == 6)
+      { // 6 n3 doubles, 128-byte lines
+        const uintptr_t b0 = reinterpret_cast<uintptr_t>(Gc + (size_t)p * 6 * n3), b1 = b0 + 6 * n3 * 8;
         for (uintptr_t a = (b0 & ~(uintptr_t)127) + 128 * lane; a < b1; a += 128 * 32)
           asm volatile("prefetch.global.L2 [%0];" ::"l"(a));
       }
@@ -272,49 +274,22 @@ k_apply_affine_mma(const double* __restrict__ x, double* __restrict__ y, const d
   }
 }
 
-// CTAs of two warps per SM the kernel is compiled for.  6 (168 registers, 16 bytes of spills at P7, 12 warps per
-// SM) against 7 (128 registers, 130-180 bytes of spills, 14 warps), measured at 100 M dofs: affine P6 1.42 vs
-// 1.54 ms, P7 1.19 vs 1.38 ms; streamed P6 2.22 vs 2.93 ms, P7 1.76 vs 2.58 ms.  5 compiles to the same code as 6.
-#ifndef PMGX_MMA_MINB
-#define PMGX_MMA_MINB 6
-#endif
-
+// STREAM = false reads Gc (one 6-vector per affine cell), STREAM = true reads G; both the COLUMN layout
 template <int P, bool STREAM>
-void launch_apply_affine_mma(pmgx_ctx* c, cudaStream_t st, const double* x, double* y, const double* Gc,
-                             const int32_t* enc, const int32_t* perm, const double* kappa, int first, int count)
+struct MmaApply
 {
-  if (count <= 0)
-    return;
-  constexpr int WPB = 2, MINB = PMGX_MMA_MINB;
+  // WPB warps (cells) per CTA; MINB CTAs per SM the kernel is compiled for.  6 (168 registers, 16 bytes of spills
+  // at P7, 12 warps per SM) against 7 (128 registers, 130-180 bytes of spills, 14 warps), measured at 100 M dofs:
+  // affine P6 1.42 vs 1.54 ms, P7 1.19 vs 1.38 ms; streamed P6 2.22 vs 2.93 ms, P7 1.76 vs 2.58 ms.  5 compiles to
+  // the same code as 6.
+  static constexpr int WPB = 2, MINB = 6;
   using C = MmaCfg<P, WPB>;
-  const bool timed = c->profiling && first == 0; // per-kernel timing covers the interior-cell launch only
-  static int ctas_per_sm[64] = {0}; // per instantiation (P, STREAM)
-  if (ctas_per_sm[c->device] == 0)
+  static constexpr bool cell_geometry = !STREAM;
+  static constexpr int cpb = 0;
+  static void name(char* s, int cap) { snprintf(s, cap, "k_apply_affine_mma<%d,%d,%s>", P, WPB, STREAM ? "streamed" : "affine"); }
+  static void launch(pmgx_ctx* c, cudaStream_t st, const ApplyArgs& a)
   {
-    PMGX_CUDA(cudaFuncSetAttribute(k_apply_affine_mma<P, WPB, MINB, STREAM>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C::smem));
-    int nb = 0;
-    PMGX_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, k_apply_affine_mma<P, WPB, MINB, STREAM>, WPB * 32, C::smem));
-    PMGX_REQUIRE(nb >= 1, "k_apply_affine_mma<%d> does not fit on an SM", P);
-    ctas_per_sm[c->device] = nb;
+    launch_persistent<k_apply_affine_mma<P, WPB, MINB, STREAM>>(c, st, a, "k_apply_affine_mma", P, WPB * 32, C::smem,
+                                                                 (a.count + WPB - 1) / WPB, a.cell0, a.count);
   }
-  // L2 prefetch of the streamed G block, measured at 100 M dofs (none / this cell / next cell): P6 2.36 / 2.22 /
-  // 2.23 ms, P7 1.76 / 1.85 / 2.19 ms (at n = 8 the 16-byte tile loads stream well on their own and the prefetch
-  // only adds DRAM traffic: 12.3 GB against 9.3 GB algorithmic, profiles/r2_apply_p7_mma.txt)
-  static const int prefetch = getenv("PMGX_MMA_PREFETCH") ? atoi(getenv("PMGX_MMA_PREFETCH")) : (P == 7 ? 0 : 1);
-  const int grid = std::min((count + WPB - 1) / WPB, ctas_per_sm[c->device] * c->num_sms);
-  cudaEvent_t e0 = nullptr, e1 = nullptr;
-  if (timed)
-  {
-    PMGX_CUDA(cudaEventCreate(&e0));
-    PMGX_CUDA(cudaEventCreate(&e1));
-    PMGX_CUDA(cudaEventRecord(e0, st));
-  }
-  k_apply_affine_mma<P, WPB, MINB, STREAM><<<grid, WPB * 32, C::smem, st>>>(x, y, Gc, enc, perm, kappa, first, count, prefetch);
-  check_launch("k_apply_affine_mma");
-  count_launch(c);
-  if (timed)
-  {
-    PMGX_CUDA(cudaEventRecord(e1, st));
-    c->prof[P].emplace_back(e0, e1);
-  }
-}
+};

@@ -13,18 +13,37 @@ from helpers import OracleLevel, GpuLevel, rel
 pytestmark = pytest.mark.gpu
 TOL = 1e-12
 
+# The apply kernel of every degree, as kernel_name() reports it: (every cell affine, G streamed per quadrature point)
+KERNELS = {
+    1: ("k_apply_affine<1,128>", "k_apply_tma<1,64,2>"),
+    2: ("k_apply_affine_shfl<2,128>", "k_apply_tma<2,128,2>"),
+    3: ("k_apply_affine2<3,64,warp-local>", "k_apply_tma<3,128,2>"),
+    4: ("k_apply_affine<4,64>", "k_apply_tma<4,128,2>"),
+    5: ("k_apply_affine<5,64>", "k_apply_tma<5,64,2>"),
+    6: ("k_apply_affine_mma<6,2,affine>", "k_apply_affine_mma<6,2,streamed>"),
+    7: ("k_apply_affine_mma<7,2,affine>", "k_apply_affine_mma<7,2,streamed>"),
+    8: ("k_apply<8>", "k_apply<8>"),
+}
+
 
 @pytest.mark.parametrize("P", [1, 2, 3, 4, 5, 6, 7, 8])
 @pytest.mark.parametrize("perturb", [0.0, 0.2])
 def test_apply_matches_oracle(ctx, P, perturb):
+    """Both apply kernels of every degree: the uniform box takes the affine one (except at P8, which has none),
+    the perturbed box and PMGX_LAP_STREAM_G (flags=4) on the uniform box the streamed-G one."""
     n = (3, 4, 5) if P <= 4 else (2, 3, 2)
     ol = OracleLevel(om.create_box(*n, perturb=perturb), P)
-    gl = GpuLevel(ctx, ol)
+    levels = [(GpuLevel(ctx, ol), KERNELS[P][0 if perturb == 0.0 else 1])]
+    if perturb == 0.0:
+        levels.append((GpuLevel(ctx, ol, flags=4), KERNELS[P][1]))
     rng = np.random.default_rng(42)
-    for x in (rng.uniform(-1, 1, ol.nd), np.ones(ol.nd)):
-        y, yo = gl.apply(x), ol.A(x)
-        e2, einf = rel(y, yo)
-        assert e2 < TOL and einf < TOL, (P, perturb, e2, einf)
+    for gl, kernel in levels:
+        assert gl.op.kernel_name() == kernel, (P, perturb, gl.op.kernel_name())
+        assert gl.op.is_affine() == (kernel == KERNELS[P][0] and P != 8)
+        for x in (rng.uniform(-1, 1, ol.nd), np.ones(ol.nd)):
+            y, yo = gl.apply(x), ol.A(x)
+            e2, einf = rel(y, yo)
+            assert e2 < TOL and einf < TOL, (P, perturb, kernel, e2, einf)
 
 
 @pytest.mark.parametrize("P", [1, 3, 4, 6])

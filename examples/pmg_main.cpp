@@ -7,7 +7,9 @@
 // Only the DOLFINx set-up (mesh, function spaces, assembly of b) is swapped for the box-mesh
 // helpers of the C ABI.
 //
-//   pmg_main [--ndofs N] [--degrees 1,2,4] [--niter 10] [--perturb 0.0] [--coarse-its 60]
+//   pmg_main [--ndofs N] [--degrees 1,2,4] [--niter 10] [--perturb 0.0] [--coarse-its 60] [--batch_size 0]
+// --batch_size N > 0: every MatFreeLaplacian keeps no geometry and recomputes it in each apply (the
+// reference's option of the same name; N itself only selects the mode).
 // Multi-GPU: one process per GPU with RANK / WORLD_SIZE / LOCAL_RANK in the environment and
 // --idfile PATH on a shared filesystem (rank 0 writes the NCCL id there; the reference uses
 // MPI for this, which this image does not have).
@@ -23,6 +25,7 @@ int main(int argc, char** argv)
   long long ndofs = 50000; // per rank, like the reference's default (:405)
   std::vector<int> degrees = {1, 2, 4};
   int niter = 10, coarse_its = 60;
+  std::size_t batch_size = 0;
   double perturb = 0.0, coarse_rtol = 1e-5; // PETSc default rtol of the reference's coarse KSP (src/amg.hpp:40)
   std::string idfile;
   for (int i = 1; i < argc; ++i)
@@ -43,6 +46,8 @@ int main(int argc, char** argv)
       coarse_its = std::atoi(next());
     else if (!std::strcmp(argv[i], "--idfile"))
       idfile = next();
+    else if (!std::strcmp(argv[i], "--batch_size"))
+      batch_size = (std::size_t)std::atoll(next());
     else if (!std::strcmp(argv[i], "--degrees"))
     {
       degrees.clear();
@@ -53,7 +58,7 @@ int main(int argc, char** argv)
     else
     {
       std::printf("usage: %s [--ndofs N] [--degrees 1,2,4] [--niter 10] [--perturb p] [--coarse-its k] "
-                  "[--idfile path]\n", argv[0]);
+                  "[--batch_size N] [--idfile path]\n", argv[0]);
       return std::strcmp(argv[i], "--help") ? 1 : 0;
     }
   }
@@ -91,7 +96,8 @@ int main(int argc, char** argv)
     for (Space& s : V)
       operators.push_back(std::make_shared<FineOperator>(s.degree, mesh.kappa.span(), s.dofmap.span(), mesh.xgeom.span(),
                                                          mesh.geometry_dofmap.span(), std::span<const T>(),
-                                                         std::span<const T>(), lcells, bcells, s.bc.span()));
+                                                         std::span<const T>(), lcells, bcells, s.bc.span(),
+                                                         batch_size));
 
     // ---- right-hand side on the finest level (:289-300, examples/pmg/poisson.py:6-8,30)
     Space& top = V.back();

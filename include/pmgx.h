@@ -142,6 +142,12 @@ int pmgx_vec_norm(pmgx_ctx* ctx, const double* a, long long n, int linf, double*
 #define PMGX_LAP_STREAM_G 4       /* always stream the per-quadrature-point G (the reference's data flow,
                                      src/laplacian.hpp:221-227); default: when every cell of the operator is
                                      affine the apply uses one geometry 6-vector per cell, G(q) = w_q Gc */
+#define PMGX_LAP_RECOMPUTE_G 8    /* keep no geometry: no per-quadrature-point G and no per-cell Gc.  Every apply,
+                                     CSR assembly and get_G computes G from the borrowed xgeom / geom_dofmap (the
+                                     reference's batch_size > 0 mode, src/laplacian.hpp:383-396), so vertices moved
+                                     in place take effect at the next apply; the diagonal is still computed once at
+                                     create.  No affinity test runs (is_affine() is 0); PMGX_LAP_STREAM_G has no
+                                     effect with it; PMGX_LAP_LITERAL_DETJ and PMGX_LAP_NO_DIAG apply as usual. */
 
 /* MatFreeLaplacian ctor (src/laplacian.hpp:289-349).  dofmap[n_cells][(P+1)^3],
  * xgeom[n_points][3], geom_dofmap[n_cells][8] (tensor-product vertex order),
@@ -164,6 +170,9 @@ int pmgx_laplacian_get_G(pmgx_operator* op, double* G_out);
 int pmgx_laplacian_is_affine(pmgx_operator* op);
 /* name and template arguments of the apply kernel this operator launches (for bench / profiles) */
 int pmgx_laplacian_kernel_name(pmgx_operator* op, char* name_h, int cap);
+/* bytes of device memory the operator owns: launch-order permutation, encoded dofmap, G, Gc and the
+ * inverse diagonal (for sizing problems, and to compare PMGX_LAP_RECOMPUTE_G against the default) */
+int pmgx_laplacian_device_bytes(pmgx_operator* op, long long* bytes_h);
 
 /* ------------------------------------------------------------- CSR operator -- */
 /* MatrixOperator (src/csr.hpp:57-131): row_ptr[n_rows+1], off_diag_offset[n_rows] (first

@@ -288,7 +288,10 @@ protected:
 
 /// Matrix-free Laplacian (src/laplacian.hpp:283-526): same constructor arguments.  The geometry
 /// tables (dphi_geometry, G_weights) are accepted for signature compatibility and regenerated
-/// internally; batch_size must be 0 (geometry is always precomputed, Appendix B of SURVEY.md).
+/// internally.  batch_size = 0 precomputes the geometry factors once, as the reference does;
+/// batch_size > 0 selects the reference's recompute mode (src/laplacian.hpp:383-396) through
+/// PMGX_LAP_RECOMPUTE_G: the operator keeps no geometry and every apply forms it inside the kernel
+/// from xgeom.  Nothing is stored per batch, so the value itself only selects the mode.
 template <typename T>
 class MatFreeLaplacian : public OperatorBase
 {
@@ -300,12 +303,11 @@ public:
                    const std::vector<int>& lcells, const std::vector<int>& bcells,
                    std::span<const std::int8_t> bc_marker, std::size_t batch_size = 0)
       : degree(degree), cell_constants(coefficients), cell_dofmap(dofmap), xgeom(xgeom),
-        geometry_dofmap(geometry_dofmap), bc_marker(bc_marker), lcells(lcells), bcells(bcells)
+        geometry_dofmap(geometry_dofmap), bc_marker(bc_marker), lcells(lcells), bcells(bcells),
+        flags(batch_size > 0 ? PMGX_LAP_RECOMPUTE_G : PMGX_LAP_DEFAULT)
   {
     if (degree < 1 || degree > PMGX_MAX_DEGREE)
       throw std::runtime_error("Unsupported degree");
-    if (batch_size != 0)
-      throw std::runtime_error("pmgx: geometry batching is not supported (batch_size must be 0)");
   }
 
 protected:
@@ -316,7 +318,7 @@ protected:
                                       cell_dofmap.data(), xgeom.data(), (int)(xgeom.size() / 3),
                                       geometry_dofmap.data(), cell_constants.data(), lcells.data(),
                                       (int)lcells.size(), bcells.data(), (int)bcells.size(), bc_marker.data(),
-                                      map->size_local(), map->num_ghosts(), map->halo(), PMGX_LAP_DEFAULT, &_op));
+                                      map->size_local(), map->num_ghosts(), map->halo(), flags, &_op));
   }
 
 private:
@@ -327,6 +329,7 @@ private:
   std::span<const std::int32_t> geometry_dofmap;
   std::span<const std::int8_t> bc_marker;
   std::vector<int> lcells, bcells;
+  int flags;
 };
 
 /// Assembled CSR operator (src/csr.hpp:57-297).  The reference assembles a DOLFINx form; here

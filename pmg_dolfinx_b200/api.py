@@ -17,6 +17,14 @@ import torch
 from .capi import lib, check, ptr, PmgxError  # noqa: F401
 
 
+# pmgx_laplacian_create flags (include/pmgx.h)
+LAP_DEFAULT = 0
+LAP_LITERAL_DETJ = 1   # detJ expression of the reference verbatim (quirk Q17)
+LAP_NO_DIAG = 2        # skip the matrix-free diagonal at create
+LAP_STREAM_G = 4       # stream the per-quadrature-point G even when every cell is affine
+LAP_RECOMPUTE_G = 8    # keep no geometry; every apply recomputes G from xgeom (the reference's batch_size > 0)
+
+
 def _np(a, dtype):
     return np.ascontiguousarray(a, dtype=dtype)
 
@@ -357,6 +365,12 @@ class MatFreeLaplacian(_Operator):
     def is_affine(self):
         """True when the apply runs the affine-geometry kernel (one geometry 6-vector per cell)."""
         return bool(lib.pmgx_laplacian_is_affine(self.h))
+
+    def device_bytes(self):
+        """Bytes of device memory the operator owns (permutation, encoded dofmap, G, Gc, inverse diagonal)."""
+        b = ctypes.c_longlong()
+        check(lib.pmgx_laplacian_device_bytes(self.h, ctypes.addressof(b)))
+        return b.value
 
     def kernel_name(self):
         buf = ctypes.create_string_buffer(96)

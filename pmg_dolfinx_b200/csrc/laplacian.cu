@@ -15,6 +15,8 @@
 //   k_apply_tma                                P1..P5, G streamed per quadrature point through a TMA ring
 //   k_apply_affine_mma                         P6, P7: FP64 tensor cores, one warp per cell (laplacian_mma.cuh)
 //   k_apply                                    P8: column kernel
+// and, for PMGX_LAP_RECOMPUTE_G, a variant of each of the last three families that forms G at its points from the
+// cell's vertices instead of reading it (no per-point geometry is stored).
 // In the slab kernels (P1..P5) a thread owns one z-index of a cell and keeps the (ix,iy) slab of
 // the element in registers: the x and y contractions are register FMAs against constant-memory
 // derivative entries, only the z contraction crosses threads.
@@ -105,6 +107,117 @@ __global__ void k_encode_dofmap(const int32_t* __restrict__ dofmap, const int32_
   }
 }
 
+// ------------------------------------------------------- geometry of the trilinear hexahedron --
+// J, K = adj(J), det J and G = s K K^T (6 unique entries xx,xy,xz,yy,yz,zz) for every path that forms G from the
+// vertices without storing it (PMGX_LAP_RECOMPUTE_G).  Vertex order k = 4a + 2b + c (src/mesh.hpp:75-84).  The
+// set-up paths go through jacobian_at; the apply kernels form J in the factored per-thread forms of
+// TrilinearMonomials.  k_geometry and k_cell_geometry below keep their own copy of the same expressions: routed
+// through these helpers, k_geometry's G changed in the last bit on perturbed meshes (different FMA contraction).
+
+// J = sum_k x_k dphi_k(xi), the vertices read from xgeom through the cell's 8 geometry dofs gd
+__device__ __forceinline__ void jacobian_at(const double* __restrict__ xgeom, const int32_t* __restrict__ gd,
+                                            const double (&xi)[3], double (&J)[3][3])
+{
+#pragma unroll
+  for (int i = 0; i < 3; ++i)
+#pragma unroll
+    for (int j = 0; j < 3; ++j)
+      J[i][j] = 0.0;
+#pragma unroll
+  for (int k = 0; k < 8; ++k)
+  {
+    const int a = (k >> 2) & 1, b = (k >> 1) & 1, c = k & 1;
+    const double la = a ? xi[0] : 1.0 - xi[0], lb = b ? xi[1] : 1.0 - xi[1],
+                 lc = c ? xi[2] : 1.0 - xi[2];
+    const double da = a ? 1.0 : -1.0, db = b ? 1.0 : -1.0, dc = c ? 1.0 : -1.0;
+    const double dphi[3] = {da * lb * lc, la * db * lc, la * lb * dc};
+    const double* xv = xgeom + 3ll * gd[k];
+#pragma unroll
+    for (int i = 0; i < 3; ++i)
+#pragma unroll
+      for (int j = 0; j < 3; ++j)
+        J[i][j] += xv[i] * dphi[j];
+  }
+}
+
+// K = adj(J) and det J; literal_detj: the expression of src/laplacian.hpp:97 (quirk Q17)
+__device__ __forceinline__ double adjugate_det(const double (&J)[3][3], bool literal_detj, double (&K)[3][3])
+{
+  K[0][0] = J[1][1] * J[2][2] - J[1][2] * J[2][1];
+  K[0][1] = -J[0][1] * J[2][2] + J[0][2] * J[2][1];
+  K[0][2] = J[0][1] * J[1][2] - J[0][2] * J[1][1];
+  K[1][0] = -J[1][0] * J[2][2] + J[1][2] * J[2][0];
+  K[1][1] = J[0][0] * J[2][2] - J[0][2] * J[2][0];
+  K[1][2] = -J[0][0] * J[1][2] + J[0][2] * J[1][0];
+  K[2][0] = J[1][0] * J[2][1] - J[1][1] * J[2][0];
+  K[2][1] = -J[0][0] * J[2][1] + J[0][1] * J[2][0];
+  K[2][2] = J[0][0] * J[1][1] - J[0][1] * J[1][0];
+  double detJ;
+  if (literal_detj)
+    detJ = J[0][0] * K[0][0] - J[1][0] * K[0][1] + J[0][2] * K[2][0];
+  else
+    detJ = J[0][0] * K[0][0] + J[0][1] * K[1][0] + J[0][2] * K[2][0];
+  return detJ;
+}
+
+// g = s K K^T (s = w / det J)
+__device__ __forceinline__ void g_from_adjugate(const double (&K)[3][3], double s, double (&g)[6])
+{
+  g[0] = (K[0][0] * K[0][0] + K[0][1] * K[0][1] + K[0][2] * K[0][2]) * s;
+  g[1] = (K[1][0] * K[0][0] + K[1][1] * K[0][1] + K[1][2] * K[0][2]) * s;
+  g[2] = (K[2][0] * K[0][0] + K[2][1] * K[0][1] + K[2][2] * K[0][2]) * s;
+  g[3] = (K[1][0] * K[1][0] + K[1][1] * K[1][1] + K[1][2] * K[1][2]) * s;
+  g[4] = (K[2][0] * K[1][0] + K[2][1] * K[1][1] + K[2][2] * K[1][2]) * s;
+  g[5] = (K[2][0] * K[2][0] + K[2][1] * K[2][1] + K[2][2] * K[2][2]) * s;
+}
+
+// g = w K K^T / det J of the Jacobian J
+__device__ __forceinline__ void g_from_jacobian(const double (&J)[3][3], bool literal_detj, double w, double (&g)[6])
+{
+  double K[3][3];
+  const double detJ = adjugate_det(J, literal_detj, K);
+  g_from_adjugate(K, w / detJ, g);
+}
+
+// The trilinear map in monomial form, x = a0 + a1 xi + a2 eta + a3 zeta + a4 xi eta + a5 xi zeta + a6 eta zeta
+// + a7 xi eta zeta (m[0..6] = a1..a7, one 3-vector each), so that the Jacobian columns are
+//   dx/dxi = a1 + a4 eta + a5 zeta + a7 eta zeta,  dx/deta = a2 + a4 xi + a6 zeta + a7 xi zeta,
+//   dx/dzeta = a3 + a5 xi + a6 eta + a7 xi eta:
+// with one or two reference coordinates fixed per thread every column is affine in the remaining one.
+struct TrilinearMonomials
+{
+  double m[7][3];
+  // from the cell's vertices v[k][i], k = 4a + 2b + c
+  __device__ __forceinline__ void from_vertices(const double (&v)[8][3])
+  {
+#pragma unroll
+    for (int i = 0; i < 3; ++i)
+    {
+      m[0][i] = v[4][i] - v[0][i];
+      m[1][i] = v[2][i] - v[0][i];
+      m[2][i] = v[1][i] - v[0][i];
+      m[3][i] = (v[6][i] - v[4][i]) - (v[2][i] - v[0][i]);
+      m[4][i] = (v[5][i] - v[4][i]) - (v[1][i] - v[0][i]);
+      m[5][i] = (v[3][i] - v[2][i]) - (v[1][i] - v[0][i]);
+      m[6][i] = ((v[7][i] - v[6][i]) - (v[5][i] - v[4][i])) - ((v[3][i] - v[2][i]) - (v[1][i] - v[0][i]));
+    }
+  }
+  // the cell with geometry dofs gd (the unit cube when gd is null: finite, inert geometry for idle threads)
+  __device__ __forceinline__ void load(const double* __restrict__ xgeom, const int32_t* gd)
+  {
+    double v[8][3];
+#pragma unroll
+    for (int k = 0; k < 8; ++k)
+    {
+      const int32_t d = gd ? gd[k] : 0;
+#pragma unroll
+      for (int i = 0; i < 3; ++i)
+        v[k][i] = gd ? xgeom[3ll * d + i] : (double)((k >> (2 - i)) & 1);
+    }
+    from_vertices(v);
+  }
+};
+
 // One thread per (cell position, quadrature point).  J = sum_k x_k dphi_k, K = adj(J),
 // G = w K K^T / detJ with 6 unique entries (xx,xy,xz,yy,yz,zz).  Also used for detJ only.
 template <bool WRITE_G>
@@ -169,6 +282,32 @@ __global__ void k_geometry(int P, const double* __restrict__ xgeom,
       detj_w[t] = w * fabs(detJ);
   }
 }
+
+// Where the set-up kernels (diagonal, CSR assembly, get_G) read G(p, comp, q) from: the stored array, or
+// computed from the vertices on the fly (PMGX_LAP_RECOMPUTE_G: no per-point geometry exists)
+struct StoredG
+{
+  const double* G;
+  Lay lay;
+  __device__ __forceinline__ double operator()(long long p, int comp, int q) const { return G[lay.g_index(p, comp, q)]; }
+};
+struct VertexG
+{
+  const double* xgeom;
+  const int32_t* geom_dofmap;
+  const int32_t* perm;
+  int P;
+  bool literal_detj;
+  __device__ double operator()(long long p, int comp, int q) const
+  {
+    const int n = P + 1, ix = q / (n * n), iy = (q / n) % n, iz = q % n;
+    const double xi[3] = {c_pts[P][ix], c_pts[P][iy], c_pts[P][iz]};
+    double J[3][3], g[6];
+    jacobian_at(xgeom, geom_dofmap + (long long)perm[p] * 8, xi, J);
+    g_from_jacobian(J, literal_detj, c_wts[P][ix] * c_wts[P][iy] * c_wts[P][iz], g);
+    return g[comp];
+  }
+};
 
 // Per cell: Gc = K K^T / det J of the trilinear map at the cell centre (weight 1), and the affinity
 // test: a cell is affine iff every vertex equals v000 + a e1 + b e2 + c e3; the deviation is
@@ -235,8 +374,97 @@ __global__ void k_cell_geometry(const double* __restrict__ xgeom, const int32_t*
   g[5] = (K[2][0] * K[2][0] + K[2][1] * K[2][1] + K[2][2] * K[2][2]) * s;
 }
 
+// Per-thread factored Jacobians of the apply kernels that recompute G.  Along a line of fixed (eta, zeta) (a
+// column thread, an mma lane): dx/dxi is constant, dx/deta and dx/dzeta are affine in xi -- 15 coefficients, 6 FMAs
+// per point.
+struct JacobianAlongXi
+{
+  double c0[3], e0[3], e1[3], z0[3], z1[3];
+  __device__ __forceinline__ void init(const TrilinearMonomials& M, double eta, double zeta)
+  {
+#pragma unroll
+    for (int i = 0; i < 3; ++i)
+    {
+      c0[i] = fma(M.m[6][i] * eta + M.m[4][i], zeta, fma(M.m[3][i], eta, M.m[0][i]));
+      e0[i] = fma(M.m[5][i], zeta, M.m[1][i]);
+      e1[i] = fma(M.m[6][i], zeta, M.m[3][i]);
+      z0[i] = fma(M.m[5][i], eta, M.m[2][i]);
+      z1[i] = fma(M.m[6][i], eta, M.m[4][i]);
+    }
+  }
+  __device__ __forceinline__ void at(double xi, double (&J)[3][3]) const
+  {
+#pragma unroll
+    for (int i = 0; i < 3; ++i)
+    {
+      J[i][0] = c0[i];
+      J[i][1] = fma(e1[i], xi, e0[i]);
+      J[i][2] = fma(z1[i], xi, z0[i]);
+    }
+  }
+};
+// On a plane of fixed zeta (a slab thread): dx/dxi = x0 + x1 eta, dx/deta = y0 + x1 xi and
+// dx/dzeta = (a3 + a5 xi) + (a6 + a7 xi) eta -- 21 coefficients, kept in shared memory (store); per plane xi
+// 9 FMAs (plane), per point 6 (at).
+struct JacobianAtZeta
+{
+  double x0[3], x1[3], y0[3], a3[3], a5[3], a6[3], a7[3];
+  __device__ __forceinline__ void init(const TrilinearMonomials& M, double zeta)
+  {
+#pragma unroll
+    for (int i = 0; i < 3; ++i)
+    {
+      x0[i] = fma(M.m[4][i], zeta, M.m[0][i]);
+      x1[i] = fma(M.m[6][i], zeta, M.m[3][i]);
+      y0[i] = fma(M.m[5][i], zeta, M.m[1][i]);
+      a3[i] = M.m[2][i], a5[i] = M.m[4][i], a6[i] = M.m[5][i], a7[i] = M.m[6][i];
+    }
+  }
+  // the 21 coefficients as rows of a [21][stride] array
+  __device__ __forceinline__ void store(double* p, int stride) const
+  {
+#pragma unroll
+    for (int i = 0; i < 3; ++i)
+    {
+      p[(0 + i) * stride] = x0[i], p[(3 + i) * stride] = x1[i], p[(6 + i) * stride] = y0[i];
+      p[(9 + i) * stride] = a3[i], p[(12 + i) * stride] = a5[i], p[(15 + i) * stride] = a6[i];
+      p[(18 + i) * stride] = a7[i];
+    }
+  }
+  // the xi-dependent parts of plane xi: dx/deta, and dx/dzeta = z0 + z1 eta
+  struct Plane
+  {
+    double y[3], z0[3], z1[3];
+  };
+  // plane() and at() on the stored form, reading each coefficient where it is used (no 21 live registers)
+  __device__ __forceinline__ static Plane plane(const volatile double* p, int stride, double xi)
+  {
+    Plane q;
+#pragma unroll
+    for (int i = 0; i < 3; ++i)
+    {
+      q.y[i] = fma(p[(3 + i) * stride], xi, p[(6 + i) * stride]);
+      q.z0[i] = fma(p[(12 + i) * stride], xi, p[(9 + i) * stride]);
+      q.z1[i] = fma(p[(18 + i) * stride], xi, p[(15 + i) * stride]);
+    }
+    return q;
+  }
+  __device__ __forceinline__ static void at(const volatile double* p, int stride, const Plane& q, double eta,
+                                            double (&J)[3][3])
+  {
+#pragma unroll
+    for (int i = 0; i < 3; ++i)
+    {
+      J[i][0] = fma(p[(3 + i) * stride], eta, p[(0 + i) * stride]);
+      J[i][1] = q.y[i];
+      J[i][2] = fma(q.z1[i], eta, q.z0[i]);
+    }
+  }
+};
+
 // diag(A) contributions, thread per (cell position, local dof); see DESIGN.md "diagonal".
-__global__ void k_diag(int P, const double* __restrict__ G, const int32_t* __restrict__ enc,
+template <typename Geo>
+__global__ void k_diag(int P, Geo G, const int32_t* __restrict__ enc,
                        const int32_t* __restrict__ perm, const double* __restrict__ kappa,
                        double* __restrict__ diag, int n_list, Lay lay)
 {
@@ -256,13 +484,13 @@ __global__ void k_diag(int P, const double* __restrict__ G, const int32_t* __res
     for (int q = 0; q < n; ++q)
     {
       const double dx = D[q * n + i], dy = D[q * n + j], dz = D[q * n + k];
-      s += dx * dx * G[lay.g_index(p, 0, q * n2 + j * n + k)];
-      s += dy * dy * G[lay.g_index(p, 3, i * n2 + q * n + k)];
-      s += dz * dz * G[lay.g_index(p, 5, i * n2 + j * n + q)];
+      s += dx * dx * G(p, 0, q * n2 + j * n + k);
+      s += dy * dy * G(p, 3, i * n2 + q * n + k);
+      s += dz * dz * G(p, 5, i * n2 + j * n + q);
     }
     const double dii = D[i * n + i], djj = D[j * n + j], dkk = D[k * n + k];
-    s += 2.0 * (G[lay.g_index(p, 1, a)] * dii * djj + G[lay.g_index(p, 2, a)] * dii * dkk
-                + G[lay.g_index(p, 4, a)] * djj * dkk);
+    s += 2.0 * (G(p, 1, a) * dii * djj + G(p, 2, a) * dii * dkk
+                + G(p, 4, a) * djj * dkk);
     atomicAdd(&diag[d], kappa[perm[p]] * s);
   }
 }
@@ -275,8 +503,8 @@ __global__ void k_invert_diag(const double* __restrict__ diag, const int8_t* __r
     dinv[i] = bc[i] ? 1.0 : 1.0 / diag[i];
 }
 
-__global__ void k_G_to_reference_layout(const double* __restrict__ G, double* __restrict__ out,
-                                        int n3, long long total, Lay lay)
+template <typename Geo>
+__global__ void k_G_to_reference_layout(Geo G, double* __restrict__ out, int n3, long long total)
 {
   const long long nth = (long long)gridDim.x * blockDim.x;
   for (long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x; t < total; t += nth)
@@ -284,7 +512,7 @@ __global__ void k_G_to_reference_layout(const double* __restrict__ G, double* __
     const long long p = t / (6 * n3);
     const int r = (int)(t - p * 6 * n3);
     const int q = r / 6, c = r % 6;
-    out[t] = G[lay.g_index(p, c, q)];
+    out[t] = G(p, c, q);
   }
 }
 
@@ -336,37 +564,39 @@ __global__ void k_fill(double* __restrict__ v, double a, int n)
 // Entry (i,j) of the element matrix kappa * B^T G B with the collocated gradient table
 // (phi = identity at the GLL points, src/laplacian.hpp:200-202): only index pairs that
 // agree in at least one direction couple.
-__device__ double element_entry(int P, const double* __restrict__ G, const Lay& lay, long long p, int i, int j)
+template <typename Geo>
+__device__ double element_entry(int P, const Geo& G, long long p, int i, int j)
 {
-  const int n = P + 1, n2 = n * n, n3 = n2 * n;
+  const int n = P + 1, n2 = n * n;
   const double* D = c_D[P];
   const int ix = i / n2, iy = (i / n) % n, iz = i % n;
   const int jx = j / n2, jy = (j / n) % n, jz = j % n;
   double s = 0.0;
   if (iy == jy && iz == jz)
     for (int q = 0; q < n; ++q)
-      s += D[q * n + ix] * D[q * n + jx] * G[lay.g_index(p, 0, q * n2 + iy * n + iz)];
+      s += D[q * n + ix] * D[q * n + jx] * G(p, 0, q * n2 + iy * n + iz);
   if (ix == jx && iz == jz)
     for (int q = 0; q < n; ++q)
-      s += D[q * n + iy] * D[q * n + jy] * G[lay.g_index(p, 3, ix * n2 + q * n + iz)];
+      s += D[q * n + iy] * D[q * n + jy] * G(p, 3, ix * n2 + q * n + iz);
   if (ix == jx && iy == jy)
     for (int q = 0; q < n; ++q)
-      s += D[q * n + iz] * D[q * n + jz] * G[lay.g_index(p, 5, ix * n2 + iy * n + q)];
+      s += D[q * n + iz] * D[q * n + jz] * G(p, 5, ix * n2 + iy * n + q);
   if (iz == jz)
-    s += D[jx * n + ix] * D[iy * n + jy] * G[lay.g_index(p, 1, jx * n2 + iy * n + iz)]
-         + D[jy * n + iy] * D[ix * n + jx] * G[lay.g_index(p, 1, ix * n2 + jy * n + iz)];
+    s += D[jx * n + ix] * D[iy * n + jy] * G(p, 1, jx * n2 + iy * n + iz)
+         + D[jy * n + iy] * D[ix * n + jx] * G(p, 1, ix * n2 + jy * n + iz);
   if (iy == jy)
-    s += D[jx * n + ix] * D[iz * n + jz] * G[lay.g_index(p, 2, jx * n2 + iy * n + iz)]
-         + D[jz * n + iz] * D[ix * n + jx] * G[lay.g_index(p, 2, ix * n2 + iy * n + jz)];
+    s += D[jx * n + ix] * D[iz * n + jz] * G(p, 2, jx * n2 + iy * n + iz)
+         + D[jz * n + iz] * D[ix * n + jx] * G(p, 2, ix * n2 + iy * n + jz);
   if (ix == jx)
-    s += D[jy * n + iy] * D[iz * n + jz] * G[lay.g_index(p, 4, ix * n2 + jy * n + iz)]
-         + D[jz * n + iz] * D[iy * n + jy] * G[lay.g_index(p, 4, ix * n2 + iy * n + jz)];
+    s += D[jy * n + iy] * D[iz * n + jz] * G(p, 4, ix * n2 + jy * n + iz)
+         + D[jz * n + iz] * D[iy * n + jy] * G(p, 4, ix * n2 + iy * n + jz);
   return s;
 }
 
 // One (key, value) per (cell, i, j); key = row * ntot + col, sentinel for dropped entries
 // (ghost rows, Dirichlet rows / columns: fem::assemble_matrix with bcs, src/csr.hpp:84).
-__global__ void k_element_triplets(int P, const double* __restrict__ G, const int32_t* __restrict__ enc,
+template <typename Geo>
+__global__ void k_element_triplets(int P, Geo G, const int32_t* __restrict__ enc,
                                    const int32_t* __restrict__ perm, const double* __restrict__ kappa,
                                    long long n_list, int n_owned, long long ntot,
                                    unsigned long long* __restrict__ keys, double* __restrict__ vals, Lay lay)
@@ -388,7 +618,7 @@ __global__ void k_element_triplets(int P, const double* __restrict__ G, const in
       continue;
     }
     keys[t] = (unsigned long long)di * (unsigned long long)ntot + (unsigned long long)dj;
-    vals[t] = kappa[perm[p]] * element_entry(P, G, lay, p, i, j);
+    vals[t] = kappa[perm[p]] * element_entry(P, G, p, i, j);
   }
 }
 
@@ -431,7 +661,8 @@ __global__ void k_offdiag(const int32_t* __restrict__ row_ptr, const int32_t* __
 // ---------------------------------------------------------------- apply launches --
 // One launch of an apply kernel: the cells [cell0, cell0 + count) of the launch list, whose first
 // batch in the SLAB layout is batch0 (the COLUMN-layout kernels ignore it); geom is Gc for the
-// kernels that take one geometry 6-vector per cell, G otherwise.
+// kernels that take one geometry 6-vector per cell, G for the streamed-G kernels.  The kernels that
+// recompute G per point read the mesh instead: xgeom, geom_dofmap (both borrowed) and the det J form.
 struct ApplyArgs
 {
   const double* x;
@@ -442,6 +673,9 @@ struct ApplyArgs
   const double* kappa;
   long long batch0;
   int cell0, count;
+  const double* xgeom;
+  const int32_t* geom_dofmap;
+  int literal_detj;
 };
 
 // Launches a persistent apply kernel of degree P: CTAs of tpb threads stay resident and walk over the
@@ -482,12 +716,12 @@ void launch_persistent(pmgx_ctx* c, cudaStream_t st, const ApplyArgs& a, const c
 }
 
 // The SLAB-layout kernels (k_apply_tma, k_apply_affine*): one block of work is one batch of Cfg::cpb cells
-template <auto kernel, typename Cfg>
-void launch_batched(pmgx_ctx* c, cudaStream_t st, const ApplyArgs& a, const char* name)
+template <auto kernel, typename Cfg, typename... Extra>
+void launch_batched(pmgx_ctx* c, cudaStream_t st, const ApplyArgs& a, const char* name, Extra... extra)
 {
   const int nbatch = (a.count + Cfg::cpb - 1) / Cfg::cpb;
   launch_persistent<kernel>(c, st, a, name, Cfg::n - 1, Cfg::tpb, Cfg::smem, nbatch, a.batch0, a.cell0, a.count,
-                            nbatch);
+                            nbatch, extra...);
 }
 
 // Every launcher below (one per kernel family) exports
@@ -512,11 +746,13 @@ struct ApplyCfg
   static constexpr int smem_doubles = cpb * (n * plane + 4 * plane);
 };
 
-template <int P>
+// RECOMPUTE: no G array; the thread forms G at its (j, k) column's point of every plane i from the cell's vertices
+template <int P, bool RECOMPUTE>
 __global__ void __launch_bounds__(ApplyCfg<P>::tpb)
 k_apply(const double* __restrict__ x, double* __restrict__ y, const double* __restrict__ G,
         const int32_t* __restrict__ enc, const int32_t* __restrict__ perm,
-        const double* __restrict__ kappa, int first, int count)
+        const double* __restrict__ kappa, int first, int count, const double* __restrict__ xgeom,
+        const int32_t* __restrict__ geom_dofmap, int literal_detj)
 {
   using C = ApplyCfg<P>;
   constexpr int n = C::n, n2 = C::n2, n3 = C::n3, ROW = C::row, PL = C::plane, CPB = C::cpb;
@@ -538,15 +774,27 @@ k_apply(const double* __restrict__ x, double* __restrict__ y, const double* __re
   double kap = 0.0;
   const double* Gp = G + p * 6 * n3 + jk;
   double g[6];
+  JacobianAlongXi jac;   // RECOMPUTE
+  double wjk = 0.0;      // RECOMPUTE: w_j w_k
+  if constexpr (RECOMPUTE)
+  {
+    TrilinearMonomials M;
+    M.load(xgeom, active ? geom_dofmap + (long long)perm[p] * 8 : nullptr);
+    jac.init(M, c_pts[P][j], c_pts[P][k]);
+    wjk = c_wts[P][j] * c_wts[P][k];
+  }
   if (active)
   {
     const int32_t* e = enc + p * n3 + jk;
 #pragma unroll
     for (int i = 0; i < n; ++i)
       d[i] = ldg_stream_i32(e + i * n2);
+    if constexpr (!RECOMPUTE)
+    {
 #pragma unroll
-    for (int c = 0; c < 6; ++c)
-      g[c] = ldg_stream(Gp + c * n3);
+      for (int c = 0; c < 6; ++c)
+        g[c] = ldg_stream(Gp + c * n3);
+    }
     kap = kappa[perm[p]];
 #pragma unroll
     for (int i = 0; i < n; ++i)
@@ -590,7 +838,13 @@ k_apply(const double* __restrict__ x, double* __restrict__ y, const double* __re
   {
     // prefetch next plane's geometry
     double gn[6];
-    if (i + 1 < n)
+    if constexpr (RECOMPUTE)
+    {
+      double J[3][3];
+      jac.at(c_pts[P][i], J);
+      g_from_jacobian(J, literal_detj, c_wts[P][i] * wjk, g);
+    }
+    else if (i + 1 < n)
     {
       if (active)
       {
@@ -637,7 +891,7 @@ k_apply(const double* __restrict__ x, double* __restrict__ y, const double* __re
       t = fma(DTk[q], sfz[j * ROW + q], t);
     }
     acc[i] += t;
-    if (i + 1 < n)
+    if (!RECOMPUTE && i + 1 < n)
     {
 #pragma unroll
       for (int c = 0; c < 6; ++c)
@@ -654,13 +908,19 @@ k_apply(const double* __restrict__ x, double* __restrict__ y, const double* __re
 }
 
 // Not persistent: one CTA per ApplyCfg<P>::cpb cells of the COLUMN layout
-template <int P>
+template <int P, bool RECOMPUTE = false>
 struct ColumnApply
 {
   using C = ApplyCfg<P>;
   static constexpr bool cell_geometry = false;
   static constexpr int cpb = 0;
-  static void name(char* s, int cap) { snprintf(s, cap, "k_apply<%d>", P); }
+  static void name(char* s, int cap)
+  {
+    if (RECOMPUTE)
+      snprintf(s, cap, "k_apply<%d,recomputed>", P);
+    else
+      snprintf(s, cap, "k_apply<%d>", P);
+  }
   static void launch(pmgx_ctx* c, cudaStream_t st, const ApplyArgs& a)
   {
     if (a.count <= 0)
@@ -669,7 +929,7 @@ struct ColumnApply
     static bool configured[64] = {false};
     if (!configured[c->device])
     {
-      PMGX_CUDA(cudaFuncSetAttribute(k_apply<P>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+      PMGX_CUDA(cudaFuncSetAttribute(k_apply<P, RECOMPUTE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
       configured[c->device] = true;
     }
     const int grid = (a.count + C::cpb - 1) / C::cpb;
@@ -681,7 +941,8 @@ struct ColumnApply
       PMGX_CUDA(cudaEventCreate(&e1));
       PMGX_CUDA(cudaEventRecord(e0, st));
     }
-    k_apply<P><<<grid, C::tpb, smem, st>>>(a.x, a.y, a.geom, a.enc, a.perm, a.kappa, a.cell0, a.count);
+    k_apply<P, RECOMPUTE><<<grid, C::tpb, smem, st>>>(a.x, a.y, a.geom, a.enc, a.perm, a.kappa, a.cell0, a.count,
+                                                      a.xgeom, a.geom_dofmap, a.literal_detj);
     check_launch("k_apply");
     count_launch(c);
     if (timed)
@@ -750,13 +1011,15 @@ __device__ __forceinline__ void bulk_g2s(void* dst, const void* src, uint32_t by
                : "memory");
 }
 
-template <int P, int TPB>
+// RECOMPUTE: no geometry ring; every thread forms G at its points from the cell's vertices (JacobianAtZeta)
+template <int P, int TPB, bool RECOMPUTE = false>
 struct TmaCfg
 {
   static constexpr int n = P + 1;
   static constexpr int n2 = n * n;
   static constexpr int tpb = TPB;
   static constexpr int R = 2; // geometry planes in flight (measured on B200: a 2-plane ring wins for P3/P4)
+  static constexpr int ring = RECOMPUTE ? 0 : R;
   static constexpr int cpb = tpb / n;
   static constexpr int S = (cpb * n + 1) & ~1;  // G rows: 16-byte multiples, (almost) no padding streamed
   static constexpr int SE = (cpb * n + 3) & ~3; // dofmap rows: 16-byte multiples of int32
@@ -770,7 +1033,11 @@ struct TmaCfg
   static constexpr uint32_t plane_bytes = plane_doubles * sizeof(double);
   static constexpr uint32_t enc_bytes = n2 * SE * sizeof(int32_t);
   static constexpr int buf_doubles = 2 * cpb * cs; // double-buffered plane rows (su and sf each)
-  static constexpr size_t off_enc = (size_t)R * plane_bytes;
+  // RECOMPUTE: instead of the ring, [21][TPB] JacobianAtZeta coefficients and [n][6][TPB] G at the thread's points
+  // of the current plane, one column per thread (written and read by the same thread: no barrier)
+  static constexpr int GS = RECOMPUTE ? TPB : S; // stride of the six G components in shared memory
+  static constexpr size_t off_gq = 21 * (size_t)TPB * sizeof(double);
+  static constexpr size_t off_enc = RECOMPUTE ? off_gq + (size_t)6 * n * TPB * sizeof(double) : (size_t)ring * plane_bytes;
   // dofmap buffers: double-buffered (read again at scatter time, next batch prefetched meanwhile)
   static constexpr size_t off_su = off_enc + 2 * enc_bytes;
   static constexpr size_t off_sf = off_su + (size_t)buf_doubles * sizeof(double);
@@ -778,16 +1045,20 @@ struct TmaCfg
   static constexpr size_t smem = off_bar + (R + 2) * sizeof(uint64_t);
 };
 
-template <int P, int TPB>
-__global__ void __launch_bounds__(TPB, TmaCfg<P, TPB>::minb)
+template <int P, int TPB, bool RECOMPUTE>
+__global__ void __launch_bounds__(TPB, TmaCfg<P, TPB, RECOMPUTE>::minb)
 k_apply_tma(const double* __restrict__ x, double* __restrict__ y, const double* __restrict__ G,
             const int32_t* __restrict__ enc, const int32_t* __restrict__ perm,
-            const double* __restrict__ kappa, long long batch0, int cell0, int count, int nbatch)
+            const double* __restrict__ kappa, long long batch0, int cell0, int count, int nbatch,
+            const double* __restrict__ xgeom, const int32_t* __restrict__ geom_dofmap, int literal_detj)
 {
-  using C = TmaCfg<P, TPB>;
+  using C = TmaCfg<P, TPB, RECOMPUTE>;
   constexpr int n = C::n, n2 = C::n2, CPB = C::cpb, S = C::S, SE = C::SE, KP = C::kp, CS = C::cs, R = C::R;
+  constexpr int GS = C::GS;
   extern __shared__ __align__(128) unsigned char smraw[];
   double* sG = reinterpret_cast<double*>(smraw);
+  double* const sJ = sG + threadIdx.x;                                             // RECOMPUTE
+  double* const sGq = reinterpret_cast<double*>(smraw + C::off_gq) + threadIdx.x; // RECOMPUTE
   const int32_t* sE = reinterpret_cast<const int32_t*>(smraw + C::off_enc);
   double* su = reinterpret_cast<double*>(smraw + C::off_su);
   double* sf = reinterpret_cast<double*>(smraw + C::off_sf);
@@ -833,8 +1104,9 @@ k_apply_tma(const double* __restrict__ x, double* __restrict__ y, const double* 
   if (tid == 0 && my_nb > 0)
   {
     issue_enc(0);
-    for (; issue_t < R && issue_t < total_planes; ++issue_t)
-      issue_plane(issue_t);
+    if constexpr (!RECOMPUTE)
+      for (; issue_t < R && issue_t < total_planes; ++issue_t)
+        issue_plane(issue_t);
   }
 
   double Dk[n], DTk[n];
@@ -844,6 +1116,7 @@ k_apply_tma(const double* __restrict__ x, double* __restrict__ y, const double* 
     Dk[l] = c_D[P][k * n + l];
     DTk[l] = c_D[P][l * n + k];
   }
+  const double zeta = c_pts[P][k], wk = c_wts[P][k]; // RECOMPUTE
 
   int stage = 0;
   uint32_t stage_parity = 0;
@@ -858,6 +1131,14 @@ k_apply_tma(const double* __restrict__ x, double* __restrict__ y, const double* 
     const int32_t* dE = sE + eb * (n2 * SE) + tid; // this thread's n2 encoded dofs
     double u[n2];
     double kap = 0.0;
+    if constexpr (RECOMPUTE)
+    { // this thread's plane zeta of the cell; the previous batch's reads of sJ / sGq were its own, earlier
+      TrilinearMonomials M;
+      M.load(xgeom, active ? geom_dofmap + (long long)perm[cell0 + pl] * 8 : nullptr);
+      JacobianAtZeta jac;
+      jac.init(M, zeta);
+      jac.store(sJ, TPB);
+    }
     if (active)
     {
       kap = kappa[perm[cell0 + pl]];
@@ -896,10 +1177,26 @@ k_apply_tma(const double* __restrict__ x, double* __restrict__ y, const double* 
 #pragma unroll
     for (int i = 0; i < n; ++i)
     {
-      mbar_wait(&fullG[stage], stage_parity);
-      const double* gs = sG + (size_t)stage * C::plane_doubles + tid;
+      if constexpr (!RECOMPUTE)
+        mbar_wait(&fullG[stage], stage_parity);
+      const double* gs = RECOMPUTE ? sGq : sG + (size_t)stage * C::plane_doubles + tid;
       const double* sup = su + ((i & 1) * CPB + cls) * CS;
       double* sfz = sf + ((i & 1) * CPB + cls) * CS;
+      if constexpr (RECOMPUTE)
+      { // G at the points (i, j, k), j = 0..n-1, one point at a time: the slab (u, acc) keeps the registers
+        const JacobianAtZeta::Plane jp = JacobianAtZeta::plane(sJ, TPB, c_pts[P][i]);
+        const double wik = c_wts[P][i] * wk;
+#pragma unroll 1
+        for (int j = 0; j < n; ++j)
+        {
+          double J[3][3], g[6];
+          JacobianAtZeta::at(sJ, TPB, jp, c_pts[P][j], J);
+          g_from_jacobian(J, literal_detj, wik * c_wts[P][j], g);
+#pragma unroll
+          for (int c = 0; c < 6; ++c)
+            sGq[(j * 6 + c) * TPB] = g[c];
+        }
+      }
       double fz[n];
 #pragma unroll
       for (int j = 0; j < n; ++j)
@@ -920,8 +1217,8 @@ k_apply_tma(const double* __restrict__ x, double* __restrict__ y, const double* 
           gx = fma(c_D[P][i * n + l], u[l * n + j], gx);
           gy = fma(c_D[P][j * n + l], u[i * n + l], gy);
         }
-        const double g0 = gs[(j * 6 + 0) * S], g1 = gs[(j * 6 + 1) * S], g2 = gs[(j * 6 + 2) * S];
-        const double g3 = gs[(j * 6 + 3) * S], g4 = gs[(j * 6 + 4) * S], g5 = gs[(j * 6 + 5) * S];
+        const double g0 = gs[(j * 6 + 0) * GS], g1 = gs[(j * 6 + 1) * GS], g2 = gs[(j * 6 + 2) * GS];
+        const double g3 = gs[(j * 6 + 3) * GS], g4 = gs[(j * 6 + 4) * GS], g5 = gs[(j * 6 + 5) * GS];
         const double fx = kap * (g0 * gx + g1 * gy + g2 * gz);
         const double fy = kap * (g1 * gx + g3 * gy + g4 * gz);
         fz[j] = kap * (g2 * gx + g4 * gy + g5 * gz);
@@ -946,15 +1243,18 @@ k_apply_tma(const double* __restrict__ x, double* __restrict__ y, const double* 
         }
       }
       __syncthreads(); // geometry stage is consumed; fz rows and next z-rows are visible
-      if (tid == 0)
+      if constexpr (!RECOMPUTE)
       {
-        if (issue_t < total_planes)
-          issue_plane(issue_t++);
-      }
-      if (++stage == R)
-      {
-        stage = 0;
-        stage_parity ^= 1u;
+        if (tid == 0)
+        {
+          if (issue_t < total_planes)
+            issue_plane(issue_t++);
+        }
+        if (++stage == R)
+        {
+          stage = 0;
+          stage_parity ^= 1u;
+        }
       }
 #pragma unroll
       for (int j = 0; j < n; ++j)
@@ -985,16 +1285,22 @@ k_apply_tma(const double* __restrict__ x, double* __restrict__ y, const double* 
   }
 }
 
-template <int P, int TPB>
+template <int P, int TPB, bool RECOMPUTE = false>
 struct TmaApply
 {
-  using C = TmaCfg<P, TPB>;
+  using C = TmaCfg<P, TPB, RECOMPUTE>;
   static constexpr bool cell_geometry = false;
   static constexpr int cpb = C::cpb;
-  static void name(char* s, int cap) { snprintf(s, cap, "k_apply_tma<%d,%d,%d>", P, TPB, C::R); }
+  static void name(char* s, int cap)
+  {
+    if (RECOMPUTE)
+      snprintf(s, cap, "k_apply_tma<%d,%d,recomputed>", P, TPB);
+    else
+      snprintf(s, cap, "k_apply_tma<%d,%d,%d>", P, TPB, C::R);
+  }
   static void launch(pmgx_ctx* c, cudaStream_t st, const ApplyArgs& a)
   {
-    launch_batched<k_apply_tma<P, TPB>, C>(c, st, a, "k_apply_tma");
+    launch_batched<k_apply_tma<P, TPB, RECOMPUTE>, C>(c, st, a, "k_apply_tma", a.xgeom, a.geom_dofmap, a.literal_detj);
   }
 };
 
@@ -1663,28 +1969,42 @@ struct Affine2Apply
 // * P8: the column kernel; the slab kernels keep 2 (P+1)^2 doubles in registers per thread (measured: P7 53 % vs
 //   47 %, P8 24 % vs 27 %) and n = 9 fits no 8-wide tensor-core tile.  It has no affine variant, so the affinity
 //   test is skipped and is_affine() stays 0.
+// * Recompute (PMGX_LAP_RECOMPUTE_G): each family's geometry-from-vertices variant, with the thread mapping and the
+//   launch configuration of its streamed-G kernel.
 template <int P>
 struct ApplyKernels;
-template <> struct ApplyKernels<1> { using Affine = AffineApply<1, 128>;     using Streamed = TmaApply<1, 64>; };
-template <> struct ApplyKernels<2> { using Affine = AffineShflApply<2, 128>; using Streamed = TmaApply<2, 128>; };
-template <> struct ApplyKernels<3> { using Affine = Affine2Apply<3, 64>;     using Streamed = TmaApply<3, 128>; };
-template <> struct ApplyKernels<4> { using Affine = AffineApply<4, 64>;      using Streamed = TmaApply<4, 128>; };
-template <> struct ApplyKernels<5> { using Affine = AffineApply<5, 64>;      using Streamed = TmaApply<5, 64>; };
-template <> struct ApplyKernels<6> { using Affine = MmaApply<6, false>;      using Streamed = MmaApply<6, true>; };
-template <> struct ApplyKernels<7> { using Affine = MmaApply<7, false>;      using Streamed = MmaApply<7, true>; };
-template <> struct ApplyKernels<8> { using Affine = ColumnApply<8>;          using Streamed = ColumnApply<8>; };
+// clang-format off
+template <> struct ApplyKernels<1> { using Affine = AffineApply<1, 128>;     using Streamed = TmaApply<1, 64>;  using Recompute = TmaApply<1, 64, true>; };
+template <> struct ApplyKernels<2> { using Affine = AffineShflApply<2, 128>; using Streamed = TmaApply<2, 128>; using Recompute = TmaApply<2, 128, true>; };
+template <> struct ApplyKernels<3> { using Affine = Affine2Apply<3, 64>;     using Streamed = TmaApply<3, 128>; using Recompute = TmaApply<3, 128, true>; };
+template <> struct ApplyKernels<4> { using Affine = AffineApply<4, 64>;      using Streamed = TmaApply<4, 128>; using Recompute = TmaApply<4, 128, true>; };
+template <> struct ApplyKernels<5> { using Affine = AffineApply<5, 64>;      using Streamed = TmaApply<5, 64>;  using Recompute = TmaApply<5, 64, true>; };
+template <> struct ApplyKernels<6> { using Affine = MmaApply<6, MMA_AFFINE>; using Streamed = MmaApply<6, MMA_STREAMED>; using Recompute = MmaApply<6, MMA_RECOMPUTED>; };
+template <> struct ApplyKernels<7> { using Affine = MmaApply<7, MMA_AFFINE>; using Streamed = MmaApply<7, MMA_STREAMED>; using Recompute = MmaApply<7, MMA_RECOMPUTED>; };
+template <> struct ApplyKernels<8> { using Affine = ColumnApply<8>;          using Streamed = ColumnApply<8>;   using Recompute = ColumnApply<8, true>; };
+// clang-format on
 
-// f(K{}) with K the launcher of the apply kernel of degree P (Affine if `affine`, else Streamed)
+// Which entry of ApplyKernels<P> an operator runs
+enum class ApplyGeometry
+{
+  Affine,
+  Streamed,
+  Recompute
+};
+
+// f(K{}) with K the launcher of the apply kernel of degree P for geometry mode `geo`
 template <typename F>
-void with_apply_kernel(int P, bool affine, F&& f)
+void with_apply_kernel(int P, ApplyGeometry geo, F&& f)
 {
   const auto pick = [&](auto deg)
   {
     using K = ApplyKernels<decltype(deg)::value>;
-    if (affine)
+    if (geo == ApplyGeometry::Affine)
       f(typename K::Affine{});
-    else
+    else if (geo == ApplyGeometry::Streamed)
       f(typename K::Streamed{});
+    else
+      f(typename K::Recompute{});
   };
   switch (P)
   {
@@ -1749,8 +2069,18 @@ struct Laplacian : pmgx_operator
   Lay lay;
   DevBuf<double> Gc;   // [n_list][6] per-cell geometry factor of affine cells
   bool affine = false; // every cell affine: ApplyKernels<P>::Affine replaces the streamed-G kernel
+  bool recompute = false; // PMGX_LAP_RECOMPUTE_G: no G, no Gc; every user of G forms it from xgeom
 
   int n_list() const { return n_l + n_b; }
+  pmgx::ApplyGeometry geometry() const
+  {
+    return recompute ? pmgx::ApplyGeometry::Recompute
+                     : (affine ? pmgx::ApplyGeometry::Affine : pmgx::ApplyGeometry::Streamed);
+  }
+  bool literal_detj() const { return (flags & PMGX_LAP_LITERAL_DETJ) != 0; }
+  // G(p, comp, q) for the set-up kernels
+  pmgx::StoredG stored_G() const { return {G.p, lay}; }
+  pmgx::VertexG vertex_G() const { return {xgeom, geom_dofmap, perm.p, P, literal_detj()}; }
 
   void apply(double* x, double* y) override
   {
@@ -1766,14 +2096,15 @@ struct Laplacian : pmgx_operator
     // where the interior kernel is long enough to hide the join anyway
     const bool side = halo && P <= 2;
     cudaStream_t bs = side ? halo_stream(halo, ctx) : ctx->stream;
-    with_apply_kernel(P, affine, [&](auto k)
+    const int lit = literal_detj();
+    with_apply_kernel(P, geometry(), [&](auto k)
     {
       using K = decltype(k);
       const double* geom = K::cell_geometry ? Gc.p : G.p;
-      K::launch(ctx, ctx->stream, {x, y, geom, enc.p, perm.p, kappa, 0, 0, n_l}); // :406-409
+      K::launch(ctx, ctx->stream, {x, y, geom, enc.p, perm.p, kappa, 0, 0, n_l, xgeom, geom_dofmap, lit}); // :406-409
       if (halo && !side)
         halo_fwd_end(halo, x); // reference order: wait for the ghosts, then the boundary launch (:425)
-      K::launch(ctx, bs, {x, y, geom, enc.p, perm.p, kappa, lay.nb_l, n_l, n_b}); // :449-452
+      K::launch(ctx, bs, {x, y, geom, enc.p, perm.p, kappa, lay.nb_l, n_l, n_b, xgeom, geom_dofmap, lit}); // :449-452
     });
     if (side)
       halo_fwd_end(halo, x);                                                      // :425 (join)
@@ -1827,6 +2158,7 @@ int pmgx_laplacian_create(pmgx_ctx* ctx, int degree, int n_cells, const int32_t*
   L->geom_dofmap = geom_dofmap;
   L->dofmap_borrowed = dofmap;
   L->flags = flags;
+  L->recompute = (flags & PMGX_LAP_RECOMPUTE_G) != 0;
 
   const int n_list = L->n_list();
   std::vector<int32_t> perm_h((size_t)n_list);
@@ -1845,8 +2177,9 @@ int pmgx_laplacian_create(pmgx_ctx* ctx, int degree, int n_cells, const int32_t*
   // affine cells: one geometry 6-vector per cell instead of one per quadrature point, for the degrees
   // that have a kernel for it (decided first: the layout follows the kernel that will run)
   bool has_affine_kernel = false;
-  pmgx::with_apply_kernel(degree, true, [&](auto k) { has_affine_kernel = decltype(k)::cell_geometry; });
-  if (n_list > 0 && has_affine_kernel && !(flags & PMGX_LAP_STREAM_G))
+  pmgx::with_apply_kernel(degree, pmgx::ApplyGeometry::Affine,
+                          [&](auto k) { has_affine_kernel = decltype(k)::cell_geometry; });
+  if (n_list > 0 && has_affine_kernel && !(flags & PMGX_LAP_STREAM_G) && !L->recompute)
   {
     L->Gc.alloc((size_t)n_list * 6);
     pmgx::DevBuf<int> bad;
@@ -1863,7 +2196,7 @@ int pmgx_laplacian_create(pmgx_ctx* ctx, int degree, int n_cells, const int32_t*
     if (!L->affine)
       L->Gc.release();
   }
-  pmgx::with_apply_kernel(degree, L->affine, [&](auto k) { lay.cpb = decltype(k)::cpb; });
+  pmgx::with_apply_kernel(degree, L->geometry(), [&](auto k) { lay.cpb = decltype(k)::cpb; });
   lay.mode = lay.cpb > 0 ? 1 : 0;
   if (lay.mode == 1)
   {
@@ -1873,24 +2206,29 @@ int pmgx_laplacian_create(pmgx_ctx* ctx, int degree, int n_cells, const int32_t*
     lay.n_batches = lay.nb_l + (n_bcells + lay.cpb - 1) / lay.cpb;
   }
   const long long enc_size = lay.mode == 1 ? lay.enc_size() : total;
-  const long long g_size = lay.mode == 1 ? lay.g_size() : total * 6;
+  const long long g_size = L->recompute ? 0 : (lay.mode == 1 ? lay.g_size() : total * 6);
   L->enc.alloc((size_t)enc_size);
   L->G.alloc((size_t)g_size);
   if (lay.mode == 1 && enc_size > 0)
   { // padded slots: inert
     PMGX_CUDA(cudaMemsetAsync(L->enc.p, 0, (size_t)enc_size * sizeof(int32_t), ctx->stream));
-    PMGX_CUDA(cudaMemsetAsync(L->G.p, 0, (size_t)g_size * sizeof(double), ctx->stream));
+    if (g_size > 0)
+      PMGX_CUDA(cudaMemsetAsync(L->G.p, 0, (size_t)g_size * sizeof(double), ctx->stream));
   }
   if (total > 0)
   {
     pmgx::k_encode_dofmap<<<pmgx::setup_grid(ctx, total), 256, 0, ctx->stream>>>(
         dofmap, L->perm.p, bc_marker, L->enc.p, L->n3, total, lay);
     pmgx::check_launch("k_encode_dofmap");
-    pmgx::k_geometry<true><<<pmgx::setup_grid(ctx, total), 256, 0, ctx->stream>>>(
-        degree, xgeom, geom_dofmap, L->perm.p, L->G.p, nullptr, n_list,
-        (flags & PMGX_LAP_LITERAL_DETJ) != 0, lay);
-    pmgx::check_launch("k_geometry");
-    pmgx::count_launch(ctx, 2);
+    pmgx::count_launch(ctx);
+    if (!L->recompute)
+    {
+      pmgx::k_geometry<true><<<pmgx::setup_grid(ctx, total), 256, 0, ctx->stream>>>(
+          degree, xgeom, geom_dofmap, L->perm.p, L->G.p, nullptr, n_list,
+          (flags & PMGX_LAP_LITERAL_DETJ) != 0, lay);
+      pmgx::check_launch("k_geometry");
+      pmgx::count_launch(ctx);
+    }
   }
   L->diag_inv.alloc((size_t)n_owned);
   if (!(flags & PMGX_LAP_NO_DIAG) && n_owned > 0)
@@ -1900,8 +2238,12 @@ int pmgx_laplacian_create(pmgx_ctx* ctx, int degree, int n_cells, const int32_t*
     PMGX_CUDA(cudaMemsetAsync(diag.p, 0, diag.n * sizeof(double), ctx->stream));
     if (total > 0)
     {
-      pmgx::k_diag<<<pmgx::setup_grid(ctx, total), 256, 0, ctx->stream>>>(
-          degree, L->G.p, L->enc.p, L->perm.p, kappa, diag.p, n_list, lay);
+      if (L->recompute)
+        pmgx::k_diag<<<pmgx::setup_grid(ctx, total), 256, 0, ctx->stream>>>(
+            degree, L->vertex_G(), L->enc.p, L->perm.p, kappa, diag.p, n_list, lay);
+      else
+        pmgx::k_diag<<<pmgx::setup_grid(ctx, total), 256, 0, ctx->stream>>>(
+            degree, L->stored_G(), L->enc.p, L->perm.p, kappa, diag.p, n_list, lay);
       pmgx::check_launch("k_diag");
     }
     pmgx::k_invert_diag<<<(n_owned + 255) / 256, 256, 0, ctx->stream>>>(diag.p, bc_marker,
@@ -1926,8 +2268,12 @@ int pmgx_laplacian_get_G(pmgx_operator* op, double* G_out)
   if (total > 0)
   {
     PMGX_CUDA(cudaSetDevice(L->ctx->device));
-    pmgx::k_G_to_reference_layout<<<pmgx::setup_grid(L->ctx, total), 256, 0, L->ctx->stream>>>(
-        L->G.p, G_out, L->n3, total, L->lay);
+    if (L->recompute) // straight into the caller's buffer: no G exists
+      pmgx::k_G_to_reference_layout<<<pmgx::setup_grid(L->ctx, total), 256, 0, L->ctx->stream>>>(
+          L->vertex_G(), G_out, L->n3, total);
+    else
+      pmgx::k_G_to_reference_layout<<<pmgx::setup_grid(L->ctx, total), 256, 0, L->ctx->stream>>>(
+          L->stored_G(), G_out, L->n3, total);
     pmgx::check_launch("k_G_to_reference_layout");
     pmgx::count_launch(L->ctx);
   }
@@ -1944,7 +2290,17 @@ int pmgx_laplacian_kernel_name(pmgx_operator* op, char* name_h, int cap)
   PMGX_API_BEGIN
   PMGX_REQUIRE(op && op->kind == pmgx_operator::LAPLACIAN && name_h && cap > 0, "laplacian_kernel_name: bad arguments");
   auto* L = static_cast<Laplacian*>(op);
-  pmgx::with_apply_kernel(L->P, L->affine, [&](auto k) { decltype(k)::name(name_h, cap); });
+  pmgx::with_apply_kernel(L->P, L->geometry(), [&](auto k) { decltype(k)::name(name_h, cap); });
+  PMGX_API_END
+}
+
+int pmgx_laplacian_device_bytes(pmgx_operator* op, long long* bytes_h)
+{
+  PMGX_API_BEGIN
+  PMGX_REQUIRE(op && op->kind == pmgx_operator::LAPLACIAN && bytes_h, "laplacian_device_bytes: bad arguments");
+  auto* L = static_cast<Laplacian*>(op);
+  *bytes_h = (long long)(L->perm.n * sizeof(int32_t) + L->enc.n * sizeof(int32_t) + L->G.n * sizeof(double)
+                         + L->Gc.n * sizeof(double) + L->diag_inv.n * sizeof(double));
   PMGX_API_END
 }
 
@@ -2013,7 +2369,9 @@ int pmgx_laplacian_lift(pmgx_operator* op, const double* gvals, double* b)
   const int n_points_unknown = 0; // only used for argument checks
   const int rc = pmgx_laplacian_create(ctx, L->P, L->n_cells, L->dofmap_borrowed, L->xgeom, n_points_unknown, L->geom_dofmap,
                                        L->kappa, perm_h.data(), (int)perm_h.size(), nullptr, 0, nobc.p, L->n_owned,
-                                       L->n_ghost, nullptr, (L->flags & PMGX_LAP_LITERAL_DETJ) | PMGX_LAP_NO_DIAG, &full);
+                                       L->n_ghost, nullptr,
+                                       (L->flags & (PMGX_LAP_LITERAL_DETJ | PMGX_LAP_RECOMPUTE_G)) | PMGX_LAP_NO_DIAG,
+                                       &full);
   if (rc != PMGX_OK)
     return rc;
   pmgx::DevBuf<double> gbc, y;
@@ -2049,8 +2407,12 @@ int pmgx_csr_from_laplacian(pmgx_operator* op, pmgx_operator** out)
   vals.alloc((size_t)std::max<long long>(n_trip, 1));
   if (n_list > 0)
   {
-    pmgx::k_element_triplets<<<pmgx::setup_grid(ctx, n_list * per_cell), 256, 0, st>>>(
-        L->P, L->G.p, L->enc.p, L->perm.p, L->kappa, n_list, n_owned, ntot, keys.p, vals.p, L->lay);
+    if (L->recompute)
+      pmgx::k_element_triplets<<<pmgx::setup_grid(ctx, n_list * per_cell), 256, 0, st>>>(
+          L->P, L->vertex_G(), L->enc.p, L->perm.p, L->kappa, n_list, n_owned, ntot, keys.p, vals.p, L->lay);
+    else
+      pmgx::k_element_triplets<<<pmgx::setup_grid(ctx, n_list * per_cell), 256, 0, st>>>(
+          L->P, L->stored_G(), L->enc.p, L->perm.p, L->kappa, n_list, n_owned, ntot, keys.p, vals.p, L->lay);
     pmgx::check_launch("k_element_triplets");
   }
   if (n_owned > 0)

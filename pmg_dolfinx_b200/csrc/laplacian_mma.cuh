@@ -51,23 +51,36 @@ struct MmaCfg
   }
 };
 
-// STREAM = false: Gc[p][6], one geometry 6-vector per (affine) cell, quadrature weights applied here;
-// STREAM = true : Gc = G[p][6][n3], the reference's data flow (G per quadrature point, weights folded in),
-//                 read in layout Y one tile ahead of the flux that uses it; at P6 the cell's whole block is
-//                 prefetched into L2 first
-template <int P, int WPB, int MINB, bool STREAM>
+// Where the kernel takes the geometry from:
+//   MMA_AFFINE    : Gc[p][6], one geometry 6-vector per (affine) cell, quadrature weights applied here;
+//   MMA_STREAMED  : Gc = G[p][6][n3], the reference's data flow (G per quadrature point, weights folded in),
+//                   read in layout Y one tile ahead of the flux that uses it; at P6 the cell's whole block is
+//                   prefetched into L2 first;
+//   MMA_RECOMPUTED: no G; the cell's 8 vertices go to 24 doubles of per-warp shared memory beside the three
+//                   arrays, and every lane forms G at its two points of tile t from its JacobianAlongXi pair
+//                   (fixed eta_r, zeta_{2c+h}) right where the streamed variant consumes its G registers.
+enum MmaGeometry
+{
+  MMA_AFFINE,
+  MMA_STREAMED,
+  MMA_RECOMPUTED
+};
+template <int P, int WPB, int MINB, int GEO>
 __global__ void __launch_bounds__(WPB * 32, MINB)
 k_apply_affine_mma(const double* __restrict__ x, double* __restrict__ y, const double* __restrict__ Gc,
                    const int32_t* __restrict__ enc, const int32_t* __restrict__ perm,
-                   const double* __restrict__ kappa, int first, int count)
+                   const double* __restrict__ kappa, int first, int count, const double* __restrict__ xgeom,
+                   const int32_t* __restrict__ geom_dofmap, int literal_detj)
 {
   using C = MmaCfg<P, WPB>;
   constexpr int n = C::n, n3 = C::n3, SI = C::SI;
+  constexpr bool STREAM = GEO == MMA_STREAMED, RECOMPUTE = GEO == MMA_RECOMPUTED;
   extern __shared__ __align__(16) double smem_mma[];
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   double* const B0 = smem_mma + (size_t)warp * 3 * C::arr; // U, then gx in transit, then fx
   double* const B1 = B0 + C::arr;                          // fy, then the X accumulator in transit
   double* const B2 = B1 + C::arr;                          // fz
+  double* const SV = smem_mma + (size_t)WPB * 3 * C::arr + warp * 24; // RECOMPUTE: the cell's vertices [8][3]
   for (int i = lane; i < 3 * C::arr; i += 32)
     B0[i] = 0.0; // planes i >= n are never written again: everything the tiles read there is an exact zero
   __syncwarp();
@@ -138,6 +151,11 @@ k_apply_affine_mma(const double* __restrict__ x, double* __restrict__ y, const d
     for (int t = 0; t < n; ++t)
       *reinterpret_cast<double2*>(B0 + t * SI + yo[(t >> 1) & 1]) = make_double2(xv[t][0], xv[t][1]);
     const double kap = kappa[perm[p]]; // re-read on every apply (src/laplacian.hpp:230)
+    if constexpr (RECOMPUTE)
+    { // the previous cell's reads of SV ended before the barrier after its flux phase
+      if (lane < 24)
+        SV[lane] = xgeom[3ll * geom_dofmap[(long long)perm[p] * 8 + lane / 3] + lane % 3];
+    }
     double G00 = 0, G01 = 0, G02 = 0, G11 = 0, G12 = 0, G22 = 0;
     const double* Gq = nullptr; // STREAM: this lane's first point of the cell's G block
     double2 gq[2][6];           // STREAM: G of the lane's two points, tiles t (flux) and t + 1 (in flight)
@@ -169,7 +187,7 @@ k_apply_affine_mma(const double* __restrict__ x, double* __restrict__ y, const d
       }
       load_g(0, gq[0]);
     }
-    else
+    else if constexpr (GEO == MMA_AFFINE)
     {
       const double* gp = Gc + (size_t)p * 6;
       G00 = gp[0] * kap, G01 = gp[1] * kap, G02 = gp[2] * kap, G11 = gp[3] * kap, G12 = gp[4] * kap, G22 = gp[5] * kap;
@@ -195,17 +213,44 @@ k_apply_affine_mma(const double* __restrict__ x, double* __restrict__ y, const d
       *reinterpret_cast<double2*>(B0 + t * 8 + xo[(t >> 1) & 1]) = make_double2(gx[t][0], gx[t][1]);
     __syncwarp();
     // ---- flux at the Y points (i = t, j = r, k = 2c + h); a lane overwrites only the slots it has just read
+    // RECOMPUTE: the lane's lines (eta_r, zeta_{2c+h}) inside the cell (padding lanes: weight 0, any point)
+    const double eta = c_pts[P][r < n ? r : 0], zeta0 = c_pts[P][v0 ? 2 * c : 0], zeta1 = c_pts[P][v1 ? 2 * c + 1 : 0];
 #pragma unroll
     for (int t = 0; t < n; ++t)
     {
       const int o = t * SI + yo[(t >> 1) & 1];
       const double2 g = *reinterpret_cast<const double2*>(B0 + o);
       double w0, w1;
-      if constexpr (STREAM)
+      if constexpr (STREAM || RECOMPUTE)
       {
-        if (t + 1 < n)
+        double2 qr[6]; // RECOMPUTE: G at the lane's two points of tile t, weights folded in
+        if constexpr (RECOMPUTE)
+        { // the vertices are re-read from shared memory for every tile (volatile): held in registers across the
+          // tiles, the lane's coefficients spill next to gy, gz
+          const volatile double* sv = SV;
+          double v[8][3];
+#pragma unroll
+          for (int kk = 0; kk < 8; ++kk)
+#pragma unroll
+            for (int i = 0; i < 3; ++i)
+              v[kk][i] = sv[kk * 3 + i];
+          TrilinearMonomials M;
+          M.from_vertices(v);
+          JacobianAlongXi jac;
+          double J[3][3], g0[6], g1[6];
+          jac.init(M, eta, zeta0);
+          jac.at(c_pts[P][t], J);
+          g_from_jacobian(J, literal_detj, c_wts[P][t] * wr0, g0);
+          jac.init(M, eta, zeta1);
+          jac.at(c_pts[P][t], J);
+          g_from_jacobian(J, literal_detj, c_wts[P][t] * wr1, g1);
+#pragma unroll
+          for (int cc = 0; cc < 6; ++cc)
+            qr[cc] = make_double2(g0[cc], g1[cc]);
+        }
+        else if (t + 1 < n)
           load_g(t + 1, gq[(t + 1) & 1]);
-        const double2* q = gq[t & 1];
+        const double2* q = RECOMPUTE ? qr : gq[t & 1];
         w0 = w1 = kap;
         G00 = q[0].x, G01 = q[1].x, G02 = q[2].x, G11 = q[3].x, G12 = q[4].x, G22 = q[5].x;
         const double f0 = G00 * g.x + G01 * gy[t][0] + G02 * gz[t][0];
@@ -274,8 +319,8 @@ k_apply_affine_mma(const double* __restrict__ x, double* __restrict__ y, const d
   }
 }
 
-// STREAM = false reads Gc (one 6-vector per affine cell), STREAM = true reads G; both the COLUMN layout
-template <int P, bool STREAM>
+// MMA_AFFINE reads Gc (one 6-vector per affine cell), MMA_STREAMED reads G (the COLUMN layout), MMA_RECOMPUTED the mesh
+template <int P, int GEO>
 struct MmaApply
 {
   // WPB warps (cells) per CTA; MINB CTAs per SM the kernel is compiled for.  6 (168 registers, 16 bytes of spills
@@ -284,12 +329,18 @@ struct MmaApply
   // the same code as 6.
   static constexpr int WPB = 2, MINB = 6;
   using C = MmaCfg<P, WPB>;
-  static constexpr bool cell_geometry = !STREAM;
+  static constexpr bool cell_geometry = GEO == MMA_AFFINE;
   static constexpr int cpb = 0;
-  static void name(char* s, int cap) { snprintf(s, cap, "k_apply_affine_mma<%d,%d,%s>", P, WPB, STREAM ? "streamed" : "affine"); }
+  static constexpr size_t smem = C::smem + (GEO == MMA_RECOMPUTED ? WPB * 24 * sizeof(double) : 0);
+  static void name(char* s, int cap)
+  {
+    snprintf(s, cap, "k_apply_affine_mma<%d,%d,%s>", P, WPB,
+             GEO == MMA_AFFINE ? "affine" : (GEO == MMA_STREAMED ? "streamed" : "recomputed"));
+  }
   static void launch(pmgx_ctx* c, cudaStream_t st, const ApplyArgs& a)
   {
-    launch_persistent<k_apply_affine_mma<P, WPB, MINB, STREAM>>(c, st, a, "k_apply_affine_mma", P, WPB * 32, C::smem,
-                                                                 (a.count + WPB - 1) / WPB, a.cell0, a.count);
+    launch_persistent<k_apply_affine_mma<P, WPB, MINB, GEO>>(c, st, a, "k_apply_affine_mma", P, WPB * 32, smem,
+                                                              (a.count + WPB - 1) / WPB, a.cell0, a.count, a.xgeom,
+                                                              a.geom_dofmap, a.literal_detj);
   }
 };

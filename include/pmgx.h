@@ -316,8 +316,9 @@ int pmgx_amg_level_dist_get(pmgx_amg_hier* h, int level, int* ghost_src_h, int32
                             int32_t* recv_idx_h, double* inv_rows_h);
 /* Host helper of the coarse solver: the CSR matrix without its stored zeros (a row's diagonal entry is kept
  * whatever its value).  pmgx_csr_from_laplacian keeps the full 27-point pattern of the P1 element matrices like
- * DOLFINx's assemble_matrix does (src/csr.hpp:66-99 copies that pattern to the device); with PMGX_AMG_DROP_ZEROS=1
- * pmgx_coarse_create_amg runs its SpMVs on the matrix without them.  out_*_h may be NULL (count only: *kept_h). */
+ * DOLFINx's assemble_matrix does (src/csr.hpp:66-99 copies that pattern to the device); pmgx_coarse_create_amg
+ * builds its hierarchy from that pattern and runs its level-0 SpMVs and transfers on copies without the zeros.
+ * out_*_h may be NULL (count only: *kept_h). */
 int pmgx_csr_drop_zeros_h(int n_rows, const int32_t* ptr_h, const int32_t* cols_h, const double* vals_h,
                           int32_t* out_ptr_h, int32_t* out_cols_h, double* out_vals_h, long long* kept_h);
 int pmgx_amg_num_levels(pmgx_amg_hier* h);

@@ -308,11 +308,9 @@ int pmgx_coarse_create_amg(pmgx_ctx* ctx, pmgx_operator* A, int max_iter, double
   // Stored zeros: the device assembly keeps the full pattern of the element matrices (27 entries per row at P1),
   // of which 7 (affine boxes, collocated quadrature) to 19 are non-zero.  The set-up below gets the pattern (its
   // aggregates follow it: 3 x 3 x 3 blocks); the SpMVs of the solve -- PCG and the level-0 smoother, the only ones
-  // that stream from HBM -- can run on a copy without the zeros: the same sums minus exact-zero products.
-  // Opt-in (PMGX_AMG_DROP_ZEROS=1): written after the round's GPU budget was spent, so only its host part is
-  // tested (tests/test_amg_setup.py) and its effect is a prediction (DESIGN.md section 8), not a measurement.
+  // that stream from HBM -- run on a copy without the zeros: the same sums minus exact-zero products.
   pmgx::amg::Csr Az;
-  if (getenv("PMGX_AMG_DROP_ZEROS") && atoi(getenv("PMGX_AMG_DROP_ZEROS")) == 1 && Ac->n_owned > 0)
+  if (Ac->n_owned > 0)
   {
     A0.n_rows = Ac->n_owned;
     A0.n_cols = Ac->n_owned + Ac->n_ghost;
@@ -345,11 +343,9 @@ int pmgx_coarse_create_amg(pmgx_ctx* ctx, pmgx_operator* A, int max_iter, double
   if (const char* e = getenv("PMGX_AMG_GAMMA_FROM"))
     M->gamma_from = std::max(atoi(e), 0);
   const bool use_lp = !(getenv("PMGX_AMG_LP") && atoi(getenv("PMGX_AMG_LP")) == 0);
-  // first level whose smoother runs the fused SpMV + Chebyshev kernels.  Measured at 1.59 M rows (coarse solve,
-  // 9 iterations): fused everywhere 7.56 ms, from level 1 on 7.08 ms, nowhere 7.25 ms -- on level 0 the
-  // epilogue's barrier shortens the streaming kernel's memory-level parallelism by more than the separate
-  // (L2-resident) vector pass costs; on the small levels the saved launches win.
-  const int fuse_from = getenv("PMGX_AMG_FUSE_FROM") ? atoi(getenv("PMGX_AMG_FUSE_FROM")) : 1;
+  // first level whose smoother runs the fused SpMV + Chebyshev kernels: every level.  Level 0's smoother runs
+  // the thread-per-row sliced-ELL twin, whose epilogue needs no barrier (DESIGN.md section 3.3)
+  const int fuse_from = getenv("PMGX_AMG_FUSE_FROM") ? atoi(getenv("PMGX_AMG_FUSE_FROM")) : 0;
   const int nl = (int)H.levels.size();
   M->lv.resize((size_t)nl);
   for (int l = 0; l < nl; ++l)
@@ -429,15 +425,16 @@ int pmgx_coarse_create_amg(pmgx_ctx* ctx, pmgx_operator* A, int max_iter, double
       D.sm->max_iter = (last && !L.dense) ? 4 * nu : (l == 0 ? nu : nu_coarse);
       D.sm->fuse = l >= fuse_from;
     }
-    // level 0 is the only level that does not fit the L2: its smoother streams the matrix with FP32
-    // values and 16-bit column deltas (PMGX_AMG_LP=0: the FP64 matrix)
+    // level 0's smoother streams the matrix with FP32 values and 16-bit column deltas (PMGX_AMG_LP=0: the FP64
+    // matrix)
     if (l == 0 && !last && use_lp)
       D.A_lp = pmgx::make_lp(static_cast<pmgx::CsrOperator*>(D.A));
     D.nnz_p = L.P.nnz();
     if (!last)
     {
-      D.P.upload(L.P, ctx->stream);
-      D.R.upload(L.R, ctx->stream);
+      // the transfers are smoothed with the full rows of A and carry its stored zeros as well (level 0's most)
+      D.P.upload(pmgx::amg::drop_stored_zeros(L.P), ctx->stream);
+      D.R.upload(pmgx::amg::drop_stored_zeros(L.R), ctx->stream);
     }
     else if (L.dense)
     {

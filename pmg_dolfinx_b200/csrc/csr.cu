@@ -252,17 +252,13 @@ __global__ void k_extract_diag_inv(int n_rows, const double* __restrict__ vals,
 // ---- reduced-storage sliced-ELL twin (CsrOperatorLP, csr.hpp): thread per row, 32-row slices
 constexpr int SLICE = 32;
 
-// y[row] = sum_k val[slice_ptr[s] + k*32 + lane] * x[col]; the slice width is read once per warp
+// sum_k val[slice_ptr[s] + k*32 + lane] * x[col] of the thread's row; the slice width is read once per warp
 template <bool D16>
-__global__ void __launch_bounds__(ST)
-k_spmv_sell(int n_rows, const long long* __restrict__ slice_ptr, const float* __restrict__ vals,
-            const int16_t* __restrict__ dcol, const int32_t* __restrict__ cols, const double* __restrict__ x,
-            double* __restrict__ y)
+__device__ __forceinline__ double sell_row(int row, int n_rows, const long long* __restrict__ slice_ptr,
+                                           const float* __restrict__ vals, const int16_t* __restrict__ dcol,
+                                           const int32_t* __restrict__ cols, const double* __restrict__ x)
 {
-  const int row = blockIdx.x * blockDim.x + threadIdx.x;
   const int s = row >> 5, lane = row & 31;
-  if (s >= (n_rows + SLICE - 1) / SLICE)
-    return;
   const long long b = slice_ptr[s];
   const int w = (int)((slice_ptr[s + 1] - b) >> 5);
   const float* v = vals + b + lane;
@@ -292,8 +288,43 @@ k_spmv_sell(int n_rows, const long long* __restrict__ slice_ptr, const float* __
     const int cc = D16 ? r + (int)__ldcs(d + k * SLICE) : __ldcs(c + k * SLICE);
     s0 = fma((double)vv, x[cc], s0);
   }
+  return s0 + s1;
+}
+
+template <bool D16>
+__global__ void __launch_bounds__(ST)
+k_spmv_sell(int n_rows, const long long* __restrict__ slice_ptr, const float* __restrict__ vals,
+            const int16_t* __restrict__ dcol, const int32_t* __restrict__ cols, const double* __restrict__ x,
+            double* __restrict__ y)
+{
+  const int row = blockIdx.x * blockDim.x + threadIdx.x;
+  if ((row >> 5) >= (n_rows + SLICE - 1) / SLICE)
+    return;
+  const double s = sell_row<D16>(row, n_rows, slice_ptr, vals, dcol, cols, x);
   if (row < n_rows)
-    y[row] = s0 + s1;
+    y[row] = s;
+}
+
+// the same SpMV with the Chebyshev update as its epilogue: each thread owns a whole row, so no barrier.  Rows that
+// also hold ghost columns (off_diag non-null: the operator has some) park their partial sum in e.scratch and are
+// finished by k_spmv_cheb_ghost_rows once the halo is in
+template <bool D16, int MODE>
+__global__ void __launch_bounds__(ST)
+k_spmv_sell_cheb(int n_rows, const long long* __restrict__ slice_ptr, const float* __restrict__ vals,
+                 const int16_t* __restrict__ dcol, const int32_t* __restrict__ cols,
+                 const int32_t* __restrict__ off_diag, const int32_t* __restrict__ row_ptr,
+                 const double* __restrict__ x, const ChebEp e)
+{
+  const int row = blockIdx.x * blockDim.x + threadIdx.x;
+  if ((row >> 5) >= (n_rows + SLICE - 1) / SLICE)
+    return;
+  const double s = sell_row<D16>(row, n_rows, slice_ptr, vals, dcol, cols, x);
+  if (row >= n_rows)
+    return;
+  if (off_diag && off_diag[row] < row_ptr[row + 1])
+    e.scratch[row] = s;
+  else
+    cheb_row<MODE>(row, s, x, e);
 }
 
 // rectangular FP64 sliced-ELL product y (+)= M x (the AMG prolongator: 1..8 entries per row, thread per row)
@@ -489,6 +520,30 @@ bool CsrOperator::apply_cheb(double* in, const ChebEp& e)
   return true;
 }
 
+namespace
+{
+template <bool D16>
+void launch_sell_cheb(const CsrOperatorLP* L, const double* x, const ChebEp& e)
+{
+  const CsrOperator* A = L->src;
+  const int grid = (L->n_slices * SLICE + ST - 1) / ST;
+  const int32_t* od = A->n_ghost_rows > 0 ? A->off_diag.p : nullptr;
+#define PMGX_SC(M)                                                                                                     \
+  k_spmv_sell_cheb<D16, M><<<grid, ST, 0, L->ctx->stream>>>(L->n_owned, L->slice_ptr.p, L->vals32.p, L->dcol16.p,       \
+                                                            L->cols32.p, od, A->row_ptr.p, x, e)
+  switch (e.mode)
+  {
+  case ChebEp::INIT: PMGX_SC(ChebEp::INIT); break;
+  case ChebEp::STEP: PMGX_SC(ChebEp::STEP); break;
+  case ChebEp::LAST: PMGX_SC(ChebEp::LAST); break;
+  default: PMGX_SC(ChebEp::XONLY); break;
+  }
+#undef PMGX_SC
+  check_launch("k_spmv_sell_cheb");
+  count_launch(L->ctx);
+}
+} // namespace
+
 void CsrOperatorLP::apply(double* x, double* y)
 {
   cudaSetDevice(ctx->device);
@@ -517,6 +572,28 @@ void CsrOperatorLP::apply(double* x, double* y)
     check_launch("k_spmv_ghost_rows");
     count_launch(ctx);
   }
+}
+
+// fused apply + Chebyshev update, split like CsrOperator::apply_cheb: the owned block (overlapping the halo)
+// finishes the rows without ghost columns, the FP64 ghost block of src finishes the others behind the exchange
+bool CsrOperatorLP::apply_cheb(double* in, const ChebEp& e)
+{
+  cudaSetDevice(ctx->device);
+  PMGX_REQUIRE(src->n_ghost_rows == 0 || e.scratch, "apply_cheb: scratch vector missing");
+  if (halo)
+    halo_fwd_begin(halo, in);
+  if (n_owned > 0)
+  {
+    if (d16)
+      launch_sell_cheb<true>(this, in, e);
+    else
+      launch_sell_cheb<false>(this, in, e);
+  }
+  if (halo)
+    halo_fwd_end(halo, in);
+  if (src->n_ghost_rows > 0)
+    launch_ghost_rows_cheb(src, in, e);
+  return true;
 }
 
 CsrOperatorLP* make_lp(CsrOperator* A)

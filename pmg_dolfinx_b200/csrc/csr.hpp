@@ -40,6 +40,8 @@ struct CsrOperatorLP : pmgx_operator
   DevBuf<int16_t> dcol16;      // col - row (d16) ...
   DevBuf<int32_t> cols32;      // ... or the column itself
   void apply(double* x, double* y) override;
+  bool supports_cheb_fusion() const override { return true; }
+  bool apply_cheb(double* in, const ChebEp& e) override;
 };
 CsrOperatorLP* make_lp(CsrOperator* A);
 } // namespace pmgx

@@ -148,9 +148,21 @@ int pmgx_vec_norm(pmgx_ctx* ctx, const double* a, long long n, int linf, double*
                                      in place take effect at the next apply; the diagonal is still computed once at
                                      create.  No affinity test runs (is_affine() is 0); PMGX_LAP_STREAM_G has no
                                      effect with it; PMGX_LAP_LITERAL_DETJ and PMGX_LAP_NO_DIAG apply as usual. */
+#define PMGX_LAP_GEOM_Q2 16       /* second-order (27-node, triquadratic) geometry: geom_dofmap[n_cells][27] and xgeom
+                                     holds the geometry node coordinates.  Node k = 9a + 3b + c, a, b, c in {0, 1, 2}
+                                     at reference coordinates {0, 1/2, 1} along (x, y, z): the lexicographic
+                                     extension of the trilinear order 4a + 2b + c, with the 8 corners at k = 0, 2,
+                                     6, 8, 18, 20, 24, 26.  G and det J are formed at the GLL points from the
+                                     quadratic map.  A cell is affine when all 27 nodes sit at v000 + (a/2) e1 +
+                                     (b/2) e2 + (c/2) e3 (tolerance 1e-13 of the longest edge); a mesh of such cells
+                                     runs the same affine kernel as its 8-node form, any other mesh the streamed-G
+                                     kernel.  PMGX_LAP_LITERAL_DETJ, PMGX_LAP_NO_DIAG and PMGX_LAP_STREAM_G keep their
+                                     meaning; with PMGX_LAP_RECOMPUTE_G create fails with PMGX_ERR_UNSUPPORTED (the
+                                     recompute apply kernels form trilinear Jacobians only). */
 
 /* MatFreeLaplacian ctor (src/laplacian.hpp:289-349).  dofmap[n_cells][(P+1)^3],
- * xgeom[n_points][3], geom_dofmap[n_cells][8] (tensor-product vertex order),
+ * xgeom[n_points][3], geom_dofmap[n_cells][8] (tensor-product vertex order; [n_cells][27] with
+ * PMGX_LAP_GEOM_Q2),
  * kappa[n_cells] (read on every apply, like cell_constants :230), lcells_h/bcells_h:
  * host lists (src/mesh.hpp:105-143), bc_marker[n_owned+n_ghost].  The 1-D GLL table,
  * the trilinear geometry table and the weights (dphi_geometry / G_weights arguments of
@@ -392,6 +404,17 @@ int pmgx_boxmesh_fit(long long ndofs_total, int order, int* nxyz_h);
 int pmgx_ghostmesh_create(int rank, int nranks, long long n_cells, const long long* cell_vertices_h,
                           const int* cell_owner_h, long long n_vertices, const double* coords_h,
                           pmgx_ghostmesh** out);
+/* The same for second-order (27-node) hexahedra: cell_nodes_h[n_cells][27] global node ids in the order of
+ * PMGX_LAP_GEOM_Q2 (k = 9a + 3b + c), coords_h[n_nodes][3].  Topology -- ghosting by vertex sharing, lcells /
+ * bcells, dof numbering and orientation -- uses the 8 corner nodes only; every node keeps its place in its cell's
+ * tensor-product frame.  pmgx_ghostmesh_geometry then writes geom_dofmap_h[n_cells][27] (local node ids) and
+ * xgeom_h over all local nodes, and pmgx_ghostmesh_space computes dof coordinates through the quadratic map.
+ * Fails on node ids out of range and on a corner id repeated within a cell. */
+int pmgx_ghostmesh_create_q2(int rank, int nranks, long long n_cells, const long long* cell_nodes_h,
+                             const int* cell_owner_h, long long n_nodes, const double* coords_h,
+                             pmgx_ghostmesh** out);
+/* geometry nodes per cell of the mesh: 8 (pmgx_ghostmesh_create) or 27 (pmgx_ghostmesh_create_q2) */
+int pmgx_ghostmesh_nodes_per_cell(pmgx_ghostmesh* m);
 int pmgx_ghostmesh_destroy(pmgx_ghostmesh* m);
 int pmgx_ghostmesh_sizes(pmgx_ghostmesh* m, long long* out_h);
 int pmgx_ghostmesh_geometry(pmgx_ghostmesh* m, double* xgeom_h, int32_t* geom_dofmap_h, long long* cell_gid_h);
@@ -411,7 +434,9 @@ int pmgx_laplacian_rhs(pmgx_operator* lap, const double* fvals, double g, double
  * fem::locate_dofs_topological on the host in the reference, examples/pmg/main.cpp:173-185): marker_out[i] = 1
  * for every dof on a facet that belongs to exactly one cell, owned and ghost entries alike.  geom_dofmap
  * [n_cells][8] (tp vertex order), dofmap[n_cells][(P+1)^3] are device arrays over the owned + ghost cells of
- * a ghost-layer mesh (src/mesh.hpp:16-98); halo: the forward-scatter plan of the space (NULL on one rank) --
+ * a ghost-layer mesh (src/mesh.hpp:16-98); for a 27-node (PMGX_LAP_GEOM_Q2) mesh pass its corner columns
+ * 0, 2, 6, 8, 18, 20, 24, 26, which are the 8-vertex map in this order; halo: the forward-scatter plan of the
+ * space (NULL on one rank) --
  * facet counts are exact for owned dofs, the ghost entries are taken from their owners.  COLLECTIVE like any
  * halo update. */
 int pmgx_bc_marker_exterior(pmgx_ctx* ctx, int degree, int n_cells, const int32_t* geom_dofmap,

@@ -292,6 +292,8 @@ protected:
 /// batch_size > 0 selects the reference's recompute mode (src/laplacian.hpp:383-396) through
 /// PMGX_LAP_RECOMPUTE_G: the operator keeps no geometry and every apply forms it inside the kernel
 /// from xgeom.  Nothing is stored per batch, so the value itself only selects the mode.
+/// A geometry dofmap with 27 entries per cell is second-order geometry (PMGX_LAP_GEOM_Q2, node order
+/// 9a + 3b + c; see INTEGRATION.md for the permutation from DOLFINx's); it does not combine with batch_size > 0.
 template <typename T>
 class MatFreeLaplacian : public OperatorBase
 {
@@ -308,6 +310,9 @@ public:
   {
     if (degree < 1 || degree > PMGX_MAX_DEGREE)
       throw std::runtime_error("Unsupported degree");
+    const std::size_t n_cells = dofmap.size() / ((degree + 1) * (degree + 1) * (degree + 1));
+    if (n_cells > 0 && geometry_dofmap.size() == 27 * n_cells)
+      flags |= PMGX_LAP_GEOM_Q2;
   }
 
 protected:

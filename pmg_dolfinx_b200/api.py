@@ -23,6 +23,17 @@ LAP_LITERAL_DETJ = 1   # detJ expression of the reference verbatim (quirk Q17)
 LAP_NO_DIAG = 2        # skip the matrix-free diagonal at create
 LAP_STREAM_G = 4       # stream the per-quadrature-point G even when every cell is affine
 LAP_RECOMPUTE_G = 8    # keep no geometry; every apply recomputes G from xgeom (the reference's batch_size > 0)
+LAP_GEOM_Q2 = 16       # 27-node (triquadratic) geometry: geometry_dofmap [n_cells, 27], node k = 9a + 3b + c
+
+# the 8 corner nodes of a 27-node cell, in the trilinear vertex order 4a + 2b + c
+Q2_CORNERS = (0, 2, 6, 8, 18, 20, 24, 26)
+
+
+def corner_columns(geometry_dofmap):
+    """The 8-vertex geometry dofmap of a 27-node one (numpy array or torch tensor of shape [n_cells, 27]), e.g. for
+    exterior_bc_marker."""
+    g = geometry_dofmap.reshape(-1, 27)[:, list(Q2_CORNERS)]
+    return g.contiguous() if isinstance(g, torch.Tensor) else np.ascontiguousarray(g)
 
 
 def _np(a, dtype):
@@ -167,20 +178,25 @@ class GhostLayerMesh:
     """General conforming hex mesh + partition -> this rank's arrays (pmgx_ghostmesh_*): the stand-in for
     create_mesh + ghost_layer_mesh + compute_boundary_cells + dofmaps + BC marker + Scatterer lists of
     examples/pmg/main.cpp:199-256 / src/mesh.hpp:16-143 for meshes that are not lexicographic boxes.
-    Same attribute surface as BoxMesh."""
+    Same attribute surface as BoxMesh.  ``cell_vertices`` of shape [n, 27] is a second-order mesh (node order of
+    LAP_GEOM_Q2; pmgx_ghostmesh_create_q2): geom_dofmap is then [n_cells, 27], and nodes_per_cell is 27."""
 
     def __init__(self, cell_vertices, cell_owner, coords, rank=0, nranks=1):
-        cv = _np(cell_vertices, np.int64).reshape(-1, 8)
+        cv = _np(cell_vertices, np.int64)
+        npc = 27 if cv.ndim == 2 and cv.shape[1] == 27 else 8
+        cv = cv.reshape(-1, npc)
         ow = _np(cell_owner, np.int32)
         xs = _np(coords, np.float64).reshape(-1, 3)
         h = ctypes.c_void_p()
-        check(lib.pmgx_ghostmesh_create(rank, nranks, len(cv), ptr(cv), ptr(ow), len(xs), ptr(xs), ctypes.addressof(h)))
+        create = lib.pmgx_ghostmesh_create_q2 if npc == 27 else lib.pmgx_ghostmesh_create
+        check(create(rank, nranks, len(cv), ptr(cv), ptr(ow), len(xs), ptr(xs), ctypes.addressof(h)))
         self.h, self.rank, self.nranks = h, rank, nranks
+        self.nodes_per_cell = int(lib.pmgx_ghostmesh_nodes_per_cell(self.h))
         s = np.zeros(5, dtype=np.int64)
         check(lib.pmgx_ghostmesh_sizes(self.h, ptr(s)))
         self.n_cells, self.n_owned_cells, self.n_points, nl, nb = (int(v) for v in s)
         self.xgeom = np.zeros((self.n_points, 3))
-        self.geom_dofmap = np.zeros((self.n_cells, 8), dtype=np.int32)
+        self.geom_dofmap = np.zeros((self.n_cells, self.nodes_per_cell), dtype=np.int32)
         self.cell_gid = np.zeros(self.n_cells, dtype=np.int64)
         check(lib.pmgx_ghostmesh_geometry(self.h, ptr(self.xgeom), ptr(self.geom_dofmap), ptr(self.cell_gid)))
         self.lcells = np.zeros(nl, dtype=np.int32)

@@ -18,6 +18,9 @@
 // launcher reads or generates the mesh on every rank), so entity numbering and ownership need no
 // communication.  Dof ownership: the lowest rank owning a cell that contains the dof's entity.
 // Local numbering: owned dofs by global id, then ghosts by (owner, global id).
+// Second-order (27-node) meshes (pmgx_ghostmesh_create_q2): the 8 corner nodes of every cell, renumbered densely in
+// node-id order, are the vertices of all of the above; the geometry keeps all 27 nodes of each cell in the cell's
+// own frame, and dof coordinates go through the triquadratic map.
 #include "common.hpp"
 
 #include <algorithm>
@@ -58,10 +61,12 @@ struct pmgx_ghostmesh
 {
   int rank = 0, nranks = 1;
   i64 n_cells_global = 0, n_vertices_global = 0;
+  int npc = 8;                  // geometry nodes per cell: 8, or 27 (pmgx_ghostmesh_create_q2)
   // global description (kept: spaces are built lazily per degree)
-  std::vector<i64> gcells;      // [ncg][8]
+  std::vector<i64> gcells;      // [ncg][8] vertex ids (the topology)
+  std::vector<i64> gnodes;      // [ncg][27] global node ids of a 27-node mesh (empty with 8 nodes: gcells)
   std::vector<int> gowner;      // [ncg]
-  std::vector<double> gcoords;  // [nvg][3]
+  std::vector<double> gcoords;  // [n_nodes][3], indexed by node id (the vertex id of an 8-node mesh)
   std::vector<uint64_t> vranks; // per global vertex: bit q set iff a cell owned by q contains it
   // global entity tables
   std::vector<uint64_t> edges;  // sorted unique (vmin << 32 | vmax)
@@ -71,8 +76,8 @@ struct pmgx_ghostmesh
   // local part
   std::vector<i64> cells;       // global id of each local cell: owned first, then ghosts by (owner, id)
   i64 n_owned_cells = 0;
-  std::vector<i64> lverts;      // global id of each local vertex
-  std::vector<int32_t> geom_dofmap; // [n_cells][8] local vertex ids
+  std::vector<i64> lverts;      // global node id of each local geometry node
+  std::vector<int32_t> geom_dofmap; // [n_cells][npc] local geometry node ids
   std::vector<int32_t> lcells, bcells;
   std::map<int, std::unique_ptr<GSpace>> spaces;
 
@@ -87,6 +92,7 @@ struct pmgx_ghostmesh
     return std::lower_bound(faces.begin(), faces.end(), k) - faces.begin();
   }
 
+  const i64* cell_nodes(i64 c) const { return npc == 8 ? &gcells[(size_t)c * 8] : &gnodes[(size_t)c * 27]; }
   GSpace& space(int P);
 };
 
@@ -244,12 +250,12 @@ GSpace& pmgx_ghostmesh::space(int P)
   s.dofmap.resize(gdof.size());
   for (size_t i = 0; i < gdof.size(); ++i)
     s.dofmap[i] = g2l[gdof[i]];
-  // dof coordinates: trilinear map of the first local cell that holds the dof
+  // dof coordinates: trilinear (8 nodes) or triquadratic (27 nodes) map of the first local cell that holds the dof
   s.coords.assign((size_t)nl * 3, 0.0);
   std::vector<char> have((size_t)nl, 0);
   for (i64 lc = 0; lc < nc; ++lc)
   {
-    const i64* cv = &gcells[(size_t)cells[lc] * 8];
+    const i64* cv = cell_nodes(cells[lc]);
     for (int a = 0; a < n3; ++a)
     {
       const int32_t d = s.dofmap[(size_t)lc * n3 + a];
@@ -257,12 +263,28 @@ GSpace& pmgx_ghostmesh::space(int P)
         continue;
       have[d] = 1;
       const double xi[3] = {pts[a / (n * n)], pts[(a / n) % n], pts[a % n]};
-      for (int k = 0; k < 8; ++k)
+      if (npc == 8)
+        for (int k = 0; k < 8; ++k)
+        {
+          const int ka = (k >> 2) & 1, kb = (k >> 1) & 1, kc = k & 1;
+          const double w = (ka ? xi[0] : 1 - xi[0]) * (kb ? xi[1] : 1 - xi[1]) * (kc ? xi[2] : 1 - xi[2]);
+          for (int dd = 0; dd < 3; ++dd)
+            s.coords[(size_t)d * 3 + dd] += w * gcoords[(size_t)cv[k] * 3 + dd];
+        }
+      else
       {
-        const int ka = (k >> 2) & 1, kb = (k >> 1) & 1, kc = k & 1;
-        const double w = (ka ? xi[0] : 1 - xi[0]) * (kb ? xi[1] : 1 - xi[1]) * (kc ? xi[2] : 1 - xi[2]);
-        for (int dd = 0; dd < 3; ++dd)
-          s.coords[(size_t)d * 3 + dd] += w * gcoords[(size_t)cv[k] * 3 + dd];
+        double l[3][3]; // quadratic Lagrange basis on {0, 1/2, 1} at xi[dir]
+        for (int dir = 0; dir < 3; ++dir)
+        {
+          const double t = xi[dir];
+          l[dir][0] = (2 * t - 1) * (t - 1), l[dir][1] = 4 * t * (1 - t), l[dir][2] = t * (2 * t - 1);
+        }
+        for (int k = 0; k < 27; ++k)
+        {
+          const double w = l[0][k / 9] * l[1][(k / 3) % 3] * l[2][k % 3];
+          for (int dd = 0; dd < 3; ++dd)
+            s.coords[(size_t)d * 3 + dd] += w * gcoords[(size_t)cv[k] * 3 + dd];
+        }
       }
     }
   }
@@ -319,26 +341,15 @@ GSpace& pmgx_ghostmesh::space(int P)
   return ref;
 }
 
-extern "C"
+namespace
 {
-int pmgx_ghostmesh_create(int rank, int nranks, long long n_cells, const long long* cell_vertices_h,
-                          const int* cell_owner_h, long long n_vertices, const double* coords_h,
-                          pmgx_ghostmesh** out)
+// Everything after the global vertex table M->gcells [n_cells][8] (vertex ids < n_vertices), M->gowner and
+// M->gcoords are in place; fills the entity tables, the local cells and the local geometry of M->npc nodes per cell.
+void build_ghostmesh(pmgx_ghostmesh* M, i64 n_vertices)
 {
-  PMGX_API_BEGIN
-  PMGX_REQUIRE(out && cell_vertices_h && cell_owner_h && coords_h, "ghostmesh_create: null argument");
-  PMGX_REQUIRE(nranks >= 1 && nranks <= 64 && rank >= 0 && rank < nranks, "ghostmesh_create: bad rank (1..64 ranks)");
-  PMGX_REQUIRE(n_cells >= 0 && n_vertices >= 0 && n_vertices < (1ll << 32), "ghostmesh_create: bad sizes");
-  std::unique_ptr<pmgx_ghostmesh> M(new pmgx_ghostmesh());
-  M->rank = rank;
-  M->nranks = nranks;
-  M->n_cells_global = n_cells;
+  const int rank = M->rank, nranks = M->nranks, npc = M->npc;
+  const i64 n_cells = M->n_cells_global;
   M->n_vertices_global = n_vertices;
-  M->gcells.assign(cell_vertices_h, cell_vertices_h + n_cells * 8);
-  M->gowner.assign(cell_owner_h, cell_owner_h + n_cells);
-  M->gcoords.assign(coords_h, coords_h + n_vertices * 3);
-  for (i64 v : M->gcells)
-    PMGX_REQUIRE(v >= 0 && v < n_vertices, "ghostmesh_create: vertex id out of range");
   for (int o : M->gowner)
     PMGX_REQUIRE(o >= 0 && o < nranks, "ghostmesh_create: cell owner out of range");
   // which ranks touch each vertex; vertex owner = lowest of them
@@ -440,21 +451,21 @@ int pmgx_ghostmesh_create(int rank, int nranks, long long n_cells, const long lo
   std::sort(ghosts.begin(), ghosts.end());
   for (auto& g : ghosts)
     M->cells.push_back(g.second);
-  // local vertices (first-touch order) and the geometry dofmap
+  // local geometry nodes (first-touch order) and the geometry dofmap
   {
     std::map<i64, int32_t> vmap;
-    M->geom_dofmap.resize(M->cells.size() * 8);
+    M->geom_dofmap.resize(M->cells.size() * npc);
     for (size_t lc = 0; lc < M->cells.size(); ++lc)
-      for (int k = 0; k < 8; ++k)
+      for (int k = 0; k < npc; ++k)
       {
-        const i64 v = M->gcells[(size_t)M->cells[lc] * 8 + k];
+        const i64 v = M->cell_nodes(M->cells[lc])[k];
         auto it = vmap.find(v);
         if (it == vmap.end())
         {
           it = vmap.emplace(v, (int32_t)M->lverts.size()).first;
           M->lverts.push_back(v);
         }
-        M->geom_dofmap[lc * 8 + k] = it->second;
+        M->geom_dofmap[lc * npc + k] = it->second;
       }
   }
   // lcells / bcells (src/mesh.hpp:119-138): an owned cell is local iff every vertex of it is owned by this rank
@@ -465,9 +476,81 @@ int pmgx_ghostmesh_create(int rank, int nranks, long long n_cells, const long lo
       local = M->vertex_owner[M->gcells[(size_t)M->cells[lc] * 8 + k]] == rank;
     (local ? M->lcells : M->bcells).push_back((int32_t)lc);
   }
+}
+
+void check_create_args(int rank, int nranks, long long n_cells, const long long* cells_h, const int* cell_owner_h,
+                       long long n_nodes, const double* coords_h, pmgx_ghostmesh** out)
+{
+  PMGX_REQUIRE(out && cells_h && cell_owner_h && coords_h, "ghostmesh_create: null argument");
+  PMGX_REQUIRE(nranks >= 1 && nranks <= 64 && rank >= 0 && rank < nranks, "ghostmesh_create: bad rank (1..64 ranks)");
+  PMGX_REQUIRE(n_cells >= 0 && n_nodes >= 0 && n_nodes < (1ll << 32), "ghostmesh_create: bad sizes");
+}
+} // namespace
+
+extern "C"
+{
+int pmgx_ghostmesh_create(int rank, int nranks, long long n_cells, const long long* cell_vertices_h,
+                          const int* cell_owner_h, long long n_vertices, const double* coords_h,
+                          pmgx_ghostmesh** out)
+{
+  PMGX_API_BEGIN
+  check_create_args(rank, nranks, n_cells, cell_vertices_h, cell_owner_h, n_vertices, coords_h, out);
+  std::unique_ptr<pmgx_ghostmesh> M(new pmgx_ghostmesh());
+  M->rank = rank;
+  M->nranks = nranks;
+  M->n_cells_global = n_cells;
+  M->gcells.assign(cell_vertices_h, cell_vertices_h + n_cells * 8);
+  M->gowner.assign(cell_owner_h, cell_owner_h + n_cells);
+  M->gcoords.assign(coords_h, coords_h + n_vertices * 3);
+  for (i64 v : M->gcells)
+    PMGX_REQUIRE(v >= 0 && v < n_vertices, "ghostmesh_create: vertex id out of range");
+  build_ghostmesh(M.get(), n_vertices);
   *out = M.release();
   PMGX_API_END
 }
+
+int pmgx_ghostmesh_create_q2(int rank, int nranks, long long n_cells, const long long* cell_nodes_h,
+                             const int* cell_owner_h, long long n_nodes, const double* coords_h,
+                             pmgx_ghostmesh** out)
+{
+  PMGX_API_BEGIN
+  check_create_args(rank, nranks, n_cells, cell_nodes_h, cell_owner_h, n_nodes, coords_h, out);
+  std::unique_ptr<pmgx_ghostmesh> M(new pmgx_ghostmesh());
+  M->rank = rank;
+  M->nranks = nranks;
+  M->npc = 27;
+  M->n_cells_global = n_cells;
+  M->gnodes.assign(cell_nodes_h, cell_nodes_h + n_cells * 27);
+  M->gowner.assign(cell_owner_h, cell_owner_h + n_cells);
+  M->gcoords.assign(coords_h, coords_h + n_nodes * 3);
+  for (i64 v : M->gnodes)
+    PMGX_REQUIRE(v >= 0 && v < n_nodes, "ghostmesh_create_q2: node id out of range");
+  // the corners, node k = 18a + 6b + 2c for vertex 4a + 2b + c, renumbered densely in node-id order: the order
+  // that fixes the entity frames is the node order, so every rank derives the same numbering
+  static const int corner[8] = {0, 2, 6, 8, 18, 20, 24, 26};
+  std::vector<i64> vid((size_t)n_nodes, -1);
+  for (i64 c = 0; c < n_cells; ++c)
+    for (int k = 0; k < 8; ++k)
+    {
+      const i64 v = M->gnodes[(size_t)c * 27 + corner[k]];
+      for (int j = 0; j < k; ++j)
+        PMGX_REQUIRE(M->gnodes[(size_t)c * 27 + corner[j]] != v, "ghostmesh_create_q2: cell %lld repeats corner node %lld", c, v);
+      vid[v] = 0;
+    }
+  i64 nv = 0;
+  for (i64& v : vid)
+    if (v == 0)
+      v = nv++;
+  M->gcells.resize((size_t)n_cells * 8);
+  for (i64 c = 0; c < n_cells; ++c)
+    for (int k = 0; k < 8; ++k)
+      M->gcells[(size_t)c * 8 + k] = vid[M->gnodes[(size_t)c * 27 + corner[k]]];
+  build_ghostmesh(M.get(), nv);
+  *out = M.release();
+  PMGX_API_END
+}
+
+int pmgx_ghostmesh_nodes_per_cell(pmgx_ghostmesh* m) { return m ? m->npc : -1; }
 
 int pmgx_ghostmesh_destroy(pmgx_ghostmesh* m)
 {

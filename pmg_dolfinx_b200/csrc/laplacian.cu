@@ -374,6 +374,143 @@ __global__ void k_cell_geometry(const double* __restrict__ xgeom, const int32_t*
   g[5] = (K[2][0] * K[2][0] + K[2][1] * K[2][1] + K[2][2] * K[2][2]) * s;
 }
 
+// ------------------------------------------------------ geometry of the 27-node hexahedron --
+// PMGX_LAP_GEOM_Q2: the triquadratic map x(xi) = sum_k x_k L_a(xi) L_b(eta) L_c(zeta) with node k = 9a + 3b + c at
+// reference coordinates {0, 1/2, 1}^3.  The corners are k = 18a' + 6b' + 2c' for the trilinear vertex (a',b',c').
+constexpr int Q2_NODES = 27;
+
+// the quadratic Lagrange basis on {0, 1/2, 1} and its derivative at t
+__device__ __forceinline__ void q2_basis(double t, double (&l)[3], double (&d)[3])
+{
+  l[0] = (2.0 * t - 1.0) * (t - 1.0);
+  l[1] = 4.0 * t * (1.0 - t);
+  l[2] = t * (2.0 * t - 1.0);
+  d[0] = 4.0 * t - 3.0;
+  d[1] = 4.0 - 8.0 * t;
+  d[2] = 4.0 * t - 1.0;
+}
+
+// J at xi of the cell whose node coordinates are X(k, i), by sum factorisation over the 3 x 3 x 3 basis: the zeta
+// direction first (value and derivative), then eta, then xi.
+template <typename Nodes>
+__device__ __forceinline__ void jacobian_q2(const Nodes& X, const double (&xi)[3], double (&J)[3][3])
+{
+  double la[3], da[3], lb[3], db[3], lc[3], dc[3];
+  q2_basis(xi[0], la, da);
+  q2_basis(xi[1], lb, db);
+  q2_basis(xi[2], lc, dc);
+#pragma unroll
+  for (int i = 0; i < 3; ++i)
+  {
+    double j0 = 0.0, j1 = 0.0, j2 = 0.0;
+#pragma unroll
+    for (int a = 0; a < 3; ++a)
+    {
+      double u = 0.0, ueta = 0.0, uzeta = 0.0; // sum_bc x L_b L_c, x L_b' L_c, x L_b L_c'
+#pragma unroll
+      for (int b = 0; b < 3; ++b)
+      {
+        double s = 0.0, t = 0.0; // sum_c x L_c, x L_c'
+#pragma unroll
+        for (int c = 0; c < 3; ++c)
+        {
+          const double x = X(9 * a + 3 * b + c, i);
+          s = fma(x, lc[c], s);
+          t = fma(x, dc[c], t);
+        }
+        u = fma(s, lb[b], u);
+        ueta = fma(s, db[b], ueta);
+        uzeta = fma(t, lb[b], uzeta);
+      }
+      j0 = fma(u, da[a], j0);
+      j1 = fma(ueta, la[a], j1);
+      j2 = fma(uzeta, la[a], j2);
+    }
+    J[i][0] = j0, J[i][1] = j1, J[i][2] = j2;
+  }
+}
+
+// G (WRITE_G) or w |det J| at every quadrature point of the 27-node cells.  One warp per launch position: the warp
+// stages the cell's 27 x 3 coordinates in shared memory once, then each lane forms J at its points from the staged
+// copy and G = w K K^T / det J through the same helpers as every other path.
+constexpr int Q2_GEOM_WARPS = 8;
+template <bool WRITE_G>
+__global__ void __launch_bounds__(32 * Q2_GEOM_WARPS)
+    k_geometry_q2(int P, const double* __restrict__ xgeom, const int32_t* __restrict__ geom_dofmap,
+                  const int32_t* __restrict__ perm, double* __restrict__ G, double* __restrict__ detj_w, int n_list,
+                  bool literal_detj, Lay lay)
+{
+  __shared__ double nodes[Q2_GEOM_WARPS][Q2_NODES * 3];
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  double* xs = nodes[warp];
+  const auto X = [xs](int k, int i) { return xs[3 * k + i]; };
+  const int n = P + 1, n2 = n * n, n3 = n2 * n;
+  const long long stride = (long long)gridDim.x * Q2_GEOM_WARPS;
+  for (long long p = (long long)blockIdx.x * Q2_GEOM_WARPS + warp; p < n_list; p += stride)
+  {
+    const int32_t* gd = geom_dofmap + (long long)perm[p] * Q2_NODES;
+    for (int e = lane; e < Q2_NODES * 3; e += 32)
+      xs[e] = xgeom[3ll * gd[e / 3] + e % 3];
+    __syncwarp();
+    for (int q = lane; q < n3; q += 32)
+    {
+      const int ix = q / n2, iy = (q / n) % n, iz = q % n;
+      const double xi[3] = {c_pts[P][ix], c_pts[P][iy], c_pts[P][iz]};
+      const double w = c_wts[P][ix] * c_wts[P][iy] * c_wts[P][iz];
+      double J[3][3], K[3][3];
+      jacobian_q2(X, xi, J);
+      const double detJ = adjugate_det(J, literal_detj, K);
+      if (WRITE_G)
+      {
+        double g[6];
+        g_from_adjugate(K, w / detJ, g);
+#pragma unroll
+        for (int c = 0; c < 6; ++c)
+          G[lay.g_index(p, c, q)] = g[c];
+      }
+      else
+        detj_w[p * n3 + q] = w * fabs(detJ);
+    }
+    __syncwarp(); // the next cell overwrites xs
+  }
+}
+
+// Per cell: Gc = K K^T / det J of the triquadratic map at the cell centre (weight 1), and the affinity test: a cell is
+// affine iff every node equals v000 + (a/2) e1 + (b/2) e2 + (c/2) e3 (e1, e2, e3 the edges from v000), measured
+// against the longest edge like k_cell_geometry.  One thread per launch position.
+__global__ void k_cell_geometry_q2(const double* __restrict__ xgeom, const int32_t* __restrict__ geom_dofmap,
+                                   const int32_t* __restrict__ perm, double* __restrict__ Gc, int n_list,
+                                   bool literal_detj, double tol, int* __restrict__ n_nonaffine)
+{
+  const int p = blockIdx.x * blockDim.x + threadIdx.x;
+  if (p >= n_list)
+    return;
+  const int32_t* gd = geom_dofmap + (long long)perm[p] * Q2_NODES;
+  const auto X = [xgeom, gd](int k, int i) { return xgeom[3ll * gd[k] + i]; };
+  double scale = 0.0, dev = 0.0;
+#pragma unroll
+  for (int i = 0; i < 3; ++i)
+  {
+    const double v0 = X(0, i), e1 = X(18, i) - v0, e2 = X(6, i) - v0, e3 = X(2, i) - v0;
+    scale = fmax(scale, fmax(fabs(e1), fmax(fabs(e2), fabs(e3))));
+    for (int k = 1; k < Q2_NODES; ++k)
+    {
+      const int a = k / 9, b = (k / 3) % 3, c = k % 3;
+      dev = fmax(dev, fabs(X(k, i) - (v0 + 0.5 * (a * e1 + b * e2 + c * e3))));
+    }
+  }
+  if (!(dev <= tol * scale))
+    atomicAdd(n_nonaffine, 1);
+  const double centre[3] = {0.5, 0.5, 0.5};
+  double J[3][3], K[3][3], g[6];
+  jacobian_q2(X, centre, J);
+  const double detJ = adjugate_det(J, literal_detj, K);
+  g_from_adjugate(K, 1.0 / detJ, g);
+#pragma unroll
+  for (int c = 0; c < 6; ++c)
+    Gc[(size_t)p * 6 + c] = g[c];
+}
+
 // Per-thread factored Jacobians of the apply kernels that recompute G.  Along a line of fixed (eta, zeta) (a
 // column thread, an mma lane): dx/dxi is constant, dx/deta and dx/dzeta are affine in xi -- 15 coefficients, 6 FMAs
 // per point.
@@ -2070,6 +2207,7 @@ struct Laplacian : pmgx_operator
   DevBuf<double> Gc;   // [n_list][6] per-cell geometry factor of affine cells
   bool affine = false; // every cell affine: ApplyKernels<P>::Affine replaces the streamed-G kernel
   bool recompute = false; // PMGX_LAP_RECOMPUTE_G: no G, no Gc; every user of G forms it from xgeom
+  bool q2 = false;        // PMGX_LAP_GEOM_Q2: 27 geometry nodes per cell
 
   int n_list() const { return n_l + n_b; }
   pmgx::ApplyGeometry geometry() const
@@ -2136,6 +2274,12 @@ int pmgx_laplacian_create(pmgx_ctx* ctx, int degree, int n_cells, const int32_t*
   PMGX_REQUIRE(n_owned >= 0 && n_ghost >= 0 && n_points >= 0, "laplacian_create: bad sizes");
   PMGX_REQUIRE(!halo || (halo->n_owned == n_owned && halo->n_ghost == n_ghost),
                "laplacian_create: halo does not match the vector layout");
+  if ((flags & PMGX_LAP_GEOM_Q2) && (flags & PMGX_LAP_RECOMPUTE_G))
+  {
+    pmgx::set_error("laplacian_create: PMGX_LAP_GEOM_Q2 is not supported with PMGX_LAP_RECOMPUTE_G (the recompute "
+                    "apply kernels form trilinear Jacobians only)");
+    return PMGX_ERR_UNSUPPORTED;
+  }
   PMGX_CUDA(cudaSetDevice(ctx->device));
   pmgx::upload_tables(ctx);
 
@@ -2159,6 +2303,7 @@ int pmgx_laplacian_create(pmgx_ctx* ctx, int degree, int n_cells, const int32_t*
   L->dofmap_borrowed = dofmap;
   L->flags = flags;
   L->recompute = (flags & PMGX_LAP_RECOMPUTE_G) != 0;
+  L->q2 = (flags & PMGX_LAP_GEOM_Q2) != 0;
 
   const int n_list = L->n_list();
   std::vector<int32_t> perm_h((size_t)n_list);
@@ -2185,8 +2330,12 @@ int pmgx_laplacian_create(pmgx_ctx* ctx, int degree, int n_cells, const int32_t*
     pmgx::DevBuf<int> bad;
     bad.alloc(1);
     PMGX_CUDA(cudaMemsetAsync(bad.p, 0, sizeof(int), ctx->stream));
-    pmgx::k_cell_geometry<<<(n_list + 255) / 256, 256, 0, ctx->stream>>>(
-        xgeom, geom_dofmap, L->perm.p, L->Gc.p, n_list, (flags & PMGX_LAP_LITERAL_DETJ) != 0, 1e-13, bad.p);
+    if (L->q2)
+      pmgx::k_cell_geometry_q2<<<(n_list + 255) / 256, 256, 0, ctx->stream>>>(
+          xgeom, geom_dofmap, L->perm.p, L->Gc.p, n_list, (flags & PMGX_LAP_LITERAL_DETJ) != 0, 1e-13, bad.p);
+    else
+      pmgx::k_cell_geometry<<<(n_list + 255) / 256, 256, 0, ctx->stream>>>(
+          xgeom, geom_dofmap, L->perm.p, L->Gc.p, n_list, (flags & PMGX_LAP_LITERAL_DETJ) != 0, 1e-13, bad.p);
     pmgx::check_launch("k_cell_geometry");
     pmgx::count_launch(ctx);
     int n_bad = 0;
@@ -2221,7 +2370,14 @@ int pmgx_laplacian_create(pmgx_ctx* ctx, int degree, int n_cells, const int32_t*
         dofmap, L->perm.p, bc_marker, L->enc.p, L->n3, total, lay);
     pmgx::check_launch("k_encode_dofmap");
     pmgx::count_launch(ctx);
-    if (!L->recompute)
+    if (L->q2)
+    {
+      pmgx::k_geometry_q2<true><<<pmgx::setup_grid(ctx, 32ll * n_list), 32 * pmgx::Q2_GEOM_WARPS, 0, ctx->stream>>>(
+          degree, xgeom, geom_dofmap, L->perm.p, L->G.p, nullptr, n_list, (flags & PMGX_LAP_LITERAL_DETJ) != 0, lay);
+      pmgx::check_launch("k_geometry_q2");
+      pmgx::count_launch(ctx);
+    }
+    else if (!L->recompute)
     {
       pmgx::k_geometry<true><<<pmgx::setup_grid(ctx, total), 256, 0, ctx->stream>>>(
           degree, xgeom, geom_dofmap, L->perm.p, L->G.p, nullptr, n_list,
@@ -2318,8 +2474,12 @@ int pmgx_laplacian_rhs(pmgx_operator* op, const double* fvals, double g, double*
   {
     pmgx::DevBuf<double> dw;
     dw.alloc((size_t)total);
-    pmgx::k_geometry<false><<<pmgx::setup_grid(ctx, total), 256, 0, ctx->stream>>>(
-        L->P, L->xgeom, L->geom_dofmap, L->perm.p, nullptr, dw.p, L->n_list(), false, L->lay);
+    if (L->q2)
+      pmgx::k_geometry_q2<false><<<pmgx::setup_grid(ctx, 32ll * L->n_list()), 32 * pmgx::Q2_GEOM_WARPS, 0, ctx->stream>>>(
+          L->P, L->xgeom, L->geom_dofmap, L->perm.p, nullptr, dw.p, L->n_list(), false, L->lay);
+    else
+      pmgx::k_geometry<false><<<pmgx::setup_grid(ctx, total), 256, 0, ctx->stream>>>(
+          L->P, L->xgeom, L->geom_dofmap, L->perm.p, nullptr, dw.p, L->n_list(), false, L->lay);
     pmgx::check_launch("k_geometry(detJ)");
     pmgx::k_rhs<<<pmgx::setup_grid(ctx, total), 256, 0, ctx->stream>>>(dw.p, L->enc.p, fvals, b, total, L->n3, L->lay);
     pmgx::check_launch("k_rhs");
@@ -2370,7 +2530,7 @@ int pmgx_laplacian_lift(pmgx_operator* op, const double* gvals, double* b)
   const int rc = pmgx_laplacian_create(ctx, L->P, L->n_cells, L->dofmap_borrowed, L->xgeom, n_points_unknown, L->geom_dofmap,
                                        L->kappa, perm_h.data(), (int)perm_h.size(), nullptr, 0, nobc.p, L->n_owned,
                                        L->n_ghost, nullptr,
-                                       (L->flags & (PMGX_LAP_LITERAL_DETJ | PMGX_LAP_RECOMPUTE_G)) | PMGX_LAP_NO_DIAG,
+                                       (L->flags & (PMGX_LAP_LITERAL_DETJ | PMGX_LAP_RECOMPUTE_G | PMGX_LAP_GEOM_Q2)) | PMGX_LAP_NO_DIAG,
                                        &full);
   if (rc != PMGX_OK)
     return rc;

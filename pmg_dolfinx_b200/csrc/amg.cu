@@ -17,7 +17,6 @@
 #include "amg.hpp"
 
 #include <algorithm>
-#include <cstdlib>
 #include <cstring>
 
 namespace pmgx
@@ -111,9 +110,8 @@ pmgx_halo* make_halo(pmgx_ctx* c, int n_owned, int n_ghost, const amg::Plan& p)
                                   p.recv_idx.data(), &h);
   if (rc != PMGX_OK)
     throw Error{rc};
-  // latency-bound exchanges: stay on the compute stream (PMGX_AMG_SINGLE_STREAM=0: dual-stream like level 0)
-  static const bool ss = !(getenv("PMGX_AMG_SINGLE_STREAM") && atoi(getenv("PMGX_AMG_SINGLE_STREAM")) == 0);
-  h->single_stream = ss && h->p2p && h->n_send() + h->n_recv() <= 65536;
+  // latency-bound exchanges stay on the compute stream
+  h->single_stream = h->p2p && h->n_send() + h->n_recv() <= 65536;
   return h;
 }
 
@@ -132,7 +130,6 @@ struct AmgPrecond : Precond
     RectCsr R;                 // from this level to the next coarser one (rows of P^T: long rows, 32 lanes per row)
     RectSell P;                // back (short rows, thread per row)
     DevBuf<double> x, b;       // levels >= 1 (and the private b of a dense level)
-    DevBuf<double> x2, r2;     // second coarse visit of a W-cycle (levels >= 1)
     long long nnz_p = 0;
     bool dense = false;
     int n_global = 0;
@@ -148,8 +145,6 @@ struct AmgPrecond : Precond
   pmgx_ctx* ctx = nullptr;
   std::vector<Lv> lv;
   int nu = 2;
-  int gamma = 1; // cycle index: 1 = V, 2 = W (two coarse visits; the small levels are latency, not bandwidth)
-  int gamma_from = 0; // first level whose coarse level is visited gamma times
 
   ~AmgPrecond() override
   {
@@ -207,7 +202,7 @@ struct AmgPrecond : Precond
     if (C.repl_first)
     {
       // the next level lives completely on every rank: my part of b_c, all-gather, canonical order
-      spmv_rect(ctx, C.n_mine, L.R.ptr.p, L.R.cols.p, L.R.vals.p, L.sm->r.p, C.bg.p, false, 32);
+      spmv_rect(ctx, C.n_mine, L.R.ptr.p, L.R.cols.p, L.R.vals.p, L.sm->r.p, C.bg.p);
       halo_fwd_begin(C.repl_gather, C.bg.p);
       halo_fwd_end(C.repl_gather, C.bg.p);
       k_permute<<<(C.n_owned + 255) / 256, 256, 0, ctx->stream>>>(C.n_owned, C.perm.p, C.bg.p, C.b.p);
@@ -215,22 +210,14 @@ struct AmgPrecond : Precond
       count_launch(ctx);
     }
     else
-      spmv_rect(ctx, C.n_owned, L.R.ptr.p, L.R.cols.p, L.R.vals.p, L.sm->r.p, C.b.p, false, 32); // b_c = P^T r
+      spmv_rect(ctx, C.n_owned, L.R.ptr.p, L.R.cols.p, L.R.vals.p, L.sm->r.p, C.b.p); // b_c = P^T r
     cycle(l + 1, C.b.p, C.x.p);
-    if (gamma == 2 && l >= gamma_from && l + 2 < (int)lv.size())
-    {
-      // W-cycle: a second visit on the coarse residual, x_c += B_c (b_c - A_c x_c)  (symmetric: 2B - BAB)
-      C.A->apply(C.x.p, C.r2.p);
-      vec::axpy(ctx, C.r2.p, -1.0, C.r2.p, C.b.p, C.n_owned);
-      cycle(l + 1, C.r2.p, C.x2.p);
-      vec::axpy(ctx, C.x.p, 1.0, C.x2.p, C.x.p, C.n_owned);
-    }
     if (C.halo_v) // ... and P interpolates from the neighbours' aggregates
     {
       halo_fwd_begin(C.halo_v, C.x.p);
       halo_fwd_end(C.halo_v, C.x.p);
     }
-    spmv_sell_rect(ctx, L.n_owned, L.P.slice_ptr.p, L.P.cols.p, L.P.vals.p, C.x.p, x, true); // x += P x_c
+    spmv_sell_rect(ctx, L.n_owned, L.P.slice_ptr.p, L.P.cols.p, L.P.vals.p, C.x.p, x); // x += P x_c
     cheb_solve(L.sm, As, x, b, nullptr, false, CHEB_R_NONE);          // post-smoothing (same polynomial: M is symmetric)
   }
 
@@ -258,6 +245,20 @@ amg::Plan plan_of(pmgx_halo* h)
   if (!p.recv_idx.empty())
     PMGX_CUDA(cudaMemcpy(p.recv_idx.data(), h->recv_idx.p, p.recv_idx.size() * sizeof(int32_t), cudaMemcpyDeviceToHost));
   return p;
+}
+
+// device CSR operator of a host matrix whose rows are sorted by column (owned columns < n_owned come first)
+int csr_create(pmgx_ctx* c, const amg::Csr& M, int n_owned, int n_ghost, pmgx_halo* h, pmgx_operator** out)
+{
+  std::vector<int32_t> off((size_t)n_owned); // end of each row's owned-column block
+  for (int i = 0; i < n_owned; ++i)
+  {
+    int32_t j = M.ptr[i];
+    while (j < M.ptr[i + 1] && M.cols[j] < n_owned)
+      ++j;
+    off[i] = j;
+  }
+  return pmgx_csr_create(c, n_owned, n_ghost, M.ptr.data(), off.data(), M.cols.data(), M.vals.data(), h, out);
 }
 } // namespace
 } // namespace pmgx
@@ -334,18 +335,6 @@ int pmgx_coarse_create_amg(pmgx_ctx* ctx, pmgx_operator* A, int max_iter, double
   std::unique_ptr<AmgPrecond> M(new AmgPrecond());
   M->ctx = ctx;
   M->nu = nu;
-  // A/B switches (defaults are the measured winners, DESIGN.md section 3.3)
-  int nu_coarse = nu;
-  if (const char* e = getenv("PMGX_AMG_NU_COARSE"))
-    nu_coarse = std::min(std::max(atoi(e), 1), 8);
-  if (const char* e = getenv("PMGX_AMG_GAMMA"))
-    M->gamma = atoi(e) == 2 ? 2 : 1;
-  if (const char* e = getenv("PMGX_AMG_GAMMA_FROM"))
-    M->gamma_from = std::max(atoi(e), 0);
-  const bool use_lp = !(getenv("PMGX_AMG_LP") && atoi(getenv("PMGX_AMG_LP")) == 0);
-  // first level whose smoother runs the fused SpMV + Chebyshev kernels: every level.  Level 0's smoother runs
-  // the thread-per-row sliced-ELL twin, whose epilogue needs no barrier (DESIGN.md section 3.3)
-  const int fuse_from = getenv("PMGX_AMG_FUSE_FROM") ? atoi(getenv("PMGX_AMG_FUSE_FROM")) : 0;
   const int nl = (int)H.levels.size();
   M->lv.resize((size_t)nl);
   for (int l = 0; l < nl; ++l)
@@ -362,17 +351,8 @@ int pmgx_coarse_create_amg(pmgx_ctx* ctx, pmgx_operator* A, int max_iter, double
       D.halo_v = Ac->halo;
       if (!Az.ptr.empty())
       { // ... or its copy without the stored zeros (same halo, same vectors)
-        std::vector<int32_t> off((size_t)Ac->n_owned);
-        for (int i = 0; i < Ac->n_owned; ++i)
-        {
-          int32_t j = Az.ptr[i];
-          while (j < Az.ptr[i + 1] && Az.cols[j] < Ac->n_owned)
-            ++j;
-          off[i] = j;
-        }
         pmgx_operator* Acmp = nullptr;
-        const int rc = pmgx_csr_create(ctx, Ac->n_owned, Ac->n_ghost, Az.ptr.data(), off.data(), Az.cols.data(),
-                                       Az.vals.data(), Ac->halo, &Acmp);
+        const int rc = pmgx::csr_create(ctx, Az, Ac->n_owned, Ac->n_ghost, Ac->halo, &Acmp);
         if (rc != PMGX_OK)
           return rc;
         D.A = Acmp;
@@ -396,21 +376,12 @@ int pmgx_coarse_create_amg(pmgx_ctx* ctx, pmgx_operator* A, int max_iter, double
         PMGX_CUDA(cudaMemsetAsync(D.bg.p, 0, (size_t)std::max(L.n_owned, 1) * sizeof(double), ctx->stream));
         D.perm.upload(L.gather_perm.data(), L.gather_perm.size(), ctx->stream);
       }
-      std::vector<int32_t> off((size_t)L.n_owned);
-      for (int i = 0; i < L.n_owned; ++i)
-      {
-        int32_t j = L.A.ptr[i];
-        while (j < L.A.ptr[i + 1] && L.A.cols[j] < L.n_owned)
-          ++j;
-        off[i] = j;
-      }
-      const int rc = pmgx_csr_create(ctx, L.n_owned, L.n_ghost, L.A.ptr.data(), off.data(), L.A.cols.data(),
-                                     L.A.vals.data(), D.halo, &D.A);
+      const int rc = pmgx::csr_create(ctx, L.A, L.n_owned, L.n_ghost, D.halo, &D.A);
       if (rc != PMGX_OK)
         return rc;
       D.own_A = true;
       const size_t nt = (size_t)L.n_owned + L.n_ghost;
-      for (auto* buf : {&D.x, &D.b, &D.x2, &D.r2})
+      for (auto* buf : {&D.x, &D.b})
       {
         buf->alloc(nt);
         if (nt > 0)
@@ -422,12 +393,10 @@ int pmgx_coarse_create_amg(pmgx_ctx* ctx, pmgx_operator* A, int max_iter, double
       if (rc != PMGX_OK)
         return rc;
       // a coarsest level that could not be inverted densely is smoothed harder instead
-      D.sm->max_iter = (last && !L.dense) ? 4 * nu : (l == 0 ? nu : nu_coarse);
-      D.sm->fuse = l >= fuse_from;
+      D.sm->max_iter = (last && !L.dense) ? 4 * nu : nu;
     }
-    // level 0's smoother streams the matrix with FP32 values and 16-bit column deltas (PMGX_AMG_LP=0: the FP64
-    // matrix)
-    if (l == 0 && !last && use_lp)
+    // level 0's smoother streams the matrix with FP32 values and 16-bit column deltas (DESIGN.md section 3.3)
+    if (l == 0 && !last)
       D.A_lp = pmgx::make_lp(static_cast<pmgx::CsrOperator*>(D.A));
     D.nnz_p = L.P.nnz();
     if (!last)
@@ -458,8 +427,6 @@ int pmgx_coarse_create_amg(pmgx_ctx* ctx, pmgx_operator* A, int max_iter, double
     return rc;
   cs->M = M.release();
   cs->check_every = 1; // an iteration costs ~0.7 ms, a host look at r.M^-1 r ~10 us
-  if (const char* e = getenv("PMGX_COARSE_CHECK_EVERY"))
-    cs->check_every = std::max(atoi(e), 1);
   *out = cs;
   PMGX_API_END
 }

@@ -15,7 +15,7 @@ namespace
 constexpr int LPR = 8; // lanes per row
 constexpr int ST = 256;
 
-// y[i] (=|+=) sum_{j in [beg[i], end[i])} v[j] x[col[j]]: 8 lanes per row, one row per lane
+// y[i] = sum_{j in [beg[i], end[i])} v[j] x[col[j]]: 8 lanes per row, one row per lane
 // group.  Every lane keeps UNR independent (value, column) loads in flight, so the dependent
 // chain per row is three loads deep (row bounds -> columns/values -> x) and the matrix stream is
 // latency-hidden; values / columns are streamed once (evict-first) so that x and y stay in L2.
@@ -23,7 +23,6 @@ constexpr int ST = 256;
 // Fusing the CG inner products into this kernel was tried and dropped: a last-block ticket over
 // 49 k CTAs serialises on one atomic (234 us), a grid-stride version with few CTAs is latency-bound.
 constexpr int UNR = 4;
-template <bool ACCUM>
 __global__ void __launch_bounds__(ST)
 k_spmv(int n_rows, const double* __restrict__ vals, const int32_t* __restrict__ beg,
        const int32_t* __restrict__ end, const int32_t* __restrict__ cols,
@@ -57,7 +56,7 @@ k_spmv(int n_rows, const double* __restrict__ vals, const int32_t* __restrict__ 
   for (int o = LPR / 2; o > 0; o >>= 1)
     s += __shfl_xor_sync(0xffffffffu, s, o);
   if (row < n_rows && lane == 0)
-    y[row] = ACCUM ? y[row] + s : s;
+    y[row] = s;
 }
 
 // ghost-column block of the rows that have one (the rows of dofs on a partition interface):
@@ -116,11 +115,11 @@ __device__ __forceinline__ void cheb_row(int i, double q, const double* __restri
 
 // owned-column block; rows that also hold ghost columns park their partial sum in e.scratch and are
 // finished by k_spmv_cheb_ghost_rows once the halo is in
-template <typename VT, bool D16, int MODE>
+template <int MODE>
 __global__ void __launch_bounds__(ST)
-k_spmv_cheb(int n_rows, const VT* __restrict__ vals, const int32_t* __restrict__ beg, const int32_t* __restrict__ end,
-            const int32_t* __restrict__ row_ptr, const int16_t* __restrict__ dcol, const int32_t* __restrict__ cols,
-            const double* __restrict__ x, const ChebEp e)
+k_spmv_cheb(int n_rows, const double* __restrict__ vals, const int32_t* __restrict__ row_ptr,
+            const int32_t* __restrict__ end, const int32_t* __restrict__ cols, const double* __restrict__ x,
+            const ChebEp e)
 {
   const int gt = blockIdx.x * blockDim.x + threadIdx.x;
   const int row = gt / LPR, lane = gt % LPR;
@@ -128,22 +127,22 @@ k_spmv_cheb(int n_rows, const VT* __restrict__ vals, const int32_t* __restrict__
   if (row < n_rows)
   {
     const int en = end[row];
-    for (int j0 = beg[row] + lane; j0 < en; j0 += UNR * LPR)
+    for (int j0 = row_ptr[row] + lane; j0 < en; j0 += UNR * LPR)
     {
       int c[UNR];
-      VT v[UNR];
+      double v[UNR];
 #pragma unroll
       for (int t = 0; t < UNR; ++t)
       {
         const int jj = j0 + t * LPR;
         const bool ok = jj < en;
-        c[t] = ok ? (D16 ? row + (int)__ldcs(dcol + jj) : __ldcs(cols + jj)) : -1;
-        v[t] = ok ? __ldcs(vals + jj) : VT(0);
+        c[t] = ok ? __ldcs(cols + jj) : -1;
+        v[t] = ok ? __ldcs(vals + jj) : 0.0;
       }
 #pragma unroll
       for (int t = 0; t < UNR; ++t)
         if (c[t] >= 0)
-          s = fma((double)v[t], x[c[t]], s);
+          s = fma(v[t], x[c[t]], s);
     }
   }
 #pragma unroll
@@ -192,16 +191,15 @@ k_spmv_cheb_ghost_rows(int n_list, const int32_t* __restrict__ rows, const doubl
     cheb_row<MODE>(row, e.scratch[row] + s, x, e);
 }
 
-template <typename VT, bool D16>
-void launch_spmv_cheb(pmgx_ctx* c, int grid, int n_rows, const VT* vals, const int32_t* beg, const int32_t* end,
-                      const int32_t* row_ptr, const int16_t* dcol, const int32_t* cols, const double* x, const ChebEp& e)
+void launch_spmv_cheb(pmgx_ctx* c, int grid, int n_rows, const double* vals, const int32_t* row_ptr, const int32_t* end,
+                      const int32_t* cols, const double* x, const ChebEp& e)
 {
   switch (e.mode)
   {
-  case ChebEp::INIT: k_spmv_cheb<VT, D16, ChebEp::INIT><<<grid, ST, 0, c->stream>>>(n_rows, vals, beg, end, row_ptr, dcol, cols, x, e); break;
-  case ChebEp::STEP: k_spmv_cheb<VT, D16, ChebEp::STEP><<<grid, ST, 0, c->stream>>>(n_rows, vals, beg, end, row_ptr, dcol, cols, x, e); break;
-  case ChebEp::LAST: k_spmv_cheb<VT, D16, ChebEp::LAST><<<grid, ST, 0, c->stream>>>(n_rows, vals, beg, end, row_ptr, dcol, cols, x, e); break;
-  default: k_spmv_cheb<VT, D16, ChebEp::XONLY><<<grid, ST, 0, c->stream>>>(n_rows, vals, beg, end, row_ptr, dcol, cols, x, e); break;
+  case ChebEp::INIT: k_spmv_cheb<ChebEp::INIT><<<grid, ST, 0, c->stream>>>(n_rows, vals, row_ptr, end, cols, x, e); break;
+  case ChebEp::STEP: k_spmv_cheb<ChebEp::STEP><<<grid, ST, 0, c->stream>>>(n_rows, vals, row_ptr, end, cols, x, e); break;
+  case ChebEp::LAST: k_spmv_cheb<ChebEp::LAST><<<grid, ST, 0, c->stream>>>(n_rows, vals, row_ptr, end, cols, x, e); break;
+  default: k_spmv_cheb<ChebEp::XONLY><<<grid, ST, 0, c->stream>>>(n_rows, vals, row_ptr, end, cols, x, e); break;
   }
   check_launch("k_spmv_cheb");
   count_launch(c);
@@ -327,8 +325,7 @@ k_spmv_sell_cheb(int n_rows, const long long* __restrict__ slice_ptr, const floa
     cheb_row<MODE>(row, s, x, e);
 }
 
-// rectangular FP64 sliced-ELL product y (+)= M x (the AMG prolongator: 1..8 entries per row, thread per row)
-template <bool ACCUM>
+// rectangular FP64 sliced-ELL product y += M x (the AMG prolongator: 1..8 entries per row, thread per row)
 __global__ void __launch_bounds__(ST)
 k_spmv_sell_rect(int n_rows, const long long* __restrict__ slice_ptr, const double* __restrict__ vals,
                  const int32_t* __restrict__ cols, const double* __restrict__ x, double* __restrict__ y)
@@ -352,7 +349,7 @@ k_spmv_sell_rect(int n_rows, const long long* __restrict__ slice_ptr, const doub
   }
   if (k < w)
     s0 = fma(__ldcs(v + k * SLICE), x[__ldcs(c + k * SLICE)], s0);
-  y[row] = ACCUM ? y[row] + (s0 + s1) : s0 + s1;
+  y[row] = y[row] + (s0 + s1);
 }
 
 // widths[s] = 32 * max over the slice's rows of the owned-column length; overflow: a delta does not fit 16 bits
@@ -406,70 +403,45 @@ __global__ void k_sell_fill(int n_rows, const int32_t* __restrict__ row_ptr, con
   }
 }
 
-// rectangular product for the AMG transfer operators: same kernel body with LANES lanes per row
-template <int LANES, bool ACCUM>
+// rectangular product y = M x for the AMG restriction (long rows of P^T): a warp per row
 __global__ void __launch_bounds__(ST)
 k_spmv_rect(int n_rows, const double* __restrict__ vals, const int32_t* __restrict__ ptr,
             const int32_t* __restrict__ cols, const double* __restrict__ x, double* __restrict__ y)
 {
   const int gt = blockIdx.x * blockDim.x + threadIdx.x;
-  const int row = gt / LANES, lane = gt % LANES;
+  const int row = gt / 32, lane = gt % 32;
   double s = 0.0;
   if (row < n_rows)
   {
     const int e = ptr[row + 1];
-    for (int j = ptr[row] + lane; j < e; j += LANES)
+    for (int j = ptr[row] + lane; j < e; j += 32)
       s = fma(vals[j], x[cols[j]], s);
   }
 #pragma unroll
-  for (int o = LANES / 2; o > 0; o >>= 1)
+  for (int o = 16; o > 0; o >>= 1)
     s += __shfl_xor_sync(0xffffffffu, s, o);
   if (row < n_rows && lane == 0)
-    y[row] = ACCUM ? y[row] + s : s;
+    y[row] = s;
 }
 } // namespace
 
 void spmv_sell_rect(pmgx_ctx* c, int n_rows, const long long* slice_ptr, const int32_t* cols, const double* vals,
-                    const double* x, double* y, bool accumulate)
+                    const double* x, double* y)
 {
   if (n_rows <= 0)
     return;
-  const int grid = (n_rows + ST - 1) / ST;
-  if (accumulate)
-    k_spmv_sell_rect<true><<<grid, ST, 0, c->stream>>>(n_rows, slice_ptr, vals, cols, x, y);
-  else
-    k_spmv_sell_rect<false><<<grid, ST, 0, c->stream>>>(n_rows, slice_ptr, vals, cols, x, y);
+  k_spmv_sell_rect<<<(n_rows + ST - 1) / ST, ST, 0, c->stream>>>(n_rows, slice_ptr, vals, cols, x, y);
   check_launch("k_spmv_sell_rect");
   count_launch(c);
 }
 
 void spmv_rect(pmgx_ctx* c, int n_rows, const int32_t* row_ptr, const int32_t* cols, const double* vals,
-               const double* x, double* y, bool accumulate, int lanes)
+               const double* x, double* y)
 {
   if (n_rows <= 0)
     return;
-  const int grid = (int)(((long long)n_rows * lanes + ST - 1) / ST);
-  if (lanes == 32)
-  {
-    if (accumulate)
-      k_spmv_rect<32, true><<<grid, ST, 0, c->stream>>>(n_rows, vals, row_ptr, cols, x, y);
-    else
-      k_spmv_rect<32, false><<<grid, ST, 0, c->stream>>>(n_rows, vals, row_ptr, cols, x, y);
-  }
-  else if (lanes == 4)
-  {
-    if (accumulate)
-      k_spmv_rect<4, true><<<grid, ST, 0, c->stream>>>(n_rows, vals, row_ptr, cols, x, y);
-    else
-      k_spmv_rect<4, false><<<grid, ST, 0, c->stream>>>(n_rows, vals, row_ptr, cols, x, y);
-  }
-  else
-  {
-    if (accumulate)
-      k_spmv_rect<8, true><<<grid, ST, 0, c->stream>>>(n_rows, vals, row_ptr, cols, x, y);
-    else
-      k_spmv_rect<8, false><<<grid, ST, 0, c->stream>>>(n_rows, vals, row_ptr, cols, x, y);
-  }
+  const int grid = (int)(((long long)n_rows * 32 + ST - 1) / ST);
+  k_spmv_rect<<<grid, ST, 0, c->stream>>>(n_rows, vals, row_ptr, cols, x, y);
   check_launch("k_spmv_rect");
   count_launch(c);
 }
@@ -485,7 +457,7 @@ void CsrOperator::apply(double* x, double* y)
     halo_fwd_begin(halo, x);                                                       // :255
   if (n_owned > 0)
   {
-    k_spmv<false><<<grid, ST, 0, ctx->stream>>>(n_owned, values.p, row_ptr.p, off_diag.p, cols.p, x, y); // :256-260
+    k_spmv<<<grid, ST, 0, ctx->stream>>>(n_owned, values.p, row_ptr.p, off_diag.p, cols.p, x, y); // :256-260
     check_launch("k_spmv");
     count_launch(ctx);
   }
@@ -512,7 +484,7 @@ bool CsrOperator::apply_cheb(double* in, const ChebEp& e)
   if (halo)
     halo_fwd_begin(halo, in);
   if (n_owned > 0)
-    launch_spmv_cheb<double, false>(ctx, grid, n_owned, values.p, row_ptr.p, off_diag.p, row_ptr.p, nullptr, cols.p, in, e);
+    launch_spmv_cheb(ctx, grid, n_owned, values.p, row_ptr.p, off_diag.p, cols.p, in, e);
   if (halo)
     halo_fwd_end(halo, in);
   if (n_ghost_rows > 0)

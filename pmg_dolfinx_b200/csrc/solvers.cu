@@ -12,7 +12,6 @@
 #include "solvers.hpp"
 
 #include <cmath>
-#include <cstdlib>
 #include <cstring>
 
 namespace pmgx
@@ -321,8 +320,7 @@ static void cheb_solve_fused(pmgx_cheb* s, pmgx_operator* A, double* x, const do
 void cheb_solve(pmgx_cheb* s, pmgx_operator* A, double* x, const double* b, double* hist, bool x_is_zero,
                 ChebResidual final_r)
 {
-  static const bool fuse = !(getenv("PMGX_CHEB_FUSE") && atoi(getenv("PMGX_CHEB_FUSE")) == 0);
-  if (fuse && s->fuse && !hist && s->max_iter >= 2 && A->supports_cheb_fusion())
+  if (!hist && s->max_iter >= 2 && A->supports_cheb_fusion())
     return cheb_solve_fused(s, A, x, b, x_is_zero, final_r);
   pmgx_ctx* c = s->ctx;
   const long long n = s->n_owned;
@@ -592,8 +590,6 @@ int cgcg_solve(pmgx_coarse* co, double* x, const double* b, bool x_is_zero)
   // blocks [k0, k0 + check_every) with k0 even, k0 >= 2 and no last iteration inside are identical
   // launch sequences: capture once, replay
   // (an odd block length alternates between two graphs, one per parity of the scalar slots)
-  static const bool graphs_enabled = !(getenv("PMGX_COARSE_GRAPH") && atoi(getenv("PMGX_COARSE_GRAPH")) == 0);
-  const bool block_ok = graphs_enabled && !s->graph_off && check_every >= 1;
   auto run_block = [&](int k0)
   {
     const void* key[3] = {A, x, reinterpret_cast<const void*>((size_t)check_every)};
@@ -649,7 +645,7 @@ int cgcg_solve(pmgx_coarse* co, double* x, const double* b, bool x_is_zero)
   co->last_rel = 0.0;
   while (k < s->max_iter)
   {
-    if (block_ok && k >= 2 && k % check_every == 0 && k + check_every < s->max_iter && !s->graph_off)
+    if (k >= 2 && k % check_every == 0 && k + check_every < s->max_iter && !s->graph_off)
     {
       run_block(k);
       k += check_every;
@@ -920,8 +916,6 @@ int pmgx_coarse_create(pmgx_ctx* ctx, pmgx_operator* A, int max_iter, double rto
   cs->cg->r.release(); // the coarse variant works in its own slab
   cs->cg->y.release();
   cs->cg->p.release();
-  if (const char* e = getenv("PMGX_COARSE_CHECK_EVERY"))
-    cs->check_every = std::max(atoi(e), 1);
   *out = cs.release();
   PMGX_API_END
 }

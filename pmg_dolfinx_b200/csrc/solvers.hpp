@@ -14,7 +14,6 @@ struct pmgx_cheb
   int max_iter = 0;
   pmgx::DevBuf<double> z, q, r; // work vectors (owned + ghost), src/chebyshev.hpp:101-105
   pmgx::DevBuf<double> z2;      // second z buffer of the fused (row-complete operator) path, allocated on first use
-  bool fuse = true;             // use the operator's fused apply + update when it has one
 };
 
 namespace pmgx
@@ -81,11 +80,11 @@ struct pmgx_coarse
 namespace pmgx
 {
 int cgcg_solve(pmgx_coarse* cs, double* x, const double* b, bool x_is_zero);
-// rectangular CSR product y (=|+=) M x, `lanes` (4, 8 or 32) lanes per row (csr.cu)
+// rectangular CSR product y = M x, 32 lanes per row, for long rows (the AMG restriction; csr.cu)
 void spmv_rect(pmgx_ctx* c, int n_rows, const int32_t* row_ptr, const int32_t* cols, const double* vals,
-               const double* x, double* y, bool accumulate, int lanes);
-// the same product for a matrix stored as sliced ELL (32-row slices, column-major inside a slice; padding:
-// value 0, column 0): thread per row, for short rows (the AMG prolongator)
+               const double* x, double* y);
+// y += M x for a matrix stored as sliced ELL (32-row slices, column-major inside a slice; padding: value 0,
+// column 0): thread per row, for short rows (the AMG prolongator)
 void spmv_sell_rect(pmgx_ctx* c, int n_rows, const long long* slice_ptr, const int32_t* cols, const double* vals,
-                    const double* x, double* y, bool accumulate);
+                    const double* x, double* y);
 } // namespace pmgx

@@ -41,6 +41,15 @@ def _hierarchy(A, min_coarse=400, max_levels=10):
     return levels
 
 
+def _fp32_level0(levels):
+    """The hierarchy as the device cycle runs it: level 0 smooths with its matrix rounded to FP32 (the sliced-ELL copy
+    of csrc/csr.cu, make_lp), and the restriction takes the smoother's residual.  Its dinv and lmax, the transfers and
+    the coarser levels stay FP64."""
+    A = levels[0]["A"].copy()
+    A.data = A.data.astype(np.float32).astype(np.float64)
+    return [dict(levels[0], A=A)] + levels[1:]
+
+
 @pytest.mark.parametrize("n", [8, 16, 24])
 def test_hierarchy_is_galerkin_and_converges_like_the_prototype(n):
     A, bc = proto.p1_matrix(n)

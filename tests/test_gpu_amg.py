@@ -3,8 +3,9 @@ CoarseSolverType::solve (src/amg.hpp:67-113: PETSc KSPCG + BoomerAMG in the refe
 
 The reference holds no numbers for this third-party solve, so the device cycle is pinned against the
 numpy V-cycle of scripts/prototype_sa_amg.py run on the SAME hierarchy (pulled back from the library's
-host set-up, which tests/test_amg_setup.py and tests/test_amg_dist_cpu.py check against scipy): one
-application u = M^-1 r to 1e-10, symmetry of M^-1, and the PCG solve against scipy's direct solution."""
+host set-up, which tests/test_amg_setup.py and tests/test_amg_dist_cpu.py check against scipy), with level 0's
+smoothing matrix rounded to FP32 as the device streams it: one application u = M^-1 r to 1e-10, symmetry of
+M^-1, and the PCG solve against scipy's direct solution."""
 import os
 import sys
 
@@ -31,18 +32,14 @@ def _setup(ctx, n, min_coarse, nu=2, rtol=1e-8, max_iter=60):
     return api, proto, A, bc, nd, op, cs
 
 
-@pytest.mark.parametrize("fuse_from", [0, 1, 99], ids=["fused-smoother-all-levels", "fused-from-level-1", "unfused"])
-@pytest.mark.parametrize("lp", [False, True], ids=["fp64-matrix", "fp32-int16-smoother-matrix"])
-@pytest.mark.parametrize("n,nu", [(8, 2), (16, 2), (16, 1), (20, 3)])
-def test_device_cycle_equals_numpy_cycle_on_the_same_hierarchy(ctx, n, nu, lp, fuse_from, monkeypatch):
-    """lp: the level-0 smoother streams the matrix with FP32 values and 16-bit column deltas (the default):
-    the cycle is then the exact cycle of a matrix rounded to FP32, i.e. equal to 1e-6 instead of 1e-10."""
-    from test_amg_setup import _hierarchy
-    monkeypatch.setenv("PMGX_AMG_LP", "1" if lp else "0")
-    # which levels run the SpMV with the Chebyshev update as its epilogue (csr.cu k_spmv_cheb): all of them, the
-    # default (levels >= 1), none -- the three must agree with the numpy cycle
-    monkeypatch.setenv("PMGX_AMG_FUSE_FROM", str(fuse_from))
-    tol = 2e-6 if lp else 1e-10
+@pytest.mark.parametrize("nu", [1, 2, 3, 4])
+@pytest.mark.parametrize("n", [6, 8, 12, 16, 20, 24])
+def test_device_cycle_equals_numpy_cycle_on_the_same_hierarchy(ctx, n, nu):
+    """The level-0 smoother streams the matrix with FP32 values and 16-bit column deltas, so the device cycle is the
+    exact cycle of the hierarchy with level 0's smoothing matrix rounded to FP32.  nu = 1 runs the stand-alone SpMVs
+    and vector passes of the smoother (csr.cu k_spmv_sell, k_spmv); nu >= 2 runs the SpMVs with the Chebyshev update
+    as their epilogue on every level (k_spmv_sell_cheb, k_spmv_cheb), nu >= 3 with more than one z swap."""
+    from test_amg_setup import _hierarchy, _fp32_level0
     api, proto, A, bc, nd, op, cs = _setup(ctx, n, 100, nu=nu)
     levels = _hierarchy(A, min_coarse=100, max_levels=12)
     info = cs.levels()
@@ -56,15 +53,15 @@ def test_device_cycle_equals_numpy_cycle_on_the_same_hierarchy(ctx, n, nu, lp, f
     rv.copy_from_host(r)
     cs.apply_preconditioner(rv, uv)
     u = uv.data_copy()
-    uo = proto.vcycle(levels, 0, r, nu)
-    assert np.linalg.norm(u - uo) <= tol * np.linalg.norm(uo)
+    uo = proto.vcycle(_fp32_level0(levels), 0, r, nu)
+    assert np.linalg.norm(u - uo) <= 1e-10 * np.linalg.norm(uo), np.linalg.norm(u - uo) / np.linalg.norm(uo)
     # M^-1 is symmetric (same Chebyshev polynomial before and after the coarse correction)
     s = rng.uniform(-1, 1, nd) * (~bc)
     sv, tv = api.Vector(ctx, nd), api.Vector(ctx, nd)
     sv.copy_from_host(s)
     cs.apply_preconditioner(sv, tv)
     a, b = float(np.dot(s, u)), float(np.dot(r, tv.data_copy()))
-    assert abs(a - b) <= 1e-10 * max(abs(a), abs(b))   # exactly symmetric with the rounded matrix too
+    assert abs(a - b) <= 1e-10 * max(abs(a), abs(b))   # the rounded matrix is symmetric too
 
 
 @pytest.mark.parametrize("n", [12, 24])

@@ -68,16 +68,15 @@ def test_hierarchy_is_built_from_the_full_pattern(ctx, perturb):
     assert [i[4] for i in info[:-1]] == [l["P"].nnz for l in levels[:-1]]
 
 
-@pytest.mark.parametrize("fuse_from", [0, 1, 99], ids=["fused-smoother-all-levels", "fused-from-level-1", "unfused"])
-@pytest.mark.parametrize("lp", [False, True], ids=["fp64-matrix", "fp32-int16-smoother-matrix"])
-@pytest.mark.parametrize("perturb", BOXES, ids=BOX_IDS)
-def test_preconditioner_equals_numpy_cycle_of_the_full_pattern(ctx, perturb, lp, fuse_from, monkeypatch):
+@pytest.mark.parametrize("nu", [1, 2], ids=["unfused-smoother", "fused-smoother"])
+@pytest.mark.parametrize("perturb", [0.0, 0.05, 0.1, 0.15, 0.2, 0.25])
+def test_preconditioner_equals_numpy_cycle_of_the_full_pattern(ctx, perturb, nu):
+    """Level 0 smooths with the copy without stored zeros, in FP32 (the rounding of a uniform box's entries is exact,
+    that of a perturbed box's is not), so the reference is the numpy cycle with level 0's matrix rounded to FP32"""
     import prototype_sa_amg as proto
-    from test_amg_setup import _hierarchy
-    monkeypatch.setenv("PMGX_AMG_LP", "1" if lp else "0")
-    monkeypatch.setenv("PMGX_AMG_FUSE_FROM", str(fuse_from))
+    from test_amg_setup import _hierarchy, _fp32_level0
     api, A, H, bc, nd = _p1_csr(ctx, perturb)
-    cs = api.CoarseSolverType(ctx, A, 60, 1e-8, amg=True, nu=2, min_coarse=100)
+    cs = api.CoarseSolverType(ctx, A, 60, 1e-8, amg=True, nu=nu, min_coarse=100)
     levels = _hierarchy(H, min_coarse=100, max_levels=12)
     rng = np.random.default_rng(7)
     r = rng.uniform(-1, 1, nd) * (~bc)
@@ -85,9 +84,8 @@ def test_preconditioner_equals_numpy_cycle_of_the_full_pattern(ctx, perturb, lp,
     rv.copy_from_host(r)
     cs.apply_preconditioner(rv, uv)
     u = uv.data_copy()
-    uo = proto.vcycle(levels, 0, r, 2)
-    tol = 2e-6 if lp else 1e-10
-    assert np.linalg.norm(u - uo) <= tol * np.linalg.norm(uo)
+    uo = proto.vcycle(_fp32_level0(levels), 0, r, nu)
+    assert np.linalg.norm(u - uo) <= 1e-10 * np.linalg.norm(uo), np.linalg.norm(u - uo) / np.linalg.norm(uo)
     s = rng.uniform(-1, 1, nd) * (~bc)
     sv, tv = api.Vector(ctx, nd), api.Vector(ctx, nd)
     sv.copy_from_host(s)

@@ -153,22 +153,20 @@ def test_permuted_matrix_needs_32_bit_columns(permuted_p1):
     assert np.abs(Zn.indices.astype(np.int64) - rn).max() <= 32767   # natural order: 16-bit deltas suffice
 
 
-def _coarse(ctx, A):
+def _coarse(ctx, A, nu=2):
     from pmg_dolfinx_b200 import api
     op = api.MatrixOperator(ctx, A.indptr, A.indptr[1:], A.indices, A.data)
-    return api, op, api.CoarseSolverType(ctx, op, 60, 1e-8, amg=True, nu=2, min_coarse=100)
+    return api, op, api.CoarseSolverType(ctx, op, 60, 1e-8, amg=True, nu=nu, min_coarse=100)
 
 
-@pytest.mark.parametrize("fuse_from", [0, 99], ids=["fused-smoother-all-levels", "unfused"])
-@pytest.mark.parametrize("lp", [True, False], ids=["fp32-int32-smoother-matrix", "fp64-matrix"])
-def test_preconditioner_on_a_matrix_with_32_bit_columns(ctx, permuted_p1, lp, fuse_from, monkeypatch):
+@pytest.mark.parametrize("nu", [1, 2, 3, 4])
+def test_preconditioner_on_a_matrix_with_32_bit_columns(ctx, permuted_p1, nu):
+    """nu = 1: the stand-alone SpMV k_spmv_sell<false>; nu >= 2: the fused k_spmv_sell_cheb<false, *>"""
     import prototype_sa_amg as proto
-    from test_amg_setup import _hierarchy
-    monkeypatch.setenv("PMGX_AMG_LP", "1" if lp else "0")
-    monkeypatch.setenv("PMGX_AMG_FUSE_FROM", str(fuse_from))
+    from test_amg_setup import _hierarchy, _fp32_level0
     A, bc = permuted_p1
     nd = A.shape[0]
-    api, op, cs = _coarse(ctx, A)
+    api, op, cs = _coarse(ctx, A, nu)
     levels = _hierarchy(A, min_coarse=100, max_levels=12)
     info = cs.levels()
     assert len(info) == len(levels) and [i[0] for i in info] == [l["A"].shape[0] for l in levels]
@@ -178,9 +176,8 @@ def test_preconditioner_on_a_matrix_with_32_bit_columns(ctx, permuted_p1, lp, fu
     rv.copy_from_host(r)
     cs.apply_preconditioner(rv, uv)
     u = uv.data_copy()
-    uo = proto.vcycle(levels, 0, r, 2)
-    tol = 2e-6 if lp else 1e-10
-    assert np.linalg.norm(u - uo) <= tol * np.linalg.norm(uo), np.linalg.norm(u - uo) / np.linalg.norm(uo)
+    uo = proto.vcycle(_fp32_level0(levels), 0, r, nu)
+    assert np.linalg.norm(u - uo) <= 1e-10 * np.linalg.norm(uo), np.linalg.norm(u - uo) / np.linalg.norm(uo)
     s = rng.uniform(-1, 1, nd) * (~bc)
     sv, tv = api.Vector(ctx, nd), api.Vector(ctx, nd)
     sv.copy_from_host(s)

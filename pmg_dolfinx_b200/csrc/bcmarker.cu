@@ -116,9 +116,11 @@ extern "C" int pmgx_bc_marker_exterior(pmgx_ctx* ctx, int degree, int n_cells, c
                                        int8_t* marker_out)
 {
   PMGX_API_BEGIN
-  PMGX_REQUIRE(ctx && marker_out && degree >= 1 && degree <= PMGX_MAX_DEGREE, "bc_marker_exterior: bad arguments");
+  PMGX_REQUIRE(ctx && degree >= 1 && degree <= PMGX_MAX_DEGREE, "bc_marker_exterior: bad arguments");
   PMGX_REQUIRE(n_cells >= 0 && n_owned >= 0 && n_ghost >= 0 && (long long)n_cells * 6 < (1ll << 31),
                "bc_marker_exterior: bad sizes");
+  // a rank without cells has a zero-length marker, whose device pointer may be null
+  PMGX_REQUIRE(marker_out || n_owned + n_ghost == 0, "bc_marker_exterior: null marker");
   PMGX_REQUIRE(n_cells == 0 || (geom_dofmap && dofmap), "bc_marker_exterior: null array");
   PMGX_REQUIRE(!halo || (halo->n_owned == n_owned && halo->n_ghost == n_ghost), "bc_marker_exterior: halo does not match the layout");
   PMGX_CUDA(cudaSetDevice(ctx->device));

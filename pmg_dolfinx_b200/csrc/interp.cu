@@ -520,7 +520,9 @@ int pmgx_interp_create(pmgx_ctx* ctx, int degree_coarse, int degree_fine, int n_
 int pmgx_interp_prolong(pmgx_interp* it, double* coarse, double* fine)
 {
   PMGX_API_BEGIN
-  PMGX_REQUIRE(it && coarse && fine, "interp_prolong: null argument");
+  // a rank without cells has zero-length vectors, whose device pointers may be null
+  PMGX_REQUIRE(it && (coarse || it->n_coarse_total == 0) && (fine || it->n_fine_total == 0),
+               "interp_prolong: null argument");
   pmgx::interp_prolong(it, coarse, fine, false);
   PMGX_API_END
 }
@@ -528,7 +530,8 @@ int pmgx_interp_prolong(pmgx_interp* it, double* coarse, double* fine)
 int pmgx_interp_restrict(pmgx_interp* it, double* fine, double* coarse)
 {
   PMGX_API_BEGIN
-  PMGX_REQUIRE(it && coarse && fine, "interp_restrict: null argument");
+  PMGX_REQUIRE(it && (coarse || it->n_coarse_total == 0) && (fine || it->n_fine_total == 0),
+               "interp_restrict: null argument");
   pmgx::interp_restrict(it, fine, nullptr, coarse);
   PMGX_API_END
 }

@@ -2463,8 +2463,10 @@ int pmgx_laplacian_device_bytes(pmgx_operator* op, long long* bytes_h)
 int pmgx_laplacian_rhs(pmgx_operator* op, const double* fvals, double g, double* b)
 {
   PMGX_API_BEGIN
-  PMGX_REQUIRE(op && op->kind == pmgx_operator::LAPLACIAN && fvals && b, "laplacian_rhs: bad arguments");
+  PMGX_REQUIRE(op && op->kind == pmgx_operator::LAPLACIAN, "laplacian_rhs: bad arguments");
   auto* L = static_cast<Laplacian*>(op);
+  // a rank without cells has zero-length vectors, whose device pointers may be null
+  PMGX_REQUIRE((fvals && b) || L->n_owned + L->n_ghost == 0, "laplacian_rhs: null argument");
   pmgx_ctx* ctx = L->ctx;
   PMGX_CUDA(cudaSetDevice(ctx->device));
   const long long total = (long long)L->n_list() * L->n3;
@@ -2510,8 +2512,9 @@ int pmgx_laplacian_rhs(pmgx_operator* op, const double* fvals, double g, double*
 int pmgx_laplacian_lift(pmgx_operator* op, const double* gvals, double* b)
 {
   PMGX_API_BEGIN
-  PMGX_REQUIRE(op && op->kind == pmgx_operator::LAPLACIAN && gvals && b, "laplacian_lift: bad arguments");
+  PMGX_REQUIRE(op && op->kind == pmgx_operator::LAPLACIAN, "laplacian_lift: bad arguments");
   auto* L = static_cast<Laplacian*>(op);
+  PMGX_REQUIRE((gvals && b) || L->n_owned + L->n_ghost == 0, "laplacian_lift: null argument");
   pmgx_ctx* ctx = L->ctx;
   PMGX_CUDA(cudaSetDevice(ctx->device));
   const int ntot = L->n_owned + L->n_ghost;
@@ -2650,7 +2653,11 @@ int pmgx_csr_from_laplacian(pmgx_operator* op, pmgx_operator** out)
 int pmgx_operator_apply(pmgx_operator* op, double* x, double* y)
 {
   PMGX_API_BEGIN
-  PMGX_REQUIRE(op && x && y, "operator_apply: null argument");
+  PMGX_REQUIRE(op, "operator_apply: null argument");
+  // a rank without dofs has zero-length vectors, whose device pointers may be null
+  if (op->n_owned + op->n_ghost == 0 && !(x && y))
+    return PMGX_OK;
+  PMGX_REQUIRE(x && y, "operator_apply: null argument");
   PMGX_REQUIRE(x != y, "operator_apply: in-place apply is not supported");
   op->apply(x, y);
   PMGX_API_END
@@ -2659,7 +2666,7 @@ int pmgx_operator_apply(pmgx_operator* op, double* x, double* y)
 int pmgx_operator_get_diag_inverse(pmgx_operator* op, double* out)
 {
   PMGX_API_BEGIN
-  PMGX_REQUIRE(op && out, "get_diag_inverse: null argument");
+  PMGX_REQUIRE(op && (out || op->n_owned == 0), "get_diag_inverse: null argument");
   pmgx::vec::copy(op->ctx, out, op->diag_inv.p, op->n_owned);
   PMGX_API_END
 }
@@ -2667,7 +2674,7 @@ int pmgx_operator_get_diag_inverse(pmgx_operator* op, double* out)
 int pmgx_operator_set_diag_inverse(pmgx_operator* op, const double* in)
 {
   PMGX_API_BEGIN
-  PMGX_REQUIRE(op && in, "set_diag_inverse: null argument");
+  PMGX_REQUIRE(op && (in || op->n_owned == 0), "set_diag_inverse: null argument");
   pmgx::vec::copy(op->ctx, op->diag_inv.p, in, op->n_owned);
   PMGX_API_END
 }

@@ -3,9 +3,11 @@ columns of the sliced-ELL smoother matrix.
 
 Ghost columns: a MatrixOperator whose rows have entries after off_diag_offset runs k_spmv_ghost_rows in the SpMV
 and, in the fused Chebyshev solve, parks the owned-column partial sum of those rows in a scratch vector and finishes
-them in k_spmv_cheb_ghost_rows.  Without a halo the ghost block of x is whatever the caller put there, and the
-smoother's internal vectors keep a zero ghost block (they are zeroed at allocation), so the solve is the Chebyshev
-iteration of A_oo with right-hand side b - A_og x_g.
+them in k_spmv_cheb_ghost_rows.  The Chebyshev test takes two such matrices: one built from host arrays, and the P1
+matrix of one rank of a box partition, assembled on the device with its ghost-column block (pmgx_csr_from_laplacian).
+Without a halo the ghost block of x is whatever the caller put there, and the smoother's internal vectors keep a zero
+ghost block (they are zeroed at allocation), so the solve is the Chebyshev iteration of A_oo with right-hand side
+b - A_og x_g.
 
 32-bit columns: the AMG level-0 smoother matrix stores FP32 values with 16-bit column deltas, and falls back to 32-bit
 columns when some owned-column delta leaves +-32767.  A randomly permuted P1 matrix has such deltas.
@@ -64,6 +66,23 @@ def _ghost_operator(ctx):
     return api, R, n_o, k, op
 
 
+def _device_ghost_operator(ctx):
+    """rank 0 of a (2, 1, 1) partition of a perturbed box: its P1 matrix assembled on the device, as (api, the owned
+    rows [A_oo A_og], owned count, ghost count, operator)"""
+    from pmg_dolfinx_b200 import api
+    m = api.BoxMesh((6, 5, 7), (2, 1, 1), 0, perturb=0.15)
+    s = m.space(1)
+    kap = np.random.default_rng(4).uniform(0.5, 2.0, m.n_cells)
+    d = [ctx.to_device(a) for a in (kap, s.dofmap, m.xgeom, m.geom_dofmap, s.bc)]
+    lap = api.MatFreeLaplacian(ctx, 1, d[0], d[1], d[2], d[3], m.lcells, m.bcells, d[4], s.n_owned, s.n_ghost)
+    op = lap.to_csr()
+    m.close()
+    rp, co, va = op.to_host()
+    R = sp.csr_matrix((va, co, rp), shape=(s.n_owned, s.n_owned + s.n_ghost))
+    assert s.n_ghost > 0 and R[:, s.n_owned:].nnz > 0
+    return api, R, s.n_owned, s.n_ghost, op
+
+
 def _vec(api, ctx, n_o, k, owned, ghost):
     v = api.Vector(ctx, n_o, k)
     v.data[:n_o].copy_(torch.from_numpy(np.ascontiguousarray(owned)))
@@ -88,10 +107,11 @@ def test_spmv_with_ghost_columns_and_no_halo(ctx):
 
 @pytest.mark.parametrize("its", [2, 3, 5])
 @pytest.mark.parametrize("x0", ["zero", "nonzero"])
-def test_chebyshev_with_ghost_columns_fused_and_unfused(ctx, its, x0):
+@pytest.mark.parametrize("matrix", ["host", "device"])
+def test_chebyshev_with_ghost_columns_fused_and_unfused(ctx, its, x0, matrix):
     """silent solve: the fused path (k_spmv_cheb + k_spmv_cheb_ghost_rows with the parked sums); verbose solve: the
     unfused path (SpMV, then a vector pass).  Both against the oracle's Chebyshev on A_oo, b - A_og x_g."""
-    api, R, n_o, k, op = _ghost_operator(ctx)
+    api, R, n_o, k, op = (_ghost_operator if matrix == "host" else _device_ghost_operator)(ctx)
     Aoo, Aog = R[:, :n_o].tocsr(), R[:, n_o:].tocsr()
     dinv = 1.0 / Aoo.diagonal()
     dv = api.Vector(ctx, n_o, k)

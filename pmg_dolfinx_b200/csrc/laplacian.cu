@@ -63,6 +63,22 @@ __device__ __forceinline__ int ldg_stream_i32(const int* p) { return __ldcs(p); 
 //           batch = cpb consecutive cells of the launch list (cpb of the kernel that runs),
 //           slot = cell_in_batch*n + iz, S / SE padded to 16-byte rows; lcells and bcells
 //           batches are padded separately.
+// The host lays out enc and G with slab_S / slab_SE, and the slab kernels read them with the strides of SlabCfg
+// (and TmaCfg::S), which come from the same two functions: the layout and the kernel that reads it cannot disagree.
+constexpr int slab_S(int cpb, int n) { return (cpb * n + 1) & ~1; }  // G rows: 16-byte multiples, (almost) no padding streamed
+constexpr int slab_SE(int cpb, int n) { return (cpb * n + 3) & ~3; } // dofmap rows: 16-byte multiples of int32
+
+// The SLAB layout as a slab kernel of degree P with CPB cells per batch reads it
+template <int P, int CPB>
+struct SlabCfg
+{
+  static constexpr int n = P + 1;
+  static constexpr int n2 = n * n;
+  static constexpr int cpb = CPB;
+  static constexpr int SE = slab_SE(CPB, n);
+  static constexpr uint32_t enc_bytes = n2 * SE * sizeof(int32_t); // one batch of the encoded dofmap
+};
+
 struct Lay
 {
   int mode; // 0 COLUMN, 1 SLAB
@@ -815,6 +831,29 @@ struct ApplyArgs
   int literal_detj;
 };
 
+// Runs launch() (one apply-kernel launch of degree P on stream st), checks and counts it; with profiling on,
+// the interior-cell launch is timed into c->prof[P]
+template <typename F>
+void timed_launch(pmgx_ctx* c, cudaStream_t st, const ApplyArgs& a, const char* name, int P, F&& launch)
+{
+  const bool timed = c->profiling && a.cell0 == 0; // per-kernel timing covers the interior-cell launch only
+  cudaEvent_t e0 = nullptr, e1 = nullptr;
+  if (timed)
+  {
+    PMGX_CUDA(cudaEventCreate(&e0));
+    PMGX_CUDA(cudaEventCreate(&e1));
+    PMGX_CUDA(cudaEventRecord(e0, st));
+  }
+  launch();
+  check_launch(name);
+  count_launch(c);
+  if (timed)
+  {
+    PMGX_CUDA(cudaEventRecord(e1, st));
+    c->prof[P].emplace_back(e0, e1);
+  }
+}
+
 // Launches a persistent apply kernel of degree P: CTAs of tpb threads stay resident and walk over the
 // n_blocks blocks of work (blockIdx.x, + gridDim.x, ...), so exactly as many are launched as fit on the
 // device at once.  The shared-memory opt-in and the occupancy query run once per device and kernel.
@@ -834,22 +873,8 @@ void launch_persistent(pmgx_ctx* c, cudaStream_t st, const ApplyArgs& a, const c
     ctas_per_sm[c->device] = nb;
   }
   const int grid = std::min(n_blocks, ctas_per_sm[c->device] * c->num_sms);
-  const bool timed = c->profiling && a.cell0 == 0; // per-kernel timing covers the interior-cell launch only
-  cudaEvent_t e0 = nullptr, e1 = nullptr;
-  if (timed)
-  {
-    PMGX_CUDA(cudaEventCreate(&e0));
-    PMGX_CUDA(cudaEventCreate(&e1));
-    PMGX_CUDA(cudaEventRecord(e0, st));
-  }
-  kernel<<<grid, tpb, smem, st>>>(a.x, a.y, a.geom, a.enc, a.perm, a.kappa, tail...);
-  check_launch(name);
-  count_launch(c);
-  if (timed)
-  {
-    PMGX_CUDA(cudaEventRecord(e1, st));
-    c->prof[P].emplace_back(e0, e1);
-  }
+  timed_launch(c, st, a, name, P,
+               [&] { kernel<<<grid, tpb, smem, st>>>(a.x, a.y, a.geom, a.enc, a.perm, a.kappa, tail...); });
 }
 
 // The SLAB-layout kernels (k_apply_tma, k_apply_affine*): one block of work is one batch of Cfg::cpb cells
@@ -1070,23 +1095,12 @@ struct ColumnApply
       configured[c->device] = true;
     }
     const int grid = (a.count + C::cpb - 1) / C::cpb;
-    const bool timed = c->profiling && a.cell0 == 0; // per-kernel timing covers the interior-cell launch only
-    cudaEvent_t e0 = nullptr, e1 = nullptr;
-    if (timed)
-    {
-      PMGX_CUDA(cudaEventCreate(&e0));
-      PMGX_CUDA(cudaEventCreate(&e1));
-      PMGX_CUDA(cudaEventRecord(e0, st));
-    }
-    k_apply<P, RECOMPUTE><<<grid, C::tpb, smem, st>>>(a.x, a.y, a.geom, a.enc, a.perm, a.kappa, a.cell0, a.count,
-                                                      a.xgeom, a.geom_dofmap, a.literal_detj);
-    check_launch("k_apply");
-    count_launch(c);
-    if (timed)
-    {
-      PMGX_CUDA(cudaEventRecord(e1, st));
-      c->prof[P].emplace_back(e0, e1);
-    }
+    timed_launch(c, st, a, "k_apply", P,
+                 [&]
+                 {
+                   k_apply<P, RECOMPUTE><<<grid, C::tpb, smem, st>>>(a.x, a.y, a.geom, a.enc, a.perm, a.kappa, a.cell0,
+                                                                     a.count, a.xgeom, a.geom_dofmap, a.literal_detj);
+                 });
   }
 };
 
@@ -1103,6 +1117,10 @@ struct ColumnApply
 // keeps a ring of R geometry planes (and the next batch's dofmap) in flight with
 // cp.async.bulk (TMA) into shared memory, completion tracked by mbarriers.  Memory-level
 // parallelism is then set by the ring depth, not by occupancy or register count.
+// The four slab kernels share their layout (SlabCfg) but each writes out its own dofmap pipeline, gather and
+// scatter: routed through shared device helpers in the same instruction order, ptxas allocated registers
+// differently in 6 of the 15 instantiations (k_apply_affine2<3,64> 158 -> 180 registers, k_apply_affine<5,64>
+// 48 -> 64 B of spills, CUDA 12.9).
 __device__ __forceinline__ uint32_t smem_u32(const void* p)
 {
   return static_cast<uint32_t>(__cvta_generic_to_shared(p));
@@ -1150,16 +1168,14 @@ __device__ __forceinline__ void bulk_g2s(void* dst, const void* src, uint32_t by
 
 // RECOMPUTE: no geometry ring; every thread forms G at its points from the cell's vertices (JacobianAtZeta)
 template <int P, int TPB, bool RECOMPUTE = false>
-struct TmaCfg
+struct TmaCfg : SlabCfg<P, TPB / (P + 1)>
 {
-  static constexpr int n = P + 1;
-  static constexpr int n2 = n * n;
+  using Slab = SlabCfg<P, TPB / (P + 1)>;
+  using Slab::n, Slab::cpb, Slab::enc_bytes;
   static constexpr int tpb = TPB;
   static constexpr int R = 2; // geometry planes in flight (measured on B200: a 2-plane ring wins for P3/P4)
   static constexpr int ring = RECOMPUTE ? 0 : R;
-  static constexpr int cpb = tpb / n;
-  static constexpr int S = (cpb * n + 1) & ~1;  // G rows: 16-byte multiples, (almost) no padding streamed
-  static constexpr int SE = (cpb * n + 3) & ~3; // dofmap rows: 16-byte multiples of int32
+  static constexpr int S = slab_S(cpb, n);
   static constexpr int minb = P == 1 ? 4 : (P == 2 ? 3 : (TPB <= 64 ? 4 : 2)); // resident CTAs per SM
   static constexpr int kp = n + (n & 1);
   // per-cell stride of a z-row plane buffer: an odd number of 16-byte chunks, so the cells of
@@ -1168,7 +1184,6 @@ struct TmaCfg
   static constexpr int cs = ((n * kp / 2) & 1) ? n * kp : n * kp + 2;
   static constexpr int plane_doubles = n * 6 * S;
   static constexpr uint32_t plane_bytes = plane_doubles * sizeof(double);
-  static constexpr uint32_t enc_bytes = n2 * SE * sizeof(int32_t);
   static constexpr int buf_doubles = 2 * cpb * cs; // double-buffered plane rows (su and sf each)
   // RECOMPUTE: instead of the ring, [21][TPB] JacobianAtZeta coefficients and [n][6][TPB] G at the thread's points
   // of the current plane, one column per thread (written and read by the same thread: no barrier)
@@ -1452,16 +1467,13 @@ struct TmaApply
 // buffer); the kernel is then bound by the gather / atomic traffic of x and y in L2, not by HBM.
 // Meshes with any non-affine cell keep the streamed-G kernels; PMGX_LAP_STREAM_G forces them.
 template <int P, int TPB>
-struct AffCfg
+struct AffCfg : SlabCfg<P, TPB / (P + 1)>
 {
-  static constexpr int n = P + 1;
-  static constexpr int n2 = n * n;
+  using Slab = SlabCfg<P, TPB / (P + 1)>;
+  using Slab::n, Slab::cpb, Slab::enc_bytes;
   static constexpr int tpb = TPB;
-  static constexpr int cpb = tpb / n;
-  static constexpr int SE = (cpb * n + 3) & ~3;
   static constexpr int kp = n + (n & 1);
   static constexpr int cs = ((n * kp / 2) & 1) ? n * kp : n * kp + 2;
-  static constexpr uint32_t enc_bytes = n2 * SE * sizeof(int32_t);
   static constexpr int buf_doubles = 2 * cpb * cs;
   static constexpr size_t off_su = 2 * (size_t)enc_bytes;
   static constexpr size_t off_sf = off_su + (size_t)buf_doubles * sizeof(double);
@@ -1671,16 +1683,11 @@ struct AffineApply
 // busy with 20 %-efficient broadcast reads; n double shuffles move the same data in ~40 % fewer
 // pipe cycles and the warps of a CTA no longer wait for each other.
 template <int P, int TPB>
-struct AffShCfg
+struct AffShCfg : SlabCfg<P, (TPB / 32) * (32 / (P + 1))> // a warp holds 32 / n whole cells
 {
-  static constexpr int n = P + 1;
-  static constexpr int n2 = n * n;
   static constexpr int tpb = TPB;
-  static constexpr int cpw = 32 / n;               // cells per warp
-  static constexpr int cpb = (TPB / 32) * cpw;     // cells per batch
-  static constexpr int SE = (cpb * n + 3) & ~3;
-  static constexpr uint32_t enc_bytes = n2 * SE * sizeof(int32_t);
-  static constexpr size_t off_bar = 2 * (size_t)enc_bytes;
+  static constexpr int cpw = 32 / (P + 1); // cells per warp
+  static constexpr size_t off_bar = 2 * (size_t)AffShCfg::enc_bytes;
   static constexpr size_t smem = off_bar + 2 * sizeof(uint64_t);
   static constexpr int minb = P <= 2 ? 6 : (TPB <= 64 ? 4 : 2);
 };
@@ -1865,17 +1872,14 @@ struct AffineShflApply
 // stride CS = n (mod 16) doubles make the 8-byte bank of BOTH access patterns (unit stride in t when
 // writing, stride SS in t when reading) equal to lane + const: every 64-bit access is conflict-free.
 template <int P, int TPB>
-struct Aff2Cfg
+struct Aff2Cfg : SlabCfg<P, (TPB / 32) * (32 / (P + 1))> // a warp holds 32 / n whole cells
 {
-  static constexpr int n = P + 1;
-  static constexpr int n2 = n * n;
+  using Slab = SlabCfg<P, (TPB / 32) * (32 / (P + 1))>;
+  using Slab::n, Slab::n2, Slab::cpb, Slab::enc_bytes;
   static constexpr int tpb = TPB;
-  static constexpr int cpw = 32 / n;               // cells per warp
-  static constexpr int cpb = (TPB / 32) * cpw;     // cells per batch
-  static constexpr int SE = (cpb * n + 3) & ~3;
-  static constexpr int ss = ((n2 - 1 + 15) / 16) * 16 + 1;                 // >= n2, = 1 mod 16
-  static constexpr int cs = ((n * ss - n + 15) / 16) * 16 + n;             // >= n * ss, = n mod 16
-  static constexpr uint32_t enc_bytes = n2 * SE * sizeof(int32_t);
+  static constexpr int cpw = 32 / n;                           // cells per warp
+  static constexpr int ss = ((n2 - 1 + 15) / 16) * 16 + 1;     // >= n2, = 1 mod 16
+  static constexpr int cs = ((n * ss - n + 15) / 16) * 16 + n; // >= n * ss, = n mod 16
   static constexpr int buf_doubles = cpb * cs;
   static constexpr size_t off_a = 2 * (size_t)enc_bytes;
   static constexpr size_t off_b = off_a + (size_t)buf_doubles * sizeof(double);
@@ -2349,8 +2353,8 @@ int pmgx_laplacian_create(pmgx_ctx* ctx, int degree, int n_cells, const int32_t*
   lay.mode = lay.cpb > 0 ? 1 : 0;
   if (lay.mode == 1)
   {
-    lay.S = (lay.cpb * n + 1) & ~1;
-    lay.SE = (lay.cpb * n + 3) & ~3;
+    lay.S = pmgx::slab_S(lay.cpb, n);
+    lay.SE = pmgx::slab_SE(lay.cpb, n);
     lay.nb_l = (n_lcells + lay.cpb - 1) / lay.cpb;
     lay.n_batches = lay.nb_l + (n_bcells + lay.cpb - 1) / lay.cpb;
   }
